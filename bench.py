@@ -23,6 +23,11 @@ observation per env-step), BASELINE.json's metric.
               72 envs (README config) and 1 env (config 1, short form; `--config single` runs test.py's full protocol).
 * `cpu_baseline` / `--impl reference`: the CPU oracle (a port of the reference's algorithm; PyBoy itself
               cannot be installed here) on the box's host cores, on a bounded sample of the same workload.
+* `--dump-outputs DIR`: what the timed path handed its caller at its last step, as float32 / float64 .npy files
+              (see dump_outputs), so that two builds can be compared output for output on identical inputs.
+
+The benchmark writes nothing into the repository tree: a library whose sources are newer than the build that
+build() left there is rebuilt in a temporary directory.
 """
 from __future__ import annotations
 
@@ -33,6 +38,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 from pathlib import Path
@@ -40,6 +46,7 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parent
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
+SCRATCH = tempfile.TemporaryDirectory(prefix="pokegym-bench-")  # rebuilds of stale libraries; removed at exit
 
 ALGO_BYTES_PER_ENV_STEP = 57_682  # BASELINE.md section 4 / SURVEY.md 8d
 ROLLOUT_T = 32
@@ -61,7 +68,7 @@ def workload_name(args) -> str:
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 200; 10,000 with --config single)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--envs-per-gpu", type=int, default=4096)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -78,7 +85,22 @@ def parse_args():
     ap.add_argument("--also-envs", type=int, default=-1,
                     help="extra single-GPU leg at this env count, reported under 'large_batch' (0 = skip; -1 = one full wave of resident envs)")
     ap.add_argument("--also-steps", type=int, default=12)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the observations, rewards, dones and info sum of the last timed step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.steps is None and not (args.config == "single" and args.impl == "ours"):  # run_single_config: None = test.py's protocol
+        args.steps = 200
+    if args.dump_outputs and (args.impl != "ours" or args.config or args.only_leg):
+        ap.error("--dump-outputs writes the outputs of the headline run: it does not combine with --impl reference, --config or --only-leg")
+    return args
+
+
+def library(build):
+    """Path of the shared library `build` (__graft_entry__.build_cuda or build_oracle) makes: the one build() left in the
+    tree while it is current, else a fresh build in SCRATCH."""
+    return build(out_dir=SCRATCH.name)
 
 
 def measured_peak():
@@ -225,7 +247,7 @@ def oracle_run(rom: bytes, seconds: float, n_envs=None, state_path=None, mixed=F
     from pokegym_b200 import _capi
     import __graft_entry__ as g
 
-    lib = _capi.GbEnvLib(g.build_oracle(), "oracle_")
+    lib = _capi.GbEnvLib(library(g.build_oracle), "oracle_")
     cores = os.cpu_count() or 1
     n = n_envs or max(cores * 16, 64)  # >= 16 envs per worker thread: thread start-up is amortised over ~20 ms of work
     h = _capi.Handle(lib, n, rom)
@@ -264,7 +286,7 @@ def run_reference(args):
     rom = build_rom(args.rom)
     cores = os.cpu_count() or 1
     n = max(cores * 16, 64)
-    lib = _capi.GbEnvLib(g.build_oracle(), "oracle_")
+    lib = _capi.GbEnvLib(library(g.build_oracle), "oracle_")
     h = _capi.Handle(lib, n, rom)
     start_envs(h, args.state, n)
     obs = np.zeros((n, _capi.OBS_BYTES), dtype=np.uint8)
@@ -355,6 +377,35 @@ def e2e_host_loop(hs, E, n_e2e, world=1, dev=None):
     return world * E * n_e2e / e2e_s
 
 
+DUMP_OBS_ENVS = 512  # observations of at most this many envs: 512 x 23,040 values x 4 B = 47 MB of float32
+
+
+def dump_outputs(out_dir, obs, reward, done, info_sum):
+    """--dump-outputs: what the caller of the timed path (rank 0's E envs) holds after its last step, as DIR/<name>.npy --
+    obs.npy      float32 [n, 72, 80, 4]  the step's observations of n = min(E, DUMP_OBS_ENVS) envs: all of them, or for
+                                         larger batches the envs numpy.random.default_rng(0).choice(E, n, replace=False)
+                                         picks, in ascending order;
+    reward.npy   float64 [E]             the step's rewards;
+    done.npy     float32 [E]             the step's done flags;
+    info_sum.npy float64 [72]            the episode-info sums of the last reduction.
+    The actions come from a seeded generator and every env starts from the same state, so the same arguments give the same
+    inputs on every run and every build."""
+    import numpy as np
+    import torch
+
+    from pokegym_b200 import _capi
+
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    E = obs.shape[0]
+    ids = np.sort(np.random.default_rng(0).choice(E, DUMP_OBS_ENVS, replace=False)) if E > DUMP_OBS_ENVS else np.arange(E)
+    sample = obs[torch.from_numpy(ids).to(obs.device)].cpu().numpy()
+    np.save(out / "obs.npy", sample.reshape(len(ids), _capi.OBS_H, _capi.OBS_W, _capi.OBS_C).astype(np.float32))
+    np.save(out / "reward.npy", reward.cpu().numpy().astype(np.float64))
+    np.save(out / "done.npy", done.cpu().numpy().astype(np.float32))
+    np.save(out / "info_sum.npy", info_sum.cpu().numpy().astype(np.float64))
+
+
 def run_leg(lib, rom, E, steps, warmup, preroll, dev, device_id, seed=7, state_path=None, mixed=False, lanes=None, e2e_steps=0):
     """One single-GPU workload: E envs, device-resident actions, obs into a 4-deep device ring.  CUDA-event timed."""
     import torch
@@ -424,7 +475,7 @@ def run_single_config(args):
     from pokegym_b200 import Environment
 
     rom = build_rom(args.rom)
-    warm, steps = (1000, 10000) if args.steps == 200 else (max(args.warmup, 3), args.steps)
+    warm, steps = (1000, 10000) if args.steps is None else (max(args.warmup, 3), args.steps)
     env = Environment(rom, state_path=args.state)
     env.reset()
     for _ in range(warm):
@@ -469,13 +520,14 @@ def main():
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     if args.config == "single":
-        g.build_cuda()
+        if library(g.build_cuda) != _capi.DEFAULT_LIB:  # pokegym_b200.Environment loads the in-tree library
+            raise SystemExit(f"{_capi.DEFAULT_LIB} is older than its sources: run build() before --config single")
         run_single_config(args)
         return
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    # GBENV_LIB: A/B builds of the kernel while tuning (tools/quick_bench.sh); the judged runs use the in-tree library
-    lib = _capi.GbEnvLib(os.environ.get("GBENV_LIB") or (g.build_cuda() if rank == 0 or not _capi.DEFAULT_LIB.exists() else _capi.DEFAULT_LIB))
+    # GBENV_LIB: another build of the kernel library, for A/B runs while tuning (tools/gpu_variants.sh)
+    lib = _capi.GbEnvLib(os.environ.get("GBENV_LIB") or library(g.build_cuda))
     if args.only_leg:
         if args.only_leg.startswith("custom:"):  # custom:rom,envs,steps,warmup,preroll,mixed  (tuning sweeps)
             f = args.only_leg[7:].split(",")
@@ -550,6 +602,9 @@ def main():
         dist.barrier()
     ms = max_over_ranks(ms, dev)
     value = world * E * K / (ms / 1000.0)
+    if args.dump_outputs and rank == 0:
+        t = (args.preroll + W + K - 1) % ROLLOUT_T  # rollout slot of the last timed step
+        dump_outputs(args.dump_outputs, rollout[t], reward[t], done[t], info_sum)
 
     # ---- end to end through the host-buffer entry points (pinned memory, copies inside the timed region).  Double
     # buffered: step t+1 is submitted before the results of step t are fetched, so the 94 MB D2H of the observations

@@ -11,7 +11,6 @@ if str(ROOT) not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
 
 
 @pytest.fixture(scope="session")
@@ -53,12 +52,3 @@ def roms():
         return cache[name]
 
     return get
-
-
-REFERENCE = Path("/root/reference/pokegym")
-
-
-def reference_states():
-    if not REFERENCE.exists():
-        return []
-    return sorted(p for p in REFERENCE.rglob("*") if p.is_file() and p.stat().st_size == 142_610)

@@ -13,6 +13,7 @@
 """
 import hashlib
 import json
+import lzma
 import sys
 import zlib
 from pathlib import Path
@@ -97,7 +98,8 @@ def wrapper_sweep_golden(oracle_lib, n_steps=6):
         rec["obs_crc"].append([zlib.crc32(o.tobytes()) for o in ref["obs"]])
         rec["reset_obs_crc"].append(zlib.crc32(ref["reset_obs"][0].tobytes()))
         rec["state_sha"].append(np.frombuffer(hashlib.sha256(ref["states"][-1]).digest(), dtype=np.uint8))
-    np.savez_compressed(OUT / "ref_wrapper_sweep.npz", states=np.stack(rec["states"]), names=np.array(rec["names"]), actions=actions,
+    states_xz = np.frombuffer(lzma.compress(np.stack(rec["states"]).tobytes(), preset=9 | lzma.PRESET_EXTREME), dtype=np.uint8)  # helpers.load_wrapper_sweep
+    np.savez_compressed(OUT / "ref_wrapper_sweep.npz", states_xz=states_xz, names=np.array(rec["names"]), actions=actions,
                         rewards=np.array(rec["rewards"], dtype=np.float64), dones=np.array(rec["dones"], dtype=np.uint8),
                         obs_crc=np.array(rec["obs_crc"], dtype=np.uint32), reset_obs_crc=np.array(rec["reset_obs_crc"], dtype=np.uint32),
                         state_sha=np.stack(rec["state_sha"]), max_episode_steps=4)

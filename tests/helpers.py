@@ -1,6 +1,7 @@
 """Shared helpers for the parity tests."""
 import hashlib
 import json
+import lzma
 import zlib
 from pathlib import Path
 
@@ -64,6 +65,14 @@ def replay_wrapper_golden(handle, gold, xp=None, to_dev=lambda a: a, to_host=lam
             sha = np.frombuffer(hashlib.sha256(handle.save_state(0)).digest(), dtype=np.uint8)
             assert np.array_equal(sha, gold["state_sha"][i]), f"step {i}: emulator state differs (RAM side effects / emulation)"
     assert np.array_equal(to_host(obs).reshape(72, 80, 4), gold["last_obs"])
+
+
+def load_wrapper_sweep():
+    """ref_wrapper_sweep.npz with its 264 save-states unpacked.  They are stored as one xz stream (`states_xz`): the
+    reference's checkpoints share most of their bytes, which xz finds and the npz's deflate does not (0.25 MB vs 2.5 MB)."""
+    gold = dict(np.load(GOLDEN / "ref_wrapper_sweep.npz"))
+    gold["states"] = np.frombuffer(lzma.decompress(gold.pop("states_xz").tobytes()), dtype=np.uint8).reshape(len(gold["names"]), -1)
+    return gold
 
 
 def replay_wrapper_sweep(handle, gold, to_dev=lambda a: a, to_host=lambda a: a):

@@ -2,7 +2,7 @@
 import numpy as np
 import pytest
 
-from helpers import GOLDEN, check_ppu_kat, replay_wrapper_golden, replay_wrapper_sweep
+from helpers import GOLDEN, check_ppu_kat, load_wrapper_sweep, replay_wrapper_golden, replay_wrapper_sweep
 from pokegym_b200 import _capi
 
 
@@ -20,5 +20,5 @@ def test_oracle_renderer_matches_pyboy_framebuffers(oracle_lib, roms):
 
 
 def test_oracle_replays_reference_wrapper_on_all_264_states(oracle_lib, roms):
-    gold = np.load(GOLDEN / "ref_wrapper_sweep.npz")
+    gold = load_wrapper_sweep()
     replay_wrapper_sweep(_capi.Handle(oracle_lib, len(gold["names"]), roms("pokelike")), gold)

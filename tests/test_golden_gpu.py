@@ -3,7 +3,7 @@ PyBoy's own framebuffers (run on the B200 box; /root/reference does not exist th
 import numpy as np
 import pytest
 
-from helpers import GOLDEN, check_ppu_kat, replay_wrapper_golden, replay_wrapper_sweep
+from helpers import GOLDEN, check_ppu_kat, load_wrapper_sweep, replay_wrapper_golden, replay_wrapper_sweep
 from pokegym_b200 import _capi
 
 pytestmark = pytest.mark.gpu
@@ -30,6 +30,6 @@ def test_cuda_replays_reference_wrapper_on_all_264_states(cuda_lib, roms):
     produced."""
     import torch
 
-    gold = np.load(GOLDEN / "ref_wrapper_sweep.npz")
+    gold = load_wrapper_sweep()
     h = _capi.Handle(cuda_lib, len(gold["names"]), roms("pokelike"), 0)
     replay_wrapper_sweep(h, gold, to_dev=lambda a: torch.from_numpy(a).cuda(), to_host=lambda t: t.cpu().numpy())

@@ -1,151 +1,33 @@
-"""Tests that need the reference tree (/root/reference, build container only): they pin the oracle to
-what the reference itself holds -- its 264 PyBoy save-states and its own unmodified Python wrapper."""
-import numpy as np
-import pytest
-
-from conftest import REFERENCE, reference_states
+"""Pin the state codec and the oracle to what the reference itself holds: its 264 PyBoy v9 save-states, stored unmodified
+in tests/golden/ref_wrapper_sweep.npz (helpers.load_wrapper_sweep) and named by their path in the reference tree."""
+from helpers import load_wrapper_sweep
 from pokegym_b200 import _capi
-from pokegym_b200.info import build_info
 from pokegym_b200.state_file import diff_states, parse_state, serialize_state
 
-pytestmark = [pytest.mark.reference, pytest.mark.skipif(not REFERENCE.exists(), reason="reference tree not mounted")]
+
+def _fixtures():
+    gold = load_wrapper_sweep()
+    return [(str(name), state.tobytes()) for name, state in zip(gold["names"], gold["states"])]
 
 
 def test_state_codec_round_trips_every_fixture():
-    files = [p for p in REFERENCE.rglob("*") if p.is_file() and p.stat().st_size in (142_610, 142_586)]
-    assert len(files) == 265
-    for p in files:
-        blob = p.read_bytes()
-        assert serialize_state(parse_state(blob)) == blob, p
+    fixtures = _fixtures()
+    assert len(fixtures) == 264
+    for name, blob in fixtures:
+        assert serialize_state(parse_state(blob)) == blob, name
 
 
 def test_oracle_load_save_and_renderer_on_all_v9_fixtures(oracle_lib, roms):
     """gb_load_state/gb_save_state are byte-exact (except STAT's read-only low bits, a PyBoy load quirk) and the
     scanline renderer reproduces, bit for bit, the framebuffer PyBoy stored in each of the 264 save-states."""
     h = _capi.Handle(oracle_lib, 1, roms("pokelike"))
-    files = reference_states()
-    assert len(files) == 264
-    for p in files:
-        blob = p.read_bytes()
+    fixtures = _fixtures()
+    assert len(fixtures) == 264
+    for name, blob in fixtures:
         tid = h.add_state_template(blob)
         h.load_template(tid)
         d = diff_states(blob, h.save_state(0))
-        assert d in ([], ["lcd_regs: 1 bytes differ (+4:81!=80)"]), (p, d)
+        assert d in ([], ["lcd_regs: 1 bytes differ (+4:81!=80)"]), (name, d)
         expected = parse_state(blob).raw["screen"].tobytes()
         h.debug_render_frame(0)
-        assert parse_state(h.save_state(0)).raw["screen"].tobytes() == expected, f"{p}: rendered frame differs from PyBoy's"
-
-
-def test_v7_state_loads(oracle_lib, roms):
-    p = REFERENCE / "unused_states" / "has_pokedex_nballs_backup.state"
-    h = _capi.Handle(oracle_lib, 1, roms("pokelike"))
-    tid = h.add_state_template(p.read_bytes())
-    h.load_template(tid)
-    st = parse_state(h.save_state(0))
-    assert st.cpu["PC"] == parse_state(p.read_bytes()).cpu["PC"]
-
-
-def _assert_info_equal(ref, mine, path="info"):
-    """Recursive comparison of the reference's info dict with build_info's (same keys, same order, same numbers)."""
-    if isinstance(ref, dict):
-        assert isinstance(mine, dict) and list(ref) == list(mine), (path, list(ref), list(mine) if isinstance(mine, dict) else mine)
-        for k in ref:
-            _assert_info_equal(ref[k], mine[k], f"{path}[{k!r}]")
-    elif isinstance(ref, set):  # stats["maps_explored"]: the reference's later duplicate key stores np.sum(set) == the set itself
-        assert len(ref) == mine, (path, ref, mine)
-    elif isinstance(ref, np.ndarray) and ref.ndim:
-        assert np.array_equal(ref, np.asarray(mine)), path
-    elif isinstance(ref, (list, tuple)):
-        assert [float(x) for x in ref] == [float(x) for x in mine], (path, ref, mine)
-    else:
-        assert abs(float(ref) - float(mine)) <= 1e-9 * max(1.0, abs(float(ref))), (path, ref, mine)
-
-
-def _compare_with_reference(oracle_lib, rom, start_blob, actions, max_episode_steps, reset_at):
-    import ref_shim
-
-    ref = ref_shim.run_reference_episode(rom, oracle_lib, start_blob, actions, max_episode_steps=max_episode_steps, reset_at=reset_at)
-    o = _capi.Handle(oracle_lib, 1, rom)
-    o.set_initial_template(o.add_state_template(start_blob))
-    obs = np.zeros((1, _capi.OBS_BYTES), np.uint8)
-    rew = np.zeros(1)
-    done = np.zeros(1, np.uint8)
-    o.reset(obs, max_episode_steps=max_episode_steps)
-    assert np.array_equal(obs.reshape(72, 80, 4), ref["reset_obs"][0])
-    assert o.save_state(0) == ref["reset_state"][0]
-    k = 1
-    n_infos = 0
-    for i, a in enumerate(actions):
-        if i in reset_at:
-            o.reset(obs, max_episode_steps=max_episode_steps)
-            assert np.array_equal(obs.reshape(72, 80, 4), ref["reset_obs"][k])
-            assert o.save_state(0) == ref["reset_state"][k], diff_states(ref["reset_state"][k], o.save_state(0))
-            k += 1
-        o.step(np.array([a], np.uint8), obs, rew, done)
-        assert rew[0] == ref["rewards"][i], (i, rew[0], ref["rewards"][i])
-        assert bool(done[0]) == ref["dones"][i]
-        assert np.array_equal(obs.reshape(72, 80, 4), ref["obs"][i]), i
-        assert o.save_state(0) == ref["states"][i], (i, diff_states(ref["states"][i], o.save_state(0)))
-        if ref["infos"][i]:  # emitted when done or time % 10000 == 0 (environment.py:1620)
-            row = np.zeros((1, _capi.INFO_SCALARS))
-            o.get_info(row)
-            mine = build_info(row[0], lambda a: int(o.read_mem(0, a, 1)[0]), counts_map=o.counts_map(0))
-            _assert_info_equal(ref["infos"][i], mine)
-            n_infos += 1
-    assert n_infos == sum(1 for x in ref["infos"] if x)
-    return ref, o, n_infos
-
-
-def test_wrapper_matches_unmodified_reference_on_synthetic_game(oracle_lib, roms):
-    rom = roms("pokelike")
-    h = _capi.Handle(oracle_lib, 1, rom)
-    h.tick(60, True)
-    actions = np.random.default_rng(3).integers(0, 8, 500)
-    ref, o, n_infos = _compare_with_reference(oracle_lib, rom, h.save_state(0), actions, 200, (200, 400))
-    assert np.count_nonzero(ref["rewards"]) > 20
-    assert n_infos >= 2, "the info dict the reference emits at `done` was not compared"
-
-
-@pytest.mark.parametrize("rel", ["current_state/Bulbasaur.state", "bin/checkpoints_battles/bulbasaur/pokemon_ai_14", "bin/checkpoints_bill/pokemon_ai_1005",
-                                 "bin/checkpoints_pallet/pokemon_ai_105", "unused_states/bill.state"])
-def test_wrapper_matches_reference_from_real_save_states(oracle_lib, roms, rel):
-    """Real Pokemon Red RAM (party, events, bag, battle / menu state) + the state-compatible synthetic ROM."""
-    p = REFERENCE / rel
-    if not p.exists():
-        cands = sorted((REFERENCE / rel).parent.glob("*"))
-        p = cands[len(cands) // 2]
-    actions = np.random.default_rng(7).integers(0, 8, 60)
-    _, _, n_infos = _compare_with_reference(oracle_lib, roms("pokelike"), p.read_bytes(), actions, 40, (45,))
-    assert n_infos >= 1
-
-
-def test_static_tables_match_reference_modules(oracle_lib):
-    """The hand-restated tables (cursor keys, event bits, tree list) against the reference's own objects."""
-    import ref_shim
-
-    ref_shim.reference_environment_class()
-    import pokegym.environment as E
-    import pokegym.ram_map_leanke as L
-    from pokegym.bin.ram_reader import red_memory_menus as M
-
-    keys = sorted(M.TEXT_MENU_CURSOR_LOCATIONS.keys())
-    src = (REFERENCE.parent.parent / "repo" / "pokegym_b200" / "csrc" / "gb_wrap.cuh").read_text()
-    import re
-
-    block = src[src.index("c_cursor_keys[48]") :]
-    vals = [int(x, 16) for x in re.findall(r"0x([0-9A-Fa-f]{4})", block[: block.index("};")])]
-    assert sorted(vals) == sorted(a | (b << 8) for a, b in keys) and len(vals) == 48
-
-    class G:  # every bit set -> each monitor returns its weights
-        def get_memory_value(self, a):
-            return 0xFF
-
-    groups = [L.monitor_silph_co_events, L.monitor_dojo_events, L.monitor_hideout_events, L.monitor_poke_tower_events, L.monitor_gym3_events,
-              L.monitor_gym4_events, L.monitor_gym5_events, L.monitor_gym6_events, L.monitor_gym7_events]
-    weights = [list(f(G()).values()) for f in groups]
-    ev = src[src.index("c_events[] = {") : src.index("#undef EV")]
-    mine = [int(w) for w in re.findall(r"EV\(0x[0-9A-F]{4}, \d, (-?\d)\)", ev)]
-    assert mine == [w for g in weights for w in g]
-    assert [len(g) for g in weights] == [53, 8, 15, 17, 6, 8, 7, 8, 8]
-    trees = [tuple(int(v) for v in t) for t in re.findall(r"\{(\d+), (\d+), (\d+)\}", src[src.index("c_trees[19][3]") : src.index("c_cursor_keys")])]
-    assert trees == [tuple(t) for t in E.TREE_POSITIONS_PIXELS]
+        assert parse_state(h.save_state(0)).raw["screen"].tobytes() == expected, f"{name}: rendered frame differs from PyBoy's"
