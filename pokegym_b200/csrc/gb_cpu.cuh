@@ -478,18 +478,25 @@ __device__ __forceinline__ bool cpu_exec(Machine &m, const uint4 d, CpuRegs &r, 
 }
 
 // Single-lane build: dispatch on the class id of the control word to an instance of the body in which handler and operand
-// flags are constants.  One indexed branch replaces the ~10 flag tests + branches the generic body spends per instruction
-// (12.3 BRA and 17.7 LOP3 of its 68 SASS instructions per emulated one); nothing diverges in a single-thread block, so
-// the code-size price (34 short bodies) is the only one.
+// flags are constants.  This replaces the ~10 flag tests + branches the generic body spends per instruction (12.3 BRA and
+// 17.7 LOP3 of its 68 SASS instructions per emulated one); nothing diverges in a single-thread block, so the code-size price
+// (34 short bodies) is the only one.  nvcc lowers a switch to a balanced compare tree (five tests for every class, hot or
+// cold), so the dispatch is the tree gb_classes.inc spells out as explicit tests, shaped by the class mix of the benchmark
+// workloads (tools/class_mix.py): the hottest class takes two tests, 3.6 per instruction on average.  Each test sees
+// the class id through an empty asm, so that nvcc cannot merge the tests back into a switch.
+__device__ __forceinline__ void gb_opaque(uint32_t &v) {  // the compiler no longer knows v's value (it is unchanged)
+#if !defined(GB_HOSTSIM)
+    asm volatile("" : "+r"(v));
+#endif
+}
 __device__ __forceinline__ bool cpu_exec_by_class(Machine &m, const uint4 d, CpuRegs &r, uint32_t &rom_off, uint32_t &mode, uint32_t &cyc, uint8_t *memb,
                                                   const uint8_t *rom, uint32_t bank_mask) {
-    switch (PD_CLASS(d.w)) {
-#define GB_CLS(id, H, F) \
-    case id: return cpu_exec<true, false, H, F>(m, d, r, rom_off, mode, cyc, memb, rom, bank_mask);
-#include "gb_classes.inc"
-#undef GB_CLS
-    default: return false;  // rare opcodes, on-the-fly decode: the slow tick
-    }
+    uint32_t c = PD_CLASS(d.w);
+#define GB_CLS_TEST(t) (gb_opaque(c), (t))
+#define GB_CLS_RUN(id, H, F) return cpu_exec<true, false, H, F>(m, d, r, rom_off, mode, cyc, memb, rom, bank_mask);
+    GB_CLS_DISPATCH(c, GB_CLS_RUN, return false;)  // rare opcodes, on-the-fly decode: the slow tick
+#undef GB_CLS_RUN
+#undef GB_CLS_TEST
 }
 
 // The fast body of the lock-step build (k_run_frames, several envs per warp) as ONE straight line of code: no handler
