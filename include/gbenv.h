@@ -32,7 +32,8 @@
 extern "C" {
 #endif
 
-#define GBENV_ABI_VERSION 3 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked */
+#define GBENV_ABI_VERSION 4 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
+                               4: gbenv_counts_map_sum, gbenv_reduce_info_masked */
 
 #define GBENV_STATE_BYTES 142610 /* PyBoy v9 save-state length (SURVEY.md 8c)              */
 #define GBENV_OBS_H 72           /* environment.py:154-166: (144//2, 160//2, 4) uint8       */
@@ -107,7 +108,11 @@ int gbenv_screen(gbenv_t *h, int env, uint8_t *rgb_host);
 /* ---- (3) Environment.reset / step with fused reward + observation ---------------------------
  * gbenv_reset == Environment.reset (environment.py:1233-1334) for envs with mask[e] != 0
  * (mask_host == NULL: all).  obs_dev: uint8[n_envs][obs_stride] (obs_stride >= GBENV_OBS_BYTES),
- * only rows of reset envs are written.                                                          */
+ * only rows of reset envs are written.
+ * Guarantee of every gbenv_reset* call: an env's info row (gbenv_get_info) is left as its last step wrote it, and its heat
+ * map keeps accumulating (it lives as long as the env).  So after an auto-reset on the `done` of a step, the info rows of
+ * the envs that just finished are still there for gbenv_reduce_info_masked(mask = that done).  The CPU oracle differs
+ * here: its reset zeroes the row (DESIGN.md section 2).                                         */
 int gbenv_reset(gbenv_t *h, const uint8_t *mask_host, int max_episode_steps, double reward_scale,
                 uint8_t *obs_dev, size_t obs_stride, void *stream);
 /* The same with a DEVICE mask (e.g. the `done` vector gbenv_step just wrote): nothing touches the host, so a vectoriser
@@ -144,11 +149,21 @@ int gbenv_fetch_host(gbenv_t *h);
 int gbenv_get_info(gbenv_t *h, double *info_dev, void *stream);
 /* Sum of the info rows over envs (+ env count in slot 0): the vector ranks all-reduce over NCCL. */
 int gbenv_reduce_info(gbenv_t *h, double *sum_dev /* GBENV_INFO_SCALARS */, void *stream);
-/* `pokemon_exploration_map` (environment.py:448,648-679,1624): int32[444*436] of one env.  Stored dense
- * (774 KB per env) while all maps fit in 4 GiB, otherwise as a per-env hash of the cells the env has touched
- * (2 GiB budget; env GBENV_COUNTS_MAP=dense|sparse|0, GBENV_COUNTS_SLOTS=<power of two>), from which this call
- * rebuilds the dense image.  A full hash stops tracking new cells and is reported through counters.faults.   */
+/* gbenv_reduce_info over the envs with mask_dev[e] != 0 only (mask_dev NULL: all envs, bit-identical to gbenv_reduce_info);
+ * slot 0 = number of those envs that have stepped at least once.  The mean a trainer logs when episodes end is this sum
+ * with mask = the `done` of the step, divided by slot 0.  Asynchronous on `stream`.                                 */
+int gbenv_reduce_info_masked(gbenv_t *h, const uint8_t *mask_dev, double *sum_dev /* GBENV_INFO_SCALARS */, void *stream);
+/* `pokemon_exploration_map` (environment.py:448,648-679,1624): int32[444*436] of one env, synchronous.  Heat maps are
+ * paged (DESIGN.md section 3): per env a directory of 28 x 28 blocks of 16 x 16 cells, blocks taken from a pool shared by
+ * all envs on first touch; this call rebuilds the dense image.  GBENV_COUNTS_MAP=0 switches heat maps off (this call then
+ * fails with GBENV_E_ARG); GBENV_COUNTS_BLOCKS sizes the pool, and a pool that runs dry is reported by gbenv_check.  */
 int gbenv_counts_map(gbenv_t *h, int env, int32_t *map_host);
+/* Sum of the heat maps of the envs with mask_dev[e] != 0 (mask_dev NULL: all envs) into sum_dev int64[444*436], which is
+ * overwritten: each cell is the plain integer sum of that cell over those envs' maps, -1 marks included (the reference
+ * trainer's exploration overlay sums the `pokemon_exploration_map`s of the envs that finished, environment.py:1624).
+ * Asynchronous on `stream`, ordered after earlier calls on the handle.  GBENV_E_ARG when heat maps are switched off;
+ * GBENV_E_NOMEM once an exhausted pool has been reported (as gbenv_step), since the maps are then incomplete.        */
+int gbenv_counts_map_sum(gbenv_t *h, const uint8_t *mask_dev, int64_t *sum_dev /* 444*436 */, void *stream);
 
 /* ---- diagnostics ----------------------------------------------------------------------------*/
 typedef struct gbenv_counters {

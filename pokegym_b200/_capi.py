@@ -18,7 +18,8 @@ STATE_BYTES = 142_610
 OBS_H, OBS_W, OBS_C = 72, 80, 4
 OBS_BYTES = OBS_H * OBS_W * OBS_C
 INFO_SCALARS = 72
-ABI_VERSION = 3
+ABI_VERSION = 4
+COUNTS_H, COUNTS_W = 444, 436
 NUM_ACTIONS = 8
 ACT_FREQ = 24
 
@@ -86,7 +87,9 @@ _SIGS = {
     "reset_host": ([C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_void_p], C.c_int),
     "get_info": ([C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
     "reduce_info": ([C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
+    "reduce_info_masked": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
     "counts_map": ([C.c_void_p, C.c_int, C.c_void_p], C.c_int),
+    "counts_map_sum": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
     "get_counters": ([C.c_void_p, C.POINTER(Counters)], C.c_int),
     "last_kernel_ms": ([C.c_void_p, C.c_int, C.POINTER(C.c_float)], C.c_int),
     "kernel_time_total": ([C.c_void_p, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_uint64)], C.c_int),
@@ -244,10 +247,18 @@ class Handle:
     def reduce_info(self, out, stream: int = 0):
         self._check(self.lib.reduce_info(self._h, _ptr(out), C.c_void_p(stream)), "reduce_info")
 
+    def reduce_info_masked(self, out, mask_dev=None, stream: int = 0):
+        """reduce_info over the envs whose mask byte is non-zero (None: all); slot 0 = how many of them have stepped."""
+        self._check(self.lib.reduce_info_masked(self._h, _ptr(mask_dev), _ptr(out), C.c_void_p(stream)), "reduce_info_masked")
+
     def counts_map(self, env: int) -> np.ndarray:
-        out = np.empty((444, 436), dtype=np.int32)
+        out = np.empty((COUNTS_H, COUNTS_W), dtype=np.int32)
         self._check(self.lib.counts_map(self._h, int(env), _ptr(out)), "counts_map")
         return out
+
+    def counts_map_sum(self, out, mask_dev=None, stream: int = 0):
+        """int64 [444, 436] sum of the heat maps of the envs whose mask byte is non-zero (None: all) -> out (overwritten)."""
+        self._check(self.lib.counts_map_sum(self._h, _ptr(mask_dev), _ptr(out), C.c_void_p(stream)), "counts_map_sum")
 
     # -- diagnostics ---------------------------------------------------------
     def sync(self):

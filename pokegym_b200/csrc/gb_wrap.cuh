@@ -647,6 +647,62 @@ __global__ void __launch_bounds__(CM_BLOCK * CM_BLOCK) k_cm_gather(WrapArrays w,
     dense[y * COUNTS_W + x] = b ? w.cm_pool[(size_t)(b - 1) * (CM_BLOCK * CM_BLOCK) + threadIdx.x] : 0;
 }
 
+// gbenv_counts_map_sum: sum[cell] += the cell over the heat maps of the envs [chunk * chunk_envs, +chunk_envs) with mask[e] != 0
+// (mask null: all).  grid (CM_DIR_ENTRIES, chunks), CM_SUM_THREADS threads; sum is zeroed beforehand on the same stream.
+// Envs that start from one save-state walk the same cells, so a per-(env, cell) atomic would pile onto a few addresses.  Instead
+// each warp takes CM_SUM_GROUP envs at a time: a lane reads the directory entries and mask bytes of CM_SUM_GROUP / 32 envs (all
+// loads in flight together), a ballot per 32 envs names the lanes with a present, masked block, and the warp then reads those
+// blocks whole (1 KiB, two 16-byte loads per lane) into 8 int64 partial sums per lane (cells 4l..4l+3 and 128+4l..128+4l+3).
+// The warps' partials meet in shared memory; each cell then takes one 64-bit atomicAdd per block.  Integer sums: the result
+// does not depend on the order in which blocks run.
+#define CM_SUM_THREADS 256
+#define CM_SUM_GROUP 128
+__global__ void __launch_bounds__(CM_SUM_THREADS) k_cm_sum(WrapArrays w, const uint8_t *mask, int n_envs, int chunk_envs, long long *sum) {
+    __shared__ long long s_part[CM_SUM_THREADS / 32][CM_BLOCK * CM_BLOCK];
+    const int entry = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int e_begin = blockIdx.y * chunk_envs, e_end = min(n_envs, e_begin + chunk_envs);
+    long long acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    for (int base = e_begin + warp * CM_SUM_GROUP; base < e_end; base += CM_SUM_GROUP * (CM_SUM_THREADS / 32)) {
+        uint32_t dir[CM_SUM_GROUP / 32];
+#pragma unroll
+        for (int u = 0; u < CM_SUM_GROUP / 32; u++) {
+            const int e = base + u * 32 + lane;
+            dir[u] = (e < e_end && (!mask || mask[e])) ? w.cm_dir[(size_t)e * CM_DIR_ENTRIES + entry] : 0u;
+        }
+#pragma unroll
+        for (int u = 0; u < CM_SUM_GROUP / 32; u++) {
+            uint32_t bits = __ballot_sync(0xFFFFFFFFu, dir[u] != 0);
+            while (bits) {  // two blocks per pass, so that four 16-byte loads per lane are in flight
+                const int l0 = __ffs(bits) - 1;
+                bits &= bits - 1;
+                const int l1 = bits ? __ffs(bits) - 1 : l0;
+                const bool two = bits != 0;
+                bits &= bits - 1;
+                const uint32_t b0 = __shfl_sync(0xFFFFFFFFu, dir[u], l0), b1 = __shfl_sync(0xFFFFFFFFu, dir[u], l1);
+                const int4 *p0 = (const int4 *)(w.cm_pool + (size_t)(b0 - 1) * (CM_BLOCK * CM_BLOCK)) + lane;
+                const int4 *p1 = (const int4 *)(w.cm_pool + (size_t)(b1 - 1) * (CM_BLOCK * CM_BLOCK)) + lane;
+                const int4 a0 = p0[0], a1 = p0[32];
+                int4 c0 = make_int4(0, 0, 0, 0), c1 = c0;
+                if (two) { c0 = p1[0]; c1 = p1[32]; }
+                acc[0] += (long long)a0.x + c0.x; acc[1] += (long long)a0.y + c0.y; acc[2] += (long long)a0.z + c0.z; acc[3] += (long long)a0.w + c0.w;
+                acc[4] += (long long)a1.x + c1.x; acc[5] += (long long)a1.y + c1.y; acc[6] += (long long)a1.z + c1.z; acc[7] += (long long)a1.w + c1.w;
+            }
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        s_part[warp][4 * lane + k] = acc[k];
+        s_part[warp][128 + 4 * lane + k] = acc[4 + k];
+    }
+    __syncthreads();
+    const int cell = threadIdx.x, by = entry / CM_BLOCKS_X, bx = entry % CM_BLOCKS_X;
+    const int y = by * CM_BLOCK + cell / CM_BLOCK, x = bx * CM_BLOCK + cell % CM_BLOCK;
+    long long t = 0;
+#pragma unroll
+    for (int k = 0; k < CM_SUM_THREADS / 32; k++) t += s_part[k][cell];
+    if (t != 0 && y < COUNTS_H && x < COUNTS_W) atomicAdd((unsigned long long *)&sum[y * COUNTS_W + x], (unsigned long long)t);
+}
+
 // Observation assembly: block = one 32-env tile, 256 threads.  For each of the 72 output rows the block
 // loads the even framebuffer line (10 words x 32 lanes, coalesced), then writes 32 x 80 RGBA-like pixels
 // as 32-bit words: [grey, grey, grey, visited] (environment.py:266-272, :233-254).
@@ -709,12 +765,14 @@ __global__ void __launch_bounds__(256) k_wrap_obs(DevArrays d, WrapArrays w, con
     }
 }
 
-// sum of the info rows over envs -> GBENV_INFO_SCALARS doubles (the vector multi-GPU runs all-reduce over NCCL)
-__global__ void k_reduce_info(const double *rows, int n_envs, double *sum) {
+// sum of the info rows over the envs with mask[e] != 0 (mask null: all) -> GBENV_INFO_SCALARS doubles (the vector multi-GPU
+// runs all-reduce over NCCL).  A masked-out row is skipped, so the unmasked envs are added in the same order as without a mask.
+__global__ void k_reduce_info(const double *rows, const uint8_t *mask, int n_envs, double *sum) {
     __shared__ double s[256];
     const int k = blockIdx.x;  // one block per info slot
     double acc = 0.0;
-    for (int e = threadIdx.x; e < n_envs; e += blockDim.x) acc += rows[(size_t)e * GBENV_INFO_SCALARS + k];
+    for (int e = threadIdx.x; e < n_envs; e += blockDim.x)
+        if (!mask || mask[e]) acc += rows[(size_t)e * GBENV_INFO_SCALARS + k];
     s[threadIdx.x] = acc;
     __syncthreads();
     for (int st = blockDim.x / 2; st > 0; st >>= 1) {

@@ -60,6 +60,7 @@ struct gbenv {
     size_t smem_opted = 48 * 1024;
     int32_t *pool_err_host = nullptr;  // pinned copy of WrapArrays.ctl[CTL_ERROR], refreshed asynchronously after every step / reset
     int32_t *d_cm_dense = nullptr;     // staging for gbenv_counts_map
+    int cm_sum_chunk = 0;              // envs per block row of k_cm_sum (0 = not chosen yet)
     std::string err;
 };
 
@@ -716,10 +717,39 @@ extern "C" int gbenv_get_info(gbenv *h, double *info_dev, void *stream) {
     return GBENV_OK;
 }
 
-extern "C" int gbenv_reduce_info(gbenv *h, double *sum_dev, void *stream) {
+extern "C" int gbenv_reduce_info_masked(gbenv *h, const uint8_t *mask_dev, double *sum_dev, void *stream) {
     if (!h || !sum_dev) return fail(h, GBENV_E_ARG, "gbenv_reduce_info: bad argument");
     CK(cudaSetDevice(h->device));
-    k_reduce_info<<<GBENV_INFO_SCALARS, 256, 0, pick(h, stream)>>>(h->d_info_rows, h->n, sum_dev);
+    k_reduce_info<<<GBENV_INFO_SCALARS, 256, 0, pick(h, stream)>>>(h->d_info_rows, mask_dev, h->n, sum_dev);
+    h->launches++;
+    CK(cudaGetLastError());
+    return GBENV_OK;
+}
+
+extern "C" int gbenv_reduce_info(gbenv *h, double *sum_dev, void *stream) { return gbenv_reduce_info_masked(h, nullptr, sum_dev, stream); }
+
+static const char *const CM_DISABLED = "gbenv_counts_map: exploration map tracking is disabled (GBENV_COUNTS_MAP=0)";
+
+extern "C" int gbenv_counts_map_sum(gbenv *h, const uint8_t *mask_dev, int64_t *sum_dev, void *stream) {
+    if (!h || !sum_dev) return fail(h, GBENV_E_ARG, "gbenv_counts_map_sum: bad argument");
+    if (!h->w.cm_dir) return fail(h, GBENV_E_ARG, CM_DISABLED);
+    CK(cudaSetDevice(h->device));
+    int rc = pool_error(h);  // a sum over maps that stopped being tracked would look valid
+    if (rc) return rc;
+    if (!h->cm_sum_chunk) {
+        // env chunks: enough blocks for four waves of the GPU, but at least 1,024 envs per chunk so that a block's reads of
+        // the maps outweigh its 256 atomics into the sum
+        int sms = 148, per_sm = 1;
+        CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device));
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_cm_sum, CM_SUM_THREADS, 0));
+        const int wanted = (4 * sms * per_sm + CM_DIR_ENTRIES - 1) / CM_DIR_ENTRIES, most = (h->n + 1023) / 1024;
+        const int chunks = wanted < most ? (wanted > 1 ? wanted : 1) : most;
+        h->cm_sum_chunk = ((h->n + chunks - 1) / chunks + CM_SUM_GROUP - 1) / CM_SUM_GROUP * CM_SUM_GROUP;
+    }
+    cudaStream_t st = pick(h, stream);
+    CK(cudaMemsetAsync(sum_dev, 0, (size_t)COUNTS_H * COUNTS_W * sizeof(int64_t), st));
+    const dim3 grid(CM_DIR_ENTRIES, (h->n + h->cm_sum_chunk - 1) / h->cm_sum_chunk);
+    k_cm_sum<<<grid, CM_SUM_THREADS, 0, st>>>(h->w, mask_dev, h->n, h->cm_sum_chunk, (long long *)sum_dev);
     h->launches++;
     CK(cudaGetLastError());
     return GBENV_OK;
@@ -727,7 +757,7 @@ extern "C" int gbenv_reduce_info(gbenv *h, double *sum_dev, void *stream) {
 
 extern "C" int gbenv_counts_map(gbenv *h, int env, int32_t *map_host) {
     if (!h || env < 0 || env >= h->n || !map_host) return fail(h, GBENV_E_ARG, "gbenv_counts_map: bad argument");
-    if (!h->w.cm_dir) return fail(h, GBENV_E_ARG, "gbenv_counts_map: exploration map tracking is disabled (GBENV_COUNTS_MAP=0)");
+    if (!h->w.cm_dir) return fail(h, GBENV_E_ARG, CM_DISABLED);
     CK(cudaSetDevice(h->device));
     cudaStream_t st = own(h);  // ordered after whatever was last queued on this handle, on any stream
     if (!h->d_cm_dense) CK(cudaMalloc((void **)&h->d_cm_dense, (size_t)COUNTS_H * COUNTS_W * sizeof(int32_t)));

@@ -1,8 +1,9 @@
 """Multi-GPU plumbing: envs shard across ranks with no data-path collective (SURVEY.md section 8e).
 
 One process per GPU (torchrun); rank r owns a contiguous slice of the global env index range; the only
-exchange is a sum all-reduce of the 72-double episode-info vector, once per rollout, over NCCL on GPUs
-(gloo in the CPU tests).  Timing of multi-rank runs is the max over ranks.
+exchange is a sum all-reduce of the 72-double episode-info vector (and, when a trainer logs it, of the int64
+exploration-map sum), once per rollout, over NCCL on GPUs (gloo in the CPU tests).  Timing of multi-rank runs is
+the max over ranks.
 """
 from __future__ import annotations
 
@@ -19,7 +20,10 @@ def shard_range(n_total: int, rank: int, world: int) -> Tuple[int, int]:
 
 
 def all_reduce_info(info_sum, group=None):
-    """In-place sum of the per-rank info vectors (slot 0 = env count).  No-op without a process group."""
+    """In-place sum of the per-rank info vectors (slot 0 = env count).  No-op without a process group.
+
+    Any dtype: the int64 [444, 436] exploration-map sum (VecEnvironment.exploration_map_sum) goes through the same call,
+    1.5 MB per all-reduce, and stays exact."""
     import torch.distributed as dist
 
     if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:

@@ -20,6 +20,7 @@ from __future__ import annotations
 from typing import List, Optional
 
 from . import _capi
+from .vec_env import device_mask
 
 
 class EnvGroups:
@@ -37,6 +38,7 @@ class EnvGroups:
             self._ready = [torch.cuda.Event() for _ in range(n_groups)]
             self._done = [torch.cuda.Event() for _ in range(n_groups)]
             self._info_parts = torch.zeros((n_groups, _capi.INFO_SCALARS), dtype=torch.float64, device=self.device)
+        self._map_parts = None  # [n_groups, 444, 436] int64, allocated by the first exploration_map_sum
         if lanes:
             for h in self.handles:
                 h.set_lanes_per_warp(lanes)
@@ -85,12 +87,28 @@ class EnvGroups:
         if join:
             self.join()
 
-    def reduce_info(self, out):
-        """sum of the 72-double info rows over every env of every group -> out (on the caller's stream, after a join)"""
+    def reduce_info(self, out, mask=None):
+        """sum of the 72-double info rows over every env of every group -> out (on the caller's stream, after a join); with
+        `mask` (u8 / bool [E], e.g. the step's done) over the envs with mask[e] != 0 only"""
+        mask = device_mask(mask, self.num_envs, self.device, "reduce_info")
+        self._fork()
         for g, (h, s) in enumerate(zip(self.handles, self.streams)):
-            h.reduce_info(self._info_parts[g], stream=s.cuda_stream)
+            h.reduce_info_masked(self._info_parts[g], self._slice(mask, g), stream=s.cuda_stream)
         self.join()
         self.torch.sum(self._info_parts, dim=0, out=out)
+        return out
+
+    def exploration_map_sum(self, out, mask=None):
+        """int64 [444, 436] sum of the heat maps of every env (or those with mask[e] != 0) of every group -> out (on the
+        caller's stream, after a join)"""
+        mask = device_mask(mask, self.num_envs, self.device, "exploration_map_sum")
+        if self._map_parts is None:
+            self._map_parts = self.torch.empty((self.n_groups, _capi.COUNTS_H, _capi.COUNTS_W), dtype=self.torch.int64, device=self.device)
+        self._fork()
+        for g, (h, s) in enumerate(zip(self.handles, self.streams)):
+            h.counts_map_sum(self._map_parts[g], self._slice(mask, g), stream=s.cuda_stream)
+        self.join()
+        self.torch.sum(self._map_parts, dim=0, out=out)
         return out
 
     # -- counters --------------------------------------------------------------------------------------------------

@@ -94,6 +94,24 @@ def _read_rom(rom_path: Union[str, os.PathLike, bytes]) -> bytes:
     )
 
 
+def device_mask(mask, n: int, device, what: str = "mask"):
+    """An env mask as the library reads it: a contiguous uint8 tensor of n entries on `device`, or None for all envs.
+    Accepts a bool / integer tensor (e.g. the `done` of a step, which then stays on the device) or an array-like."""
+    if mask is None:
+        return None
+    import torch
+
+    if not torch.is_tensor(mask):
+        mask = torch.as_tensor(np.ascontiguousarray(mask, dtype=np.uint8), device=device)
+    if mask.dtype == torch.bool:
+        mask = mask.to(torch.uint8)
+    if mask.dtype != torch.uint8 or mask.device != device or not mask.is_contiguous() or mask.numel() != n:
+        mask = mask.to(device=device, dtype=torch.uint8).contiguous().view(-1)
+        if mask.numel() != n:
+            raise ValueError(f"{what} mask must have {n} entries")
+    return mask
+
+
 class VecEnvironment:
     """N Game Boy envs on one GPU.  All tensors live on `device`; nothing returns to the host per step.
 
@@ -161,16 +179,7 @@ class VecEnvironment:
         if reward_scale is not None:
             self.reward_scale = float(reward_scale)
         obs = self._obs_target()
-        torch = self.torch
-        if mask is not None and not torch.is_tensor(mask):
-            mask = torch.as_tensor(np.ascontiguousarray(mask, dtype=np.uint8), device=self.device)
-        if mask is not None:  # a device mask (e.g. the done vector): the reset stays on the device, no host round trip
-            if mask.dtype == torch.bool:
-                mask = mask.to(torch.uint8)
-            if mask.dtype != torch.uint8 or mask.device != self.device or not mask.is_contiguous() or mask.numel() != self.num_envs:
-                mask = mask.to(device=self.device, dtype=torch.uint8).contiguous().view(-1)
-                if mask.numel() != self.num_envs:
-                    raise ValueError(f"reset mask must have {self.num_envs} entries")
+        mask = device_mask(mask, self.num_envs, self.device, "reset")
         self.handle.reset_dev(obs, mask_dev=mask, max_episode_steps=self.max_episode_steps, reward_scale=self.reward_scale,
                               obs_stride=_capi.OBS_BYTES, stream=self._stream())
         return obs.view(self.num_envs, *OBS_SHAPE), {}
@@ -219,12 +228,29 @@ class VecEnvironment:
         self.handle.get_info(self._info, stream=self._stream())
         return self._info
 
-    def info_sum(self, out=None):
-        """Sum of the info rows over this GPU's envs (the vector multi-GPU runs all-reduce)."""
+    def info_sum(self, out=None, mask=None):
+        """Sum of the info rows over this GPU's envs (the vector multi-GPU runs all-reduce); slot 0 counts the envs summed.
+        With `mask` (e.g. the `done` that step() returned), only the envs with mask[e] != 0: their rows are those of their
+        last step even after auto_reset, so this is the sum a trainer averages over the episodes that just ended."""
         torch = self.torch
         if out is None:
             out = torch.zeros(_capi.INFO_SCALARS, dtype=torch.float64, device=self.device)
-        self.handle.reduce_info(out, stream=self._stream())
+        if mask is None:
+            self.handle.reduce_info(out, stream=self._stream())
+        else:
+            self.handle.reduce_info_masked(out, device_mask(mask, self.num_envs, self.device, "info_sum"), stream=self._stream())
+        return out
+
+    def exploration_map_sum(self, mask=None, out=None):
+        """int64 [444, 436] device tensor: the sum of the envs' `pokemon_exploration_map`s (environment.py:1624), over the
+        envs with mask[e] != 0 (e.g. the `done` of step()) or over all.  Computed on the device, nothing goes to the host."""
+        torch = self.torch
+        shape = (_capi.COUNTS_H, _capi.COUNTS_W)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.int64, device=self.device)
+        elif not (torch.is_tensor(out) and out.dtype == torch.int64 and out.device == self.device and out.is_contiguous() and tuple(out.shape) == shape):
+            raise ValueError(f"out must be a contiguous int64 tensor {list(shape)} on {self.device}")
+        self.handle.counts_map_sum(out, device_mask(mask, self.num_envs, self.device, "exploration_map_sum"), stream=self._stream())
         return out
 
     def full_info(self, env: int = 0) -> dict:
