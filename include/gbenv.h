@@ -32,8 +32,8 @@
 extern "C" {
 #endif
 
-#define GBENV_ABI_VERSION 4 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
-                               4: gbenv_counts_map_sum, gbenv_reduce_info_masked */
+#define GBENV_ABI_VERSION 5 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
+                               4: gbenv_counts_map_sum, gbenv_reduce_info_masked; 5: gbenv_capture_frames, gbenv_frames_to_rgb */
 
 #define GBENV_STATE_BYTES 142610 /* PyBoy v9 save-state length (SURVEY.md 8c)              */
 #define GBENV_OBS_H 72           /* environment.py:154-166: (144//2, 160//2, 4) uint8       */
@@ -42,6 +42,7 @@ extern "C" {
 #define GBENV_OBS_BYTES (GBENV_OBS_H * GBENV_OBS_W * GBENV_OBS_C)
 #define GBENV_SCREEN_H 144
 #define GBENV_SCREEN_W 160
+#define GBENV_FRAME_WORDS 1440 /* packed frame: 144 lines x 10 words of 16 2-bit pixels (gbenv_capture_frames) */
 #define GBENV_NUM_ACTIONS 8 /* pyboy_binding.ACTIONS :40  Down Left Right Up A B Start Select */
 #define GBENV_ACT_FREQ 24   /* pyboy_binding.run_action_on_emulator :72 frame_skip=24         */
 #define GBENV_INFO_SCALARS 72
@@ -104,6 +105,20 @@ int gbenv_read_mem(gbenv_t *h, int env, uint32_t addr, uint32_t n, uint8_t *out_
 int gbenv_write_mem(gbenv_t *h, int env, uint32_t addr, uint32_t n, const uint8_t *in_host);
 /* botsupport screen().screen_ndarray(): uint8[144*160*3] of one env, synchronous.               */
 int gbenv_screen(gbenv_t *h, int env, uint8_t *rgb_host);
+/* Batched, asynchronous frames (the reference's save_video / render() frames, pyboy_binding.py:77-78,86-87).
+ * A PACKED frame is the env's framebuffer as the library stores it: 144 lines x 10 uint32 words = GBENV_FRAME_WORDS words
+ * (5,760 B, 12x smaller than RGB, lossless).  The pixel (x, y) is the 2-bit shade at bit 2*(x & 15) of word y*10 + x/16;
+ * the grey of shade s is {0xFF, 0x99, 0x55, 0x00}[s].
+ * gbenv_capture_frames: the current frame of the listed envs into frames_dev uint32[n][GBENV_FRAME_WORDS].  env_ids_dev:
+ * int32[n] on the device, any order, duplicates allowed; NULL means envs 0..n-1 (n <= n_envs).  A row whose id is outside
+ * [0, n_envs) is left untouched and nothing is read for it.  For a valid id the row is bit-identical to the framebuffer
+ * gbenv_screen decodes.  Asynchronous on `stream` and ordered after earlier calls on the handle.
+ * gbenv_frames_to_rgb: n_frames packed frames -> out_dev uint8[n_frames][144][160][channels], channels 1 = grey, 3 = RGB as
+ * gbenv_screen.  out_dev must be 16-byte aligned.  Asynchronous on `stream`.
+ * Both: GBENV_E_ARG on NULL or misaligned buffers, a negative count, channels not 1 or 3, NULL ids with n > n_envs; a count
+ * of 0 is a successful no-op.                                                                   */
+int gbenv_capture_frames(gbenv_t *h, const int32_t *env_ids_dev, int n, uint32_t *frames_dev, void *stream);
+int gbenv_frames_to_rgb(gbenv_t *h, const uint32_t *frames_dev, int n_frames, int channels, uint8_t *out_dev, void *stream);
 
 /* ---- (3) Environment.reset / step with fused reward + observation ---------------------------
  * gbenv_reset == Environment.reset (environment.py:1233-1334) for envs with mask[e] != 0

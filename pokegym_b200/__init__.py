@@ -12,6 +12,10 @@ def __getattr__(name):
         from . import vec_env
 
         return getattr(vec_env, name)
+    if name == "FrameRecorder":
+        from . import frames
+
+        return frames.FrameRecorder
     if name == "EnvGroups":
         from . import groups
 

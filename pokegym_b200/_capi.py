@@ -18,8 +18,10 @@ STATE_BYTES = 142_610
 OBS_H, OBS_W, OBS_C = 72, 80, 4
 OBS_BYTES = OBS_H * OBS_W * OBS_C
 INFO_SCALARS = 72
-ABI_VERSION = 4
+ABI_VERSION = 5
 COUNTS_H, COUNTS_W = 444, 436
+SCREEN_H, SCREEN_W = 144, 160
+FRAME_WORDS = 1440  # packed frame: 144 lines x 10 uint32 words of 16 2-bit shades (include/gbenv.h)
 NUM_ACTIONS = 8
 ACT_FREQ = 24
 
@@ -55,6 +57,11 @@ def _ptr(x) -> C.c_void_p:
     raise TypeError(f"cannot take the address of {type(x)}")
 
 
+def _nbytes(x) -> int:
+    """Size in bytes of a torch tensor or numpy array."""
+    return int(x.numel() * x.element_size()) if hasattr(x, "element_size") else int(x.nbytes)
+
+
 # name -> (argtypes, restype); shared by both libraries
 _SIGS = {
     "abi_version": ([], C.c_int),
@@ -77,6 +84,8 @@ _SIGS = {
     "read_mem": ([C.c_void_p, C.c_int, C.c_uint32, C.c_uint32, C.c_void_p], C.c_int),
     "write_mem": ([C.c_void_p, C.c_int, C.c_uint32, C.c_uint32, C.c_void_p], C.c_int),
     "screen": ([C.c_void_p, C.c_int, C.c_void_p], C.c_int),
+    "capture_frames": ([C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p], C.c_int),
+    "frames_to_rgb": ([C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p], C.c_int),
     "reset": ([C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_void_p, C.c_size_t, C.c_void_p], C.c_int),
     "reset_dev": ([C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_void_p, C.c_size_t, C.c_void_p], C.c_int),
     "submit_host": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
@@ -204,6 +213,21 @@ class Handle:
         out = np.empty((144, 160, 3), dtype=np.uint8)
         self._check(self.lib.screen(self._h, int(env), _ptr(out)), "screen")
         return out
+
+    def capture_frames(self, frames, env_ids=None, stream: int = 0):
+        """The current packed frame of the envs `env_ids` (int32, on the device for CUDA, host memory for the oracle; None:
+        envs 0..len(frames)-1) -> frames uint32 [n, FRAME_WORDS].  Rows of ids outside [0, n_envs) are left untouched."""
+        n = len(frames) if env_ids is None else len(env_ids)
+        if _nbytes(frames) < n * FRAME_WORDS * 4:
+            raise ValueError(f"frames holds fewer than {n} packed frames")
+        self._check(self.lib.capture_frames(self._h, _ptr(env_ids), int(n), _ptr(frames), C.c_void_p(stream)), "capture_frames")
+
+    def frames_to_rgb(self, frames, out, channels: int = 3, stream: int = 0):
+        """Packed frames uint32 [n, FRAME_WORDS] -> out uint8 [n, 144, 160, channels] (1 = grey, 3 = RGB as screen())."""
+        if _nbytes(frames) < len(frames) * FRAME_WORDS * 4 or _nbytes(out) < len(frames) * SCREEN_H * SCREEN_W * max(int(channels), 0):
+            raise ValueError("frames must be [n, FRAME_WORDS] words and out must hold n decoded frames")
+        self._check(self.lib.frames_to_rgb(self._h, _ptr(frames), int(len(frames)), int(channels), _ptr(out), C.c_void_p(stream)),
+                    "frames_to_rgb")
 
     # -- Environment API -----------------------------------------------------
     def reset(self, obs, mask=None, max_episode_steps: int = 20480, reward_scale: float = 4.0, obs_stride: int = OBS_BYTES, stream: int = 0):

@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "../../include/gbenv.h"
+#include "gb_frames.cuh"
 #include "gb_image.h"
 #include "gb_kernels.cuh"
 #include "gb_wrap.cuh"
@@ -500,6 +501,27 @@ extern "C" int gbenv_screen(gbenv *h, int env, uint8_t *rgb) {
         uint8_t g = grey[(fb[i >> 4] >> (2 * (i & 15))) & 3];
         rgb[3 * i] = rgb[3 * i + 1] = rgb[3 * i + 2] = g;
     }
+    return GBENV_OK;
+}
+
+extern "C" int gbenv_capture_frames(gbenv *h, const int32_t *env_ids_dev, int n, uint32_t *frames_dev, void *stream) {
+    if (!h || n < 0 || (!env_ids_dev && n > h->n) || (n && !frames_dev) || ((uintptr_t)frames_dev & 3) || ((uintptr_t)env_ids_dev & 3))
+        return fail(h, GBENV_E_ARG, "gbenv_capture_frames: bad argument (NULL or misaligned buffer, n < 0, or NULL ids with n > n_envs)");
+    if (n == 0) return GBENV_OK;
+    CK(cudaSetDevice(h->device));
+    CK(launch_frames_capture(h->d.fb, env_ids_dev, n, h->n, frames_dev, pick(h, stream)));
+    h->launches++;
+    return GBENV_OK;
+}
+
+extern "C" int gbenv_frames_to_rgb(gbenv *h, const uint32_t *frames_dev, int n_frames, int channels, uint8_t *out_dev, void *stream) {
+    if (!h || n_frames < 0 || (channels != 1 && channels != 3) || (n_frames && (!frames_dev || !out_dev)) || ((uintptr_t)frames_dev & 3) ||
+        ((uintptr_t)out_dev & 15))
+        return fail(h, GBENV_E_ARG, "gbenv_frames_to_rgb: bad argument (NULL or misaligned buffer, n_frames < 0, or channels not 1 or 3)");
+    if (n_frames == 0) return GBENV_OK;
+    CK(cudaSetDevice(h->device));
+    CK(launch_frames_to_rgb(frames_dev, n_frames, channels, out_dev, pick(h, stream)));
+    h->launches++;
     return GBENV_OK;
 }
 

@@ -18,6 +18,7 @@ from typing import Iterable, Optional, Sequence, Union
 import numpy as np
 
 from . import _capi
+from .frames import FrameRecorder, check_channels, decode_target, host_env_ids
 from .info import INFO_NAMES, build_info, info_row_to_dict  # noqa: F401
 
 try:  # gymnasium is not installed in this image; use it when it is
@@ -137,6 +138,7 @@ class VecEnvironment:
         self.rollout = rollout
         self.validate_actions = bool(validate_actions)  # off by default: the check is a device->host sync; the kernel masks actions with & 7
         self._t = 0
+        self._recorder = None
         with torch.cuda.device(self.device):
             self._obs = torch.zeros((self.num_envs, *OBS_SHAPE), dtype=torch.uint8, device=self.device)
             self._reward = torch.zeros(self.num_envs, dtype=torch.float64, device=self.device)
@@ -208,6 +210,8 @@ class VecEnvironment:
                 prev = self.rollout[(self._t - 1) % self.rollout.shape[0]]
                 obs.view(self.num_envs, -1)[skip.bool()] = prev.view(self.num_envs, -1)[skip.bool()]
             self.handle.step_masked(actions, skip, obs, self._reward, self._done, obs_stride=_capi.OBS_BYTES, stream=self._stream())
+        if self._recorder is not None:  # the frames this step ended on, before an auto-reset below
+            self._recorder._capture(self._done, self._stream())
         done = self._done.bool()
         if self.auto_reset:
             # envs that just finished are reset on the device, masked by the done vector the step wrote: their row of `obs`
@@ -216,6 +220,36 @@ class VecEnvironment:
             self.handle.reset_dev(obs, mask_dev=self._done_prev, max_episode_steps=self.max_episode_steps, reward_scale=self.reward_scale,
                                   obs_stride=_capi.OBS_BYTES, stream=self._stream())
         return obs.view(self.num_envs, *OBS_SHAPE), self._reward, done, done, {}
+
+    def screens(self, env_ids=None, channels: int = 3, out=None):
+        """uint8 [n, 144, 160, channels] device tensor: the current frame of the envs `env_ids` (None: all), grey
+        (channels=1) or RGB (3) exactly as screen() / gbenv_screen gives one env.  Captured and decoded on the device,
+        asynchronously; the ids are checked on the host (pass a list or array: a device tensor is copied there first)."""
+        torch = self.torch
+        channels = check_channels(channels)
+        ids = None
+        n = self.num_envs
+        if env_ids is not None:
+            a = host_env_ids(env_ids, self.num_envs)
+            n = a.size
+            ids = torch.from_numpy(a).pin_memory().to(self.device, non_blocking=True)
+        out = decode_target(torch, out, n, channels, self.device)
+        packed = torch.empty((n, _capi.FRAME_WORDS), dtype=torch.int32, device=self.device)
+        self.handle.capture_frames(packed, ids, stream=self._stream())
+        self.handle.frames_to_rgb(packed, out, channels, stream=self._stream())
+        return out
+
+    def record_frames(self, env_ids, capacity: Optional[int] = None) -> Optional[FrameRecorder]:
+        """Records the frame of the envs `env_ids` on every step() from now on into a new FrameRecorder holding the last
+        `capacity` steps (uint32 [capacity, len(env_ids), 1440] packed, 5,760 B per frame), and returns it.  It replaces
+        the previous recorder; record_frames(None) stops recording."""
+        if env_ids is None:
+            self._recorder = None
+            return None
+        if capacity is None:
+            raise ValueError("record_frames needs a capacity (steps held)")
+        self._recorder = FrameRecorder(self, env_ids, capacity)
+        return self._recorder
 
     @staticmethod
     def compact_view(obs):
