@@ -32,8 +32,9 @@
 extern "C" {
 #endif
 
-#define GBENV_ABI_VERSION 5 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
-                               4: gbenv_counts_map_sum, gbenv_reduce_info_masked; 5: gbenv_capture_frames, gbenv_frames_to_rgb */
+#define GBENV_ABI_VERSION 6 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
+                               4: gbenv_counts_map_sum, gbenv_reduce_info_masked; 5: gbenv_capture_frames, gbenv_frames_to_rgb;
+                               6: gbenv_event_flags */
 
 #define GBENV_STATE_BYTES 142610 /* PyBoy v9 save-state length (SURVEY.md 8c)              */
 #define GBENV_OBS_H 72           /* environment.py:154-166: (144//2, 160//2, 4) uint8       */
@@ -46,6 +47,8 @@ extern "C" {
 #define GBENV_NUM_ACTIONS 8 /* pyboy_binding.ACTIONS :40  Down Left Right Up A B Start Select */
 #define GBENV_ACT_FREQ 24   /* pyboy_binding.run_action_on_emulator :72 frame_skip=24         */
 #define GBENV_INFO_SCALARS 72
+#define GBENV_EVENT_FLAGS 130 /* entries of the reference's event table (gbenv_event_flags)                       */
+#define GBENV_EVENT_WORDS 5   /* uint32 words of one env's event flags: GBENV_EVENT_FLAGS bits rounded up to 32 */
 
 enum {
     GBENV_OK = 0,
@@ -179,6 +182,18 @@ int gbenv_counts_map(gbenv_t *h, int env, int32_t *map_host);
  * Asynchronous on `stream`, ordered after earlier calls on the handle.  GBENV_E_ARG when heat maps are switched off;
  * GBENV_E_NOMEM once an exhausted pool has been reported (as gbenv_step), since the maps are then incomplete.        */
 int gbenv_counts_map_sum(gbenv_t *h, const uint8_t *mask_dev, int64_t *sum_dev /* 444*436 */, void *stream);
+/* The event flags behind the `*_events_aggregate` / `gym_events` and `detailed_rewards_*` entries of the info dict
+ * (environment.py:1621-1810, ram_map_leanke.py monitor_*_events) for a list of envs, into flags_dev uint32[n][GBENV_EVENT_WORDS].
+ * Bit k & 31 of word k >> 5 is the WRAM bit that entry k of the reference's event table reads, as stored, whatever the sign
+ * of its weight.  The table has GBENV_EVENT_FLAGS entries in the order of pokegym_b200/event_table.json: silph_co 53,
+ * dojo 8, hideout 15, poke_tower 17, gym3 .. gym7.  Entries that read the same bit (gym 5's and gym 6's leader, D7B3 bit 1)
+ * each keep their own position; bits 130..159 are 0.  This is that table and nothing else: there is no address or length,
+ * and it is not a RAM read (gbenv_read_mem reads one env's bytes).
+ * env_ids_dev: int32[n] on the device, any order, duplicates allowed; NULL means envs 0..n-1 (n <= n_envs).  A row whose id
+ * is outside [0, n_envs) is left untouched and nothing is read for it.  Asynchronous on `stream`, ordered after earlier
+ * calls on the handle.  GBENV_E_ARG on a NULL handle, a NULL or misaligned output with n > 0, n < 0, or NULL ids with
+ * n > n_envs; n == 0 is a successful no-op.                                                                            */
+int gbenv_event_flags(gbenv_t *h, const int32_t *env_ids_dev, int n, uint32_t *flags_dev, void *stream);
 
 /* ---- diagnostics ----------------------------------------------------------------------------*/
 typedef struct gbenv_counters {

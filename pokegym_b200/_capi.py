@@ -18,10 +18,12 @@ STATE_BYTES = 142_610
 OBS_H, OBS_W, OBS_C = 72, 80, 4
 OBS_BYTES = OBS_H * OBS_W * OBS_C
 INFO_SCALARS = 72
-ABI_VERSION = 5
+ABI_VERSION = 6
 COUNTS_H, COUNTS_W = 444, 436
 SCREEN_H, SCREEN_W = 144, 160
 FRAME_WORDS = 1440  # packed frame: 144 lines x 10 uint32 words of 16 2-bit shades (include/gbenv.h)
+EVENT_FLAGS = 130  # entries of the reference's event table (pokegym_b200/event_table.json)
+EVENT_WORDS = 5  # uint32 words of one env's event flags
 NUM_ACTIONS = 8
 ACT_FREQ = 24
 
@@ -86,6 +88,7 @@ _SIGS = {
     "screen": ([C.c_void_p, C.c_int, C.c_void_p], C.c_int),
     "capture_frames": ([C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p], C.c_int),
     "frames_to_rgb": ([C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p], C.c_int),
+    "event_flags": ([C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p], C.c_int),
     "reset": ([C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_void_p, C.c_size_t, C.c_void_p], C.c_int),
     "reset_dev": ([C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_void_p, C.c_size_t, C.c_void_p], C.c_int),
     "submit_host": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
@@ -228,6 +231,15 @@ class Handle:
             raise ValueError("frames must be [n, FRAME_WORDS] words and out must hold n decoded frames")
         self._check(self.lib.frames_to_rgb(self._h, _ptr(frames), int(len(frames)), int(channels), _ptr(out), C.c_void_p(stream)),
                     "frames_to_rgb")
+
+    def event_flags(self, out, env_ids=None, stream: int = 0):
+        """The event flags of the envs `env_ids` (int32, on the device for CUDA, host memory for the oracle; None: envs
+        0..len(out)-1) -> out uint32 [n, EVENT_WORDS]: bit k & 31 of word k >> 5 is entry k of the event table.  Rows of ids
+        outside [0, n_envs) are left untouched."""
+        n = len(out) if env_ids is None else len(env_ids)
+        if _nbytes(out) < n * EVENT_WORDS * 4:
+            raise ValueError(f"out holds fewer than {n} rows of event flags")
+        self._check(self.lib.event_flags(self._h, _ptr(env_ids), int(n), _ptr(out), C.c_void_p(stream)), "event_flags")
 
     # -- Environment API -----------------------------------------------------
     def reset(self, obs, mask=None, max_episode_steps: int = 20480, reward_scale: float = 4.0, obs_stride: int = OBS_BYTES, stream: int = 0):

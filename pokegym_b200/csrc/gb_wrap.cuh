@@ -96,36 +96,11 @@ __constant__ uint16_t c_cursor_keys[48] = {
     0xC49A, 0xC4C2, 0xC4EA, 0xC4C1, 0xC4A9, 0xC4BD, 0xC4D1, 0xC4E5, 0xC4C7, 0xC3B4, 0xC3DC, 0xC404, 0xC42C, 0xC454, 0xC47C, 0xC49C,
     0xC4C4, 0xC4EC, 0xC4E9, 0xC48A, 0xC4B2, 0xC3F5, 0xC41D, 0xC445, 0x0169, 0xC4EF, 0xC44F, 0xC477, 0xC469, 0xC459, 0xC46D, 0xC481};
 
-// ram_map_leanke.py monitor_* dicts in insertion order: address | bit << 16 | (weight & 0xFF) << 24
+// ram_map_leanke.py monitor_* dicts in insertion order (event_bits.inc): address | bit << 16 | (weight & 0xFF) << 24
 #define EV(a, b, w) ((uint32_t)(a) | ((uint32_t)(b) << 16) | ((uint32_t)((w) & 0xFF) << 24))
 __constant__ uint32_t c_events[] = {
-    // silph co (53) :107-164   TRAINER 1, QUEST 5, ITEM 5, GYM_LEADER 5, TASK 2
-    EV(0xD825, 2, 1), EV(0xD825, 3, 1), EV(0xD825, 4, 1), EV(0xD825, 5, 1), EV(0xD826, 5, 5), EV(0xD826, 6, 5), EV(0xD827, 2, 1), EV(0xD827, 3, 1),
-    EV(0xD828, 0, 5), EV(0xD828, 1, 5), EV(0xD829, 2, 1), EV(0xD829, 3, 1), EV(0xD829, 4, 1), EV(0xD82A, 0, 5), EV(0xD82A, 1, 5), EV(0xD82B, 2, 1),
-    EV(0xD82B, 3, 1), EV(0xD82B, 4, 1), EV(0xD82B, 5, 1), EV(0xD82C, 0, 5), EV(0xD82C, 1, 5), EV(0xD82C, 2, 5), EV(0xD82D, 6, 1), EV(0xD82D, 7, 1),
-    EV(0xD82E, 0, 1), EV(0xD82E, 7, 5), EV(0xD82F, 5, 1), EV(0xD82F, 6, 1), EV(0xD82F, 7, 1), EV(0xD830, 0, 1), EV(0xD830, 4, 5), EV(0xD830, 5, 5),
-    EV(0xD830, 6, 5), EV(0xD831, 2, 1), EV(0xD831, 3, 1), EV(0xD831, 4, 1), EV(0xD832, 0, 5), EV(0xD833, 2, 1), EV(0xD833, 3, 1), EV(0xD833, 4, 1),
-    EV(0xD834, 0, 5), EV(0xD834, 1, 5), EV(0xD834, 2, 5), EV(0xD834, 3, 5), EV(0xD835, 1, 1), EV(0xD835, 2, 1), EV(0xD836, 0, 5), EV(0xD837, 4, 1),
-    EV(0xD837, 5, 1), EV(0xD838, 0, 5), EV(0xD838, 5, 5), EV(0xD838, 7, 5), EV(0xD7B9, 7, 2),
-    // dojo (8) :816-827   BAD -1, GYM_LEADER 5, TRAINER 1, POKEMON 3
-    EV(0xD7B1, 0, -1), EV(0xD7B1, 1, 5), EV(0xD7B1, 2, 1), EV(0xD7B1, 3, 1), EV(0xD7B1, 4, 1), EV(0xD7B1, 5, 1), EV(0xD7B1, 6, 3), EV(0xD7B1, 7, 3),
-    // hideout (15) :867-889, weights overridden to 1
-    EV(0xD815, 1, 1), EV(0xD815, 2, 1), EV(0xD815, 3, 1), EV(0xD815, 4, 1), EV(0xD815, 5, 1), EV(0xD817, 1, 1), EV(0xD819, 1, 1), EV(0xD819, 2, 1),
-    EV(0xD81B, 2, 1), EV(0xD81B, 3, 1), EV(0xD81B, 4, 1), EV(0xD81B, 5, 1), EV(0xD81B, 6, 1), EV(0xD81B, 7, 1), EV(0xD77E, 1, 1),
-    // pokemon tower (17) :936-957
-    EV(0xD765, 1, 1), EV(0xD765, 2, 1), EV(0xD765, 3, 1), EV(0xD766, 1, 1), EV(0xD766, 2, 1), EV(0xD766, 3, 1), EV(0xD767, 2, 1), EV(0xD767, 3, 1),
-    EV(0xD767, 4, 1), EV(0xD767, 5, 1), EV(0xD768, 1, 1), EV(0xD768, 2, 1), EV(0xD768, 3, 1), EV(0xD768, 7, 5), EV(0xD769, 1, 1), EV(0xD769, 2, 1),
-    EV(0xD769, 3, 1),
-    // gym 3 (6) :1038-1047   GYM_TASK 2, GYM_LEADER 5, GYM_TRAINER 2
-    EV(0xD773, 1, 2), EV(0xD773, 0, 2), EV(0xD773, 7, 5), EV(0xD773, 2, 2), EV(0xD773, 3, 2), EV(0xD773, 4, 2),
-    // gym 4 (8)
-    EV(0xD792, 1, 5), EV(0xD77C, 2, 2), EV(0xD77C, 3, 2), EV(0xD77C, 4, 2), EV(0xD77C, 5, 2), EV(0xD77C, 6, 2), EV(0xD77C, 7, 2), EV(0xD77D, 0, 2),
-    // gym 5 (7)
-    EV(0xD7B3, 1, 5), EV(0xD792, 2, 2), EV(0xD792, 3, 2), EV(0xD792, 4, 2), EV(0xD792, 5, 2), EV(0xD792, 6, 2), EV(0xD792, 7, 2),
-    // gym 6 (8): 'six' reads D7B3 bit 1 like gym 5's leader (:1064,1076)
-    EV(0xD7B3, 1, 5), EV(0xD7B3, 2, 2), EV(0xD7B3, 3, 2), EV(0xD7B3, 4, 2), EV(0xD7B3, 5, 2), EV(0xD7B3, 6, 2), EV(0xD7B3, 7, 2), EV(0xD7B4, 0, 2),
-    // gym 7 (8)
-    EV(0xD79A, 1, 5), EV(0xD79A, 2, 2), EV(0xD79A, 3, 2), EV(0xD79A, 4, 2), EV(0xD79A, 5, 2), EV(0xD79A, 6, 2), EV(0xD79A, 7, 2), EV(0xD79B, 0, 2)};
+#include "event_bits.inc"
+};
 #undef EV
 // group boundaries inside c_events: silph, dojo, hideout, tower, gym3..7
 __constant__ int c_event_groups[10] = {0, 53, 61, 76, 93, 99, 107, 114, 122, 130};

@@ -10,6 +10,7 @@
 #include <vector>
 
 #include "../../include/gbenv.h"
+#include "gb_events.cuh"
 #include "gb_frames.cuh"
 #include "gb_image.h"
 #include "gb_kernels.cuh"
@@ -521,6 +522,16 @@ extern "C" int gbenv_frames_to_rgb(gbenv *h, const uint32_t *frames_dev, int n_f
     if (n_frames == 0) return GBENV_OK;
     CK(cudaSetDevice(h->device));
     CK(launch_frames_to_rgb(frames_dev, n_frames, channels, out_dev, pick(h, stream)));
+    h->launches++;
+    return GBENV_OK;
+}
+
+extern "C" int gbenv_event_flags(gbenv *h, const int32_t *env_ids_dev, int n, uint32_t *flags_dev, void *stream) {
+    if (!h || n < 0 || (!env_ids_dev && n > h->n) || (n && !flags_dev) || ((uintptr_t)flags_dev & 3) || ((uintptr_t)env_ids_dev & 3))
+        return fail(h, GBENV_E_ARG, "gbenv_event_flags: bad argument (NULL or misaligned buffer, n < 0, or NULL ids with n > n_envs)");
+    if (n == 0) return GBENV_OK;
+    CK(cudaSetDevice(h->device));
+    CK(launch_event_flags(h->d.mem, env_ids_dev, n, h->n, flags_dev, pick(h, stream)));
     h->launches++;
     return GBENV_OK;
 }

@@ -23,7 +23,7 @@ def all_reduce_info(info_sum, group=None):
     """In-place sum of the per-rank info vectors (slot 0 = env count).  No-op without a process group.
 
     Any dtype: the int64 [444, 436] exploration-map sum (VecEnvironment.exploration_map_sum) goes through the same call,
-    1.5 MB per all-reduce, and stays exact."""
+    1.5 MB per all-reduce, and stays exact; so do the int64 [130] event-flag counts (VecEnvironment.event_counts)."""
     import torch.distributed as dist
 
     if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:

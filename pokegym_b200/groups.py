@@ -20,7 +20,7 @@ from __future__ import annotations
 from typing import List, Optional
 
 from . import _capi
-from .vec_env import device_mask
+from .vec_env import device_mask, event_counts_from_flags
 
 
 class EnvGroups:
@@ -39,6 +39,7 @@ class EnvGroups:
             self._done = [torch.cuda.Event() for _ in range(n_groups)]
             self._info_parts = torch.zeros((n_groups, _capi.INFO_SCALARS), dtype=torch.float64, device=self.device)
         self._map_parts = None  # [n_groups, 444, 436] int64, allocated by the first exploration_map_sum
+        self._flags = None  # [num_envs, 5] int32, allocated by the first event_counts
         if lanes:
             for h in self.handles:
                 h.set_lanes_per_warp(lanes)
@@ -110,6 +111,18 @@ class EnvGroups:
         self.join()
         self.torch.sum(self._map_parts, dim=0, out=out)
         return out
+
+    def event_counts(self, out, mask=None):
+        """int64 [130] count of the envs of every group (or those with mask[e] != 0) that have each event flag set -> out (on
+        the caller's stream, after a join)"""
+        mask = device_mask(mask, self.num_envs, self.device, "event_counts")
+        if self._flags is None:
+            self._flags = self.torch.empty((self.num_envs, _capi.EVENT_WORDS), dtype=self.torch.int32, device=self.device)
+        self._fork()
+        for g, (h, s) in enumerate(zip(self.handles, self.streams)):
+            h.event_flags(self._slice(self._flags, g), stream=s.cuda_stream)
+        self.join()
+        return event_counts_from_flags(self.torch, self._flags, mask, out)
 
     # -- counters --------------------------------------------------------------------------------------------------
     def counters(self):

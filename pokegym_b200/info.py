@@ -76,19 +76,72 @@ def event_table() -> Dict[str, list]:
     return _EVENT_TABLE
 
 
-def monitor_events(group: str, read_byte: Callable[[int], int]) -> Dict[str, int]:
-    """ram_map_leanke.monitor_<group>_events: name -> weight * bit."""
-    return {name: w * ((read_byte(a) >> b) & 1) for name, a, b, w in event_table()[group]}
-
-
 def event_rewards_detailed(events: Dict[str, int], base_reward=10, reward_increment=2, reward_multiplier=1) -> Dict[str, int]:
     """environment.py:1221-1231: base + value*increment*multiplier for positive entries, value*increment*multiplier otherwise."""
     return {k: (base_reward if v > 0 else 0) + v * reward_increment * reward_multiplier for k, v in events.items()}
 
 
+def event_bits(read_byte: Callable[[int], int]) -> np.ndarray:
+    """uint8 [130]: the bit that entry k of the event table reads (`read_byte(addr)`, e.g. gbenv_read_mem), in table order
+    (silph_co, dojo, hideout, poke_tower, gym3..gym7), whatever the sign of its weight."""
+    return np.array([(read_byte(a) >> b) & 1 for g in _GROUPS for _, a, b, _ in event_table()[g]], dtype=np.uint8)
+
+
+def unpack_event_words(words) -> np.ndarray:
+    """gbenv_event_flags rows [n, 5] (uint32 or int32 words: bit k & 31 of word k >> 5 is entry k) -> uint8 [n, 130]."""
+    if hasattr(words, "detach"):
+        words = words.detach().cpu().numpy()
+    w = np.ascontiguousarray(words)
+    if w.ndim != 2 or w.shape[1] != 5 or w.dtype.itemsize != 4:
+        raise ValueError("event words must be a [n, 5] array of 32-bit words")
+    return np.unpackbits(w.astype("<u4", copy=False).view(np.uint8), axis=1, bitorder="little")[:, :130]
+
+
+def _event_entries(ev: Dict[str, dict], detailed: Dict[str, dict]) -> dict:
+    """The event part of the info dict (environment.py:1790-1810) from per-group {name: value} dicts."""
+    return {
+        "detailed_rewards_silph_co": detailed["silph_co"], "detailed_rewards_dojo": detailed["dojo"],
+        "detailed_rewards_hideout": detailed["hideout"], "detailed_rewards_poke_tower": detailed["poke_tower"],
+        "detailed_rewards_gyms": {f"gym_{k}_detailed_rewards": detailed[f"gym{k}"] for k in range(3, 8)},
+        "silph_co_events_aggregate": ev["silph_co"], "dojo_events_aggregate": ev["dojo"], "hideout_events_aggregate": ev["hideout"],
+        "poke_tower_events_aggregate": ev["poke_tower"], "gym_events": {f"gym_{k}_events": ev[f"gym{k}"] for k in range(3, 8)},
+    }
+
+
+def _by_group(values) -> Dict[str, list]:
+    """group -> [(name, weight, value of its entry)] for one value per table entry, in table order."""
+    out, k = {}, 0
+    for g in _GROUPS:
+        out[g] = [(name, w, values[k + j]) for j, (name, _, _, w) in enumerate(event_table()[g])]
+        k += len(out[g])
+    return out
+
+
+def event_counts_to_means(counts, n) -> dict:
+    """Counts of set event flags over n envs (int64 [130], e.g. VecEnvironment.event_counts, all-reduced or not) -> the
+    nine aggregate dicts and the `detailed_rewards_*` dicts as means over those n envs, under the reference's keys.  Per env
+    an aggregate entry is weight * bit and a detailed one (10 if weight * bit > 0 else 0) + 2 * weight * bit."""
+    if hasattr(counts, "detach"):
+        counts = counts.detach().cpu().numpy()
+    c = np.asarray(counts, dtype=np.float64).reshape(-1)
+    if c.size != 130:
+        raise ValueError("counts must have 130 entries")
+    n = max(float(n), 1.0)
+    groups = _by_group(c)
+    ev = {g: {name: w * v / n for name, w, v in rows} for g, rows in groups.items()}
+    detailed = {g: {name: ((10 if w > 0 else 0) + 2 * w) * v / n for name, w, v in rows} for g, rows in groups.items()}
+    return _event_entries(ev, detailed)
+
+
 def build_info(row: np.ndarray, read_byte: Callable[[int], int], counts_map: Optional[np.ndarray] = None, reward_scale: float = 4.0) -> dict:
     """The dict `Environment.step` returns when `done or time % 10000 == 0` (environment.py:1621-1810), rebuilt from one
-    info row, the env's event bytes (`read_byte(addr)`, e.g. gbenv_read_mem) and its counts_map.
+    info row, the env's event bytes (`read_byte(addr)`, e.g. gbenv_read_mem) and its counts_map."""
+    return build_info_from_events(row, event_bits(read_byte), counts_map=counts_map, reward_scale=reward_scale)
+
+
+def build_info_from_events(row: np.ndarray, bits, counts_map: Optional[np.ndarray] = None, reward_scale: float = 4.0) -> dict:
+    """build_info from one info row, the env's 130 event bits (event_bits, or a row of unpack_event_words) and its
+    counts_map.
 
     Entries the reference fills from state it never updates are emitted with the constant it would hold
     (`self.badge_count`, `events`, `seen_npcs_count`, `hidden_obj_count`, `state_loaded_instead_of_resetting_in_game`: 0).
@@ -121,12 +174,6 @@ def build_info(row: np.ndarray, read_byte: Callable[[int], int], counts_map: Opt
         "has_lemonade_in_bag_reward": I["r_lemonade"], "has_silph_scope_in_bag_reward": I["r_silph_scope"],
         "has_lift_key_in_bag_reward": I["r_lift_key"], "has_pokedoll_in_bag_reward": I["r_pokedoll"], "has_bicycle_in_bag_reward": I["r_bicycle"],
     }
-    ev = {g: monitor_events(g, read_byte) for g in _GROUPS}
-    return {
-        "pokemon_exploration_map": counts_map, "stats": stats, "reward": reward,
-        "detailed_rewards_silph_co": event_rewards_detailed(ev["silph_co"]), "detailed_rewards_dojo": event_rewards_detailed(ev["dojo"]),
-        "detailed_rewards_hideout": event_rewards_detailed(ev["hideout"]), "detailed_rewards_poke_tower": event_rewards_detailed(ev["poke_tower"]),
-        "detailed_rewards_gyms": {f"gym_{k}_detailed_rewards": event_rewards_detailed(ev[f"gym{k}"]) for k in range(3, 8)},
-        "silph_co_events_aggregate": ev["silph_co"], "dojo_events_aggregate": ev["dojo"], "hideout_events_aggregate": ev["hideout"],
-        "poke_tower_events_aggregate": ev["poke_tower"], "gym_events": {f"gym_{k}_events": ev[f"gym{k}"] for k in range(3, 8)},
-    }
+    ev = {g: {name: w * int(b) for name, w, b in rows} for g, rows in _by_group(bits).items()}  # monitor_<group>_events
+    return {"pokemon_exploration_map": counts_map, "stats": stats, "reward": reward,
+            **_event_entries(ev, {g: event_rewards_detailed(v) for g, v in ev.items()})}

@@ -8,7 +8,9 @@ here, so the contract is restated from PufferLib's published vector API (pufferl
   * an env that reported `done` is reset on the NEXT `send`: that call's action for it is ignored, it is not stepped, and
     `recv` delivers its reset observation with reward 0 and terminal False (pufferlib.vector.Serial.send: `if env.done:
     o, i = env.reset() ... else: o, r, d, t, i = env.step(atn)`);
-  * infos: one dict per env that finished an episode on this step.
+  * infos: one dict per env that finished an episode on this step.  By default that is the env's stats and reward terms
+    (info_row_to_dict); with full_infos=True it is the reference's whole info dict (VecEnvironment.episode_infos: the
+    130 event flags and the detailed rewards too), without the per-env exploration map.
 
 Everything stays on the device: the reset is masked by the previous step's done vector (gbenv_reset_dev) and the same vector
 makes those envs sit the step out (gbenv_step_masked); only the per-episode info rows of finished envs come to the host.
@@ -23,10 +25,11 @@ from .vec_env import VecEnvironment
 
 
 class PufferVecAdaptor:
-    def __init__(self, vec: VecEnvironment):
+    def __init__(self, vec: VecEnvironment, full_infos: bool = False):
         if vec.auto_reset:
             raise ValueError("PufferVecAdaptor does the resets itself: construct the VecEnvironment with auto_reset=False")
         self.vec = vec
+        self.full_infos = bool(full_infos)
         self.num_envs = vec.num_envs
         self.env_ids = np.arange(self.num_envs)
         t = vec.torch
@@ -50,7 +53,9 @@ class PufferVecAdaptor:
         infos = []
         self._pending.copy_(done)
         self._any_pending = bool(done.any())  # the one host read per step; PufferLib inspects the dones on the host anyway
-        if self._any_pending:
+        if self._any_pending and self.full_infos:
+            infos = list(self.vec.episode_infos(done).values())
+        elif self._any_pending:
             rows = self.vec.info().cpu().numpy()
             infos = [info_row_to_dict(rows[e]) for e in np.nonzero(done.cpu().numpy())[0]]
         self._last = (obs, rew, done, infos)

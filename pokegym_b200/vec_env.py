@@ -19,7 +19,7 @@ import numpy as np
 
 from . import _capi
 from .frames import FrameRecorder, check_channels, decode_target, host_env_ids
-from .info import INFO_NAMES, build_info, info_row_to_dict  # noqa: F401
+from .info import INFO_NAMES, build_info, build_info_from_events, info_row_to_dict, unpack_event_words  # noqa: F401
 
 try:  # gymnasium is not installed in this image; use it when it is
     from gymnasium.spaces import Box, Discrete  # type: ignore
@@ -111,6 +111,26 @@ def device_mask(mask, n: int, device, what: str = "mask"):
         if mask.numel() != n:
             raise ValueError(f"{what} mask must have {n} entries")
     return mask
+
+
+def event_counts_from_flags(torch, flags, mask, out):
+    """int64 [130] `out` = how many rows of `flags` (int32 [n, 5] gbenv_event_flags rows, on the device) with mask[e] != 0
+    (mask None: all) have each event flag set.  Device work only: no host synchronisation."""
+    k = torch.arange(_capi.EVENT_FLAGS, device=flags.device)
+    bits = (flags[:, k >> 5] >> (k & 31).to(torch.int32)) & 1  # [n, 130] int32
+    if mask is not None:
+        bits = bits * mask.to(torch.int32)[:, None]
+    return torch.sum(bits, dim=0, dtype=torch.int64, out=out)
+
+
+def check_out(torch, out, shape, dtype, device):
+    """`out` for a result of `shape` / `dtype`: a new tensor on `device`, or the caller's, checked (raw pointers cross the
+    C ABI, so a wrong layout would be out-of-bounds device writes, not an exception)."""
+    if out is None:
+        return torch.empty(shape, dtype=dtype, device=device)
+    if not (torch.is_tensor(out) and out.dtype == dtype and out.device == device and out.is_contiguous() and tuple(out.shape) == tuple(shape)):
+        raise ValueError(f"out must be a contiguous {dtype} tensor {list(shape)} on {device}")
+    return out
 
 
 class VecEnvironment:
@@ -279,24 +299,64 @@ class VecEnvironment:
         """int64 [444, 436] device tensor: the sum of the envs' `pokemon_exploration_map`s (environment.py:1624), over the
         envs with mask[e] != 0 (e.g. the `done` of step()) or over all.  Computed on the device, nothing goes to the host."""
         torch = self.torch
-        shape = (_capi.COUNTS_H, _capi.COUNTS_W)
-        if out is None:
-            out = torch.empty(shape, dtype=torch.int64, device=self.device)
-        elif not (torch.is_tensor(out) and out.dtype == torch.int64 and out.device == self.device and out.is_contiguous() and tuple(out.shape) == shape):
-            raise ValueError(f"out must be a contiguous int64 tensor {list(shape)} on {self.device}")
+        out = check_out(torch, out, (_capi.COUNTS_H, _capi.COUNTS_W), torch.int64, self.device)
         self.handle.counts_map_sum(out, device_mask(mask, self.num_envs, self.device, "exploration_map_sum"), stream=self._stream())
         return out
 
+    def event_flags(self, env_ids=None, out=None):
+        """int32 [n, 5] device tensor: the 130 event flags of the envs `env_ids` (None: all), bit k & 31 of word k >> 5 being
+        entry k of the event table (pokegym_b200.info.event_table, unpack_event_words).  Gathered on the device,
+        asynchronously; the ids are checked on the host (pass a list or array: a device tensor is copied there first)."""
+        torch = self.torch
+        ids = None
+        n = self.num_envs
+        if env_ids is not None:
+            a = host_env_ids(env_ids, self.num_envs)
+            n = a.size
+            ids = torch.from_numpy(a).pin_memory().to(self.device, non_blocking=True)
+        out = check_out(torch, out, (n, _capi.EVENT_WORDS), torch.int32, self.device)
+        self.handle.event_flags(out, ids, stream=self._stream())
+        return out
+
+    def event_counts(self, mask=None, out=None):
+        """int64 [130] device tensor: how many of the envs with mask[e] != 0 (e.g. the `done` of step(); None: all) have
+        each event flag set, in event-table order.  Device work only, no host synchronisation; goes through
+        dist.all_reduce_info like info_sum, and info.event_counts_to_means turns it into the reference's event dicts."""
+        torch = self.torch
+        out = check_out(torch, out, (_capi.EVENT_FLAGS,), torch.int64, self.device)
+        return event_counts_from_flags(torch, self.event_flags(), device_mask(mask, self.num_envs, self.device, "event_counts"), out)
+
+    def episode_infos(self, mask) -> dict:
+        """{env: info dict} for the envs with mask[e] != 0, typically the `done` of step(), in env order.  Each dict is
+        full_info(env)'s with `pokemon_exploration_map` None (exploration_map_sum(mask) is the batched overlay).  Also right
+        after auto_reset: a reset leaves the info row as the last step wrote it and writes no event flag.
+        Two host synchronisations whatever the number of envs: one to find the ids, one copy of their rows and flags."""
+        torch = self.torch
+        mask = device_mask(mask, self.num_envs, self.device, "episode_infos")
+        ids = torch.nonzero(mask).view(-1).to(torch.int32)
+        k = ids.numel()
+        if k == 0:
+            return {}
+        flags = torch.empty((k, _capi.EVENT_WORDS), dtype=torch.int32, device=self.device)
+        self.handle.event_flags(flags, ids, stream=self._stream())
+        rows = self.info()[ids.long()]
+        packed = torch.cat([ids.view(torch.uint8).view(k, 4), rows.view(torch.uint8).view(k, -1), flags.view(torch.uint8).view(k, -1)], 1)
+        host = packed.cpu().numpy()
+        env_ids = host[:, :4].copy().view(np.int32)[:, 0]
+        rows_h = host[:, 4:4 + 8 * _capi.INFO_SCALARS].copy().view(np.float64)
+        bits = unpack_event_words(host[:, 4 + 8 * _capi.INFO_SCALARS:].copy().view(np.uint32))
+        return {int(e): build_info_from_events(rows_h[i], bits[i], counts_map=None, reward_scale=self.reward_scale) for i, e in enumerate(env_ids)}
+
     def full_info(self, env: int = 0) -> dict:
         """The reference's complete info dict for one env (environment.py:1621-1810): scalar row + the 130 named
-        event flags (read from the env's WRAM) + its counts_map.  Rare path (episode end / every 10,000 steps)."""
+        event flags (gbenv_event_flags) + its counts_map.  Rare path (episode end / every 10,000 steps)."""
         row = self.info()[env].cpu().numpy()
-        wram = self.handle.read_mem(env, 0xD700, 0x200)  # every event flag lives in 0xD7B1..0xD838
+        bits = unpack_event_words(self.event_flags([env]))[0]
         try:
             cm = self.handle.counts_map(env).astype(np.float64)
         except _capi.GbEnvError:  # heat maps switched off (GBENV_COUNTS_MAP=0)
             cm = None
-        return build_info(row, lambda a: int(wram[a - 0xD700]), counts_map=cm, reward_scale=self.reward_scale)
+        return build_info_from_events(row, bits, counts_map=cm, reward_scale=self.reward_scale)
 
     def save_state(self, env: int = 0) -> bytes:
         return self.handle.save_state(env)
