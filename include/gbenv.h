@@ -32,9 +32,9 @@
 extern "C" {
 #endif
 
-#define GBENV_ABI_VERSION 6 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
+#define GBENV_ABI_VERSION 7 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
                                4: gbenv_counts_map_sum, gbenv_reduce_info_masked; 5: gbenv_capture_frames, gbenv_frames_to_rgb;
-                               6: gbenv_event_flags */
+                               6: gbenv_event_flags; 7: gbenv_step_packed, gbenv_reset_packed, gbenv_unpack_obs */
 
 #define GBENV_STATE_BYTES 142610 /* PyBoy v9 save-state length (SURVEY.md 8c)              */
 #define GBENV_OBS_H 72           /* environment.py:154-166: (144//2, 160//2, 4) uint8       */
@@ -44,6 +44,8 @@ extern "C" {
 #define GBENV_SCREEN_H 144
 #define GBENV_SCREEN_W 160
 #define GBENV_FRAME_WORDS 1440 /* packed frame: 144 lines x 10 words of 16 2-bit pixels (gbenv_capture_frames) */
+#define GBENV_OBS_PACKED_WORDS 576  /* packed observation: 72 rows x 8 uint32 words (gbenv_step_packed)          */
+#define GBENV_OBS_PACKED_BYTES 2304
 #define GBENV_NUM_ACTIONS 8 /* pyboy_binding.ACTIONS :40  Down Left Right Up A B Start Select */
 #define GBENV_ACT_FREQ 24   /* pyboy_binding.run_action_on_emulator :72 frame_skip=24         */
 #define GBENV_INFO_SCALARS 72
@@ -150,6 +152,27 @@ int gbenv_step(gbenv_t *h, const uint8_t *actions_dev, uint8_t *obs_dev, size_t 
  * gbenv_reset_dev(mask = previous done) followed by gbenv_step_masked(skip = the same mask).                          */
 int gbenv_step_masked(gbenv_t *h, const uint8_t *actions_dev, const uint8_t *skip_dev, uint8_t *obs_dev, size_t obs_stride,
                       double *reward_dev, uint8_t *done_dev, void *stream);
+/* Packed observations: the reference observation stored losslessly in GBENV_OBS_PACKED_BYTES (2,304 B, 10x less than
+ * GBENV_OBS_BYTES), for rollout buffers that would not fit in device memory otherwise.  Channels 0-2 of the reference
+ * observation are the same grey, one of four levels, and channel 3 is 0 or 255, so a pixel is 3 bits.
+ * Layout of one env's uint32[GBENV_OBS_PACKED_WORDS]: obs row i (0..71) is words 8i .. 8i+7.
+ *   - words 8i+k, k = 0..4: obs pixels j = 16k .. 16k+15, the 2-bit shade of pixel j at bit 2*(j & 15) (the convention of the
+ *     packed frame above).  The shade of obs pixel (i, j) is the framebuffer's at (x = 2j, y = 2i); channels 0-2 are
+ *     {0xFF, 0x99, 0x55, 0x00}[shade].
+ *   - words 8i+5+m, m = 0..2: the visited bit of pixel j = 32m + b at bit b; channel 3 is 255 when it is set, 0 otherwise.
+ *     Bits of j >= 80 are 0.
+ * gbenv_step_packed is gbenv_step_masked with the observation written to packed_dev uint32[n_envs][GBENV_OBS_PACKED_WORDS]:
+ * skipped envs' rows are untouched, and rewards, dones, info rows and emulator state are those gbenv_step_masked gives.
+ * gbenv_reset_packed is gbenv_reset_dev with packed output: only the rows of reset envs are written (mask_dev NULL: all).
+ * gbenv_unpack_obs turns n packed rows into out_dev uint8[n][GBENV_OBS_BYTES], the bytes gbenv_step would have written.  It
+ * reads no emulator state, so rows of any step or rollout slot can be decoded; asynchronous on `stream`.
+ * All three: rows are contiguous; packed_dev / out_dev must be 16-byte aligned.  GBENV_E_ARG on a NULL or misaligned buffer
+ * or n < 0; n == 0 is a successful no-op.  Streams and call order as for the calls above.  The host-buffer calls below keep
+ * the reference format.                                                                          */
+int gbenv_step_packed(gbenv_t *h, const uint8_t *actions_dev, const uint8_t *skip_dev, uint32_t *packed_dev, double *reward_dev,
+                      uint8_t *done_dev, void *stream);
+int gbenv_reset_packed(gbenv_t *h, const uint8_t *mask_dev, int max_episode_steps, double reward_scale, uint32_t *packed_dev, void *stream);
+int gbenv_unpack_obs(gbenv_t *h, const uint32_t *packed_dev, int n, uint8_t *out_dev, void *stream);
 /* Same call with HOST buffers (pinned or pageable): copies in, steps, copies out, synchronises.
  * This is the reference-facing entry point a pokegym worker would call.                         */
 int gbenv_step_host(gbenv_t *h, const uint8_t *actions_host, uint8_t *obs_host, double *reward_host,

@@ -18,12 +18,14 @@ STATE_BYTES = 142_610
 OBS_H, OBS_W, OBS_C = 72, 80, 4
 OBS_BYTES = OBS_H * OBS_W * OBS_C
 INFO_SCALARS = 72
-ABI_VERSION = 6
+ABI_VERSION = 7
 COUNTS_H, COUNTS_W = 444, 436
 SCREEN_H, SCREEN_W = 144, 160
 FRAME_WORDS = 1440  # packed frame: 144 lines x 10 uint32 words of 16 2-bit shades (include/gbenv.h)
 EVENT_FLAGS = 130  # entries of the reference's event table (pokegym_b200/event_table.json)
 EVENT_WORDS = 5  # uint32 words of one env's event flags
+OBS_PACKED_WORDS = 576  # packed observation: 72 rows x 8 uint32 words, 3 bits per pixel (include/gbenv.h)
+OBS_PACKED_BYTES = OBS_PACKED_WORDS * 4
 NUM_ACTIONS = 8
 ACT_FREQ = 24
 
@@ -64,6 +66,22 @@ def _nbytes(x) -> int:
     return int(x.numel() * x.element_size()) if hasattr(x, "element_size") else int(x.nbytes)
 
 
+def _byte_rows(x, row_bytes: int, what: str, n=None) -> int:
+    """Number of rows of `x`, a C-contiguous, 16-byte aligned uint8 torch tensor or numpy array of whole `row_bytes` rows
+    (exactly `n` of them when given).  Raw pointers cross the C ABI, so a wrong buffer would be out-of-bounds writes."""
+    if isinstance(x, np.ndarray):
+        ok, addr = x.dtype == np.uint8 and x.flags["C_CONTIGUOUS"], x.ctypes.data
+    elif hasattr(x, "data_ptr"):
+        ok, addr = str(x.dtype) == "torch.uint8" and x.is_contiguous(), x.data_ptr()
+    else:
+        raise TypeError(f"{what} must be a torch tensor or numpy array, not {type(x)}")
+    size = _nbytes(x)
+    if not ok or addr % 16 or size % row_bytes or (n is not None and size != n * row_bytes):
+        rows = "whole" if n is None else str(n)
+        raise ValueError(f"{what} must be a contiguous, 16-byte aligned uint8 buffer of {rows} rows of {row_bytes} bytes")
+    return size // row_bytes
+
+
 # name -> (argtypes, restype); shared by both libraries
 _SIGS = {
     "abi_version": ([], C.c_int),
@@ -95,6 +113,9 @@ _SIGS = {
     "fetch_host": ([C.c_void_p], C.c_int),
     "step": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
     "step_masked": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
+    "step_packed": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
+    "reset_packed": ([C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_void_p, C.c_void_p], C.c_int),
+    "unpack_obs": ([C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p], C.c_int),
     "step_host": ([C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
     "reset_host": ([C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_void_p], C.c_int),
     "get_info": ([C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
@@ -269,6 +290,24 @@ class Handle:
         """Environment.step for the envs with skip[e] == 0; the others sit the step out (reward 0, done 0, obs row untouched)."""
         self._check(self.lib.step_masked(self._h, _ptr(actions), _ptr(skip), _ptr(obs), int(obs_stride), _ptr(reward), _ptr(done), C.c_void_p(stream)),
                     "step_masked")
+
+    def step_packed(self, actions, skip, packed, reward, done, stream: int = 0):
+        """step_masked with the observation packed: packed uint8 [n_envs, OBS_PACKED_BYTES] (rows of skipped envs untouched)."""
+        _byte_rows(packed, OBS_PACKED_BYTES, "packed", self.n_envs)
+        self._check(self.lib.step_packed(self._h, _ptr(actions), _ptr(skip), _ptr(packed), _ptr(reward), _ptr(done), C.c_void_p(stream)),
+                    "step_packed")
+
+    def reset_packed(self, packed, mask_dev=None, max_episode_steps: int = 20480, reward_scale: float = 4.0, stream: int = 0):
+        """reset_dev with the observation packed: packed uint8 [n_envs, OBS_PACKED_BYTES], only the reset envs' rows written."""
+        _byte_rows(packed, OBS_PACKED_BYTES, "packed", self.n_envs)
+        self._check(self.lib.reset_packed(self._h, _ptr(mask_dev), int(max_episode_steps), float(reward_scale), _ptr(packed), C.c_void_p(stream)),
+                    "reset_packed")
+
+    def unpack_obs(self, packed, out, stream: int = 0):
+        """Packed rows uint8 [n, OBS_PACKED_BYTES] -> out uint8 [n, OBS_BYTES], the reference observations."""
+        n = _byte_rows(packed, OBS_PACKED_BYTES, "packed")
+        _byte_rows(out, OBS_BYTES, "out", n)
+        self._check(self.lib.unpack_obs(self._h, _ptr(packed), n, _ptr(out), C.c_void_p(stream)), "unpack_obs")
 
     def step_host(self, actions: np.ndarray, obs: np.ndarray, reward: np.ndarray, done: np.ndarray):
         self._check(self.lib.step_host(self._h, _ptr(actions), _ptr(obs), _ptr(reward), _ptr(done)), "step_host")

@@ -59,6 +59,16 @@ enum {
     R_WORDS
 };
 
+// --- visited bitmaps (seen_coords / screen_memory, gb_wrap.cuh WrapArrays): per env a page table of WRAP_MAPS maps x
+//     VIS_BANDS row bands, each entry a page index + 1 (0 = no page); a page holds 64 rows x 256 columns, bit x & 31 of word
+//     x / 32 of a row being column x.  Shared with the packed-observation writer (gb_obs.cu).
+#define WRAP_MAPS 248
+#define VIS_ROW_WORDS 8                       // 256 columns / 32
+#define VIS_BAND_ROWS 64                      // a visited-bitmap page covers 64 rows x 256 columns of one map = 2 KiB
+#define VIS_BANDS 4
+#define VIS_PAGE_WORDS (VIS_BAND_ROWS * VIS_ROW_WORDS)
+#define VIS_PT_ENTRIES (WRAP_MAPS * VIS_BANDS)  // page-table entries per env
+
 // canonical linear per-env image used by templates / save_state staging (uint32_t words)
 #define IMG_MEM 0
 #define IMG_CRAM (IMG_MEM + MEM_WORDS)

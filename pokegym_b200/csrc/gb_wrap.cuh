@@ -16,13 +16,7 @@
 #include "../../include/gbenv_info.h"
 #include "gb_device.cuh"
 
-#define WRAP_MAPS 248
 #define WRAP_CUT_COORDS 64
-#define VIS_ROW_WORDS 8                       // 256 columns / 32
-#define VIS_BAND_ROWS 64                      // a visited-bitmap page covers 64 rows x 256 columns of one map = 2 KiB
-#define VIS_BANDS 4
-#define VIS_PAGE_WORDS (VIS_BAND_ROWS * VIS_ROW_WORDS)
-#define VIS_PT_ENTRIES (WRAP_MAPS * VIS_BANDS)  // page-table entries per env
 #define COUNTS_H 444
 #define COUNTS_W 436
 #define CM_BLOCK 16                           // heat-map blocks of 16 x 16 cells = 1 KiB

@@ -14,6 +14,7 @@
 #include "gb_frames.cuh"
 #include "gb_image.h"
 #include "gb_kernels.cuh"
+#include "gb_obs.cuh"
 #include "gb_wrap.cuh"
 
 struct StateTemplate {
@@ -572,10 +573,23 @@ static int upload_template_tables(gbenv *h, cudaStream_t st) {
     return GBENV_OK;
 }
 
+// Where a step or a reset puts the observation: reference rows (obs, stride) by k_wrap_obs, or packed rows (packed non-null)
+// by k_obs_pack.  The rows of the envs with mask[e] != 0 are written (== 0 when `invert` is set; mask null: all).
+struct ObsOut {
+    uint8_t *obs;
+    size_t stride;
+    uint32_t *packed;
+};
+
+static void launch_obs(gbenv *h, const ObsOut &o, const uint8_t *mask, int invert, cudaStream_t st) {
+    if (o.packed)
+        launch_obs_pack(h->d.mem, h->d.fb, h->w.vis_pt, h->w.vis_pool, h->n, h->n_tiles, mask, invert, o.packed, st);
+    else
+        k_wrap_obs<<<h->n_tiles, 256, 0, st>>>(h->d, h->w, mask, o.obs, o.stride, invert);
+}
+
 // Environment.reset for the envs with mask_dev[e] != 0 (mask_dev == NULL: all), everything on the device, asynchronous.
-extern "C" int gbenv_reset_dev(gbenv *h, const uint8_t *mask_dev, int max_episode_steps, double reward_scale, uint8_t *obs_dev, size_t obs_stride,
-                               void *stream) {
-    if (!h || !obs_dev || obs_stride < GBENV_OBS_BYTES || (obs_stride & 3)) return fail(h, GBENV_E_ARG, "gbenv_reset: bad argument");
+static int reset_impl(gbenv *h, const uint8_t *mask_dev, int max_episode_steps, double reward_scale, const ObsOut &o, void *stream) {
     CK(cudaSetDevice(h->device));
     cudaStream_t st = pick(h, stream);
     int rc = pool_error(h);
@@ -593,11 +607,22 @@ extern "C" int gbenv_reset_dev(gbenv *h, const uint8_t *mask_dev, int max_episod
     }
     k_vis_release<<<h->n, 256, 0, st>>>(h->w, mask_dev, h->n);  // the envs' bitmap pages go back to the pool
     k_wrap_reset_post<<<blocks, 128, 0, st>>>(h->d, h->w, mask_dev, max_episode_steps, reward_scale);
-    k_wrap_obs<<<h->n_tiles, 256, 0, st>>>(h->d, h->w, mask_dev, obs_dev, obs_stride);
+    launch_obs(h, o, mask_dev, 0, st);
     h->launches += 3;
     CK(cudaGetLastError());
     queue_pool_error_copy(h, st);
     return GBENV_OK;
+}
+
+extern "C" int gbenv_reset_dev(gbenv *h, const uint8_t *mask_dev, int max_episode_steps, double reward_scale, uint8_t *obs_dev, size_t obs_stride,
+                               void *stream) {
+    if (!h || !obs_dev || obs_stride < GBENV_OBS_BYTES || (obs_stride & 3)) return fail(h, GBENV_E_ARG, "gbenv_reset: bad argument");
+    return reset_impl(h, mask_dev, max_episode_steps, reward_scale, ObsOut{obs_dev, obs_stride, nullptr}, stream);
+}
+
+extern "C" int gbenv_reset_packed(gbenv *h, const uint8_t *mask_dev, int max_episode_steps, double reward_scale, uint32_t *packed_dev, void *stream) {
+    if (!h || !packed_dev || ((uintptr_t)packed_dev & 15)) return fail(h, GBENV_E_ARG, "gbenv_reset_packed: bad argument (NULL or misaligned buffer)");
+    return reset_impl(h, mask_dev, max_episode_steps, reward_scale, ObsOut{nullptr, 0, packed_dev}, stream);
 }
 
 extern "C" int gbenv_reset(gbenv *h, const uint8_t *mask_host, int max_episode_steps, double reward_scale, uint8_t *obs_dev, size_t obs_stride,
@@ -635,10 +660,8 @@ extern "C" int gbenv_step(gbenv *h, const uint8_t *actions_dev, uint8_t *obs_dev
 
 // Environment.step for the envs with skip_dev[e] == 0 (null: all).  A skipped env is not emulated, its wrapper state, info row
 // and observation row stay as they are, and it reports reward 0 / done 0.
-extern "C" int gbenv_step_masked(gbenv *h, const uint8_t *actions_dev, const uint8_t *skip_dev, uint8_t *obs_dev, size_t obs_stride, double *reward_dev,
-                                 uint8_t *done_dev, void *stream) {
-    if (!h || !actions_dev || !obs_dev || !reward_dev || !done_dev || obs_stride < GBENV_OBS_BYTES || (obs_stride & 3))
-        return fail(h, GBENV_E_ARG, "gbenv_step: bad argument");
+static int step_impl(gbenv *h, const uint8_t *actions_dev, const uint8_t *skip_dev, const ObsOut &o, double *reward_dev, uint8_t *done_dev,
+                     void *stream) {
     CK(cudaSetDevice(h->device));
     {
         int rce = pool_error(h);
@@ -656,13 +679,37 @@ extern "C" int gbenv_step_masked(gbenv *h, const uint8_t *actions_dev, const uin
     CK(cudaEventRecord(ev[1], st));
     int blocks = (h->n_tiles * GB_TILE + 127) / 128;
     k_wrap_step<<<blocks, 128, 0, st>>>(h->d, h->w, reward_dev, done_dev, h->d_info_rows, skip_dev);
-    k_wrap_obs<<<h->n_tiles, 256, 0, st>>>(h->d, h->w, skip_dev, obs_dev, obs_stride, 1);
+    launch_obs(h, o, skip_dev, 1, st);
     h->launches += 2;
     CK(cudaGetLastError());
     CK(cudaEventRecord(ev[2], st));
     queue_pool_error_copy(h, st);
     h->ev_step++;
     h->ev_valid = true;
+    return GBENV_OK;
+}
+
+extern "C" int gbenv_step_masked(gbenv *h, const uint8_t *actions_dev, const uint8_t *skip_dev, uint8_t *obs_dev, size_t obs_stride, double *reward_dev,
+                                 uint8_t *done_dev, void *stream) {
+    if (!h || !actions_dev || !obs_dev || !reward_dev || !done_dev || obs_stride < GBENV_OBS_BYTES || (obs_stride & 3))
+        return fail(h, GBENV_E_ARG, "gbenv_step: bad argument");
+    return step_impl(h, actions_dev, skip_dev, ObsOut{obs_dev, obs_stride, nullptr}, reward_dev, done_dev, stream);
+}
+
+extern "C" int gbenv_step_packed(gbenv *h, const uint8_t *actions_dev, const uint8_t *skip_dev, uint32_t *packed_dev, double *reward_dev,
+                                 uint8_t *done_dev, void *stream) {
+    if (!h || !actions_dev || !packed_dev || !reward_dev || !done_dev || ((uintptr_t)packed_dev & 15))
+        return fail(h, GBENV_E_ARG, "gbenv_step_packed: bad argument (NULL or misaligned buffer)");
+    return step_impl(h, actions_dev, skip_dev, ObsOut{nullptr, 0, packed_dev}, reward_dev, done_dev, stream);
+}
+
+extern "C" int gbenv_unpack_obs(gbenv *h, const uint32_t *packed_dev, int n, uint8_t *out_dev, void *stream) {
+    if (!h || n < 0 || (n && (!packed_dev || !out_dev)) || ((uintptr_t)packed_dev & 15) || ((uintptr_t)out_dev & 15))
+        return fail(h, GBENV_E_ARG, "gbenv_unpack_obs: bad argument (NULL or misaligned buffer, or n < 0)");
+    if (n == 0) return GBENV_OK;
+    CK(cudaSetDevice(h->device));
+    CK(launch_obs_unpack(packed_dev, n, out_dev, pick(h, stream)));
+    h->launches++;
     return GBENV_OK;
 }
 

@@ -12,6 +12,8 @@ while the policy looks at the other half); nothing about a single env changes --
     groups.step(actions, obs, reward, done)        # queues every group's step; returns at once
     groups.join()                                  # the caller's stream now waits for all groups (before reading obs ...)
 
+With obs_format="packed" the observation rows are u8[E, 2304] (include/gbenv.h, VecEnvironment.unpack_obs decodes them).
+
 Measured on B200 (tools/exp_groups.py): 4,096 envs 141.5 k env-steps/s as one group, 152.6 k as two, 144.1 k as four;
 32,768 envs (16 per warp: latency bound, a freed SM does not make the remaining warps faster) gain nothing.
 """
@@ -20,15 +22,19 @@ from __future__ import annotations
 from typing import List, Optional
 
 from . import _capi
-from .vec_env import device_mask, event_counts_from_flags
+from .vec_env import OBS_FORMATS, device_mask, event_counts_from_flags
 
 
 class EnvGroups:
-    def __init__(self, lib: _capi.GbEnvLib, num_envs: int, rom: bytes, n_groups: int = 2, device_id: int = 0, lanes: Optional[int] = None):
+    def __init__(self, lib: _capi.GbEnvLib, num_envs: int, rom: bytes, n_groups: int = 2, device_id: int = 0, lanes: Optional[int] = None,
+                 obs_format: str = "reference"):
         import torch
 
         if n_groups < 1 or num_envs % n_groups:
             raise ValueError("num_envs must be a multiple of n_groups")
+        if obs_format not in OBS_FORMATS:
+            raise ValueError(f"obs_format must be one of {OBS_FORMATS}, not {obs_format!r}")
+        self.packed = obs_format == "packed"
         self.torch = torch
         self.device = torch.device("cuda", device_id)
         self.num_envs, self.n_groups, self.n = int(num_envs), int(n_groups), int(num_envs) // int(n_groups)
@@ -72,19 +78,25 @@ class EnvGroups:
         self._fork()
         for g, (h, s) in enumerate(zip(self.handles, self.streams)):
             m = self._slice(mask, g)
-            if m is None:
+            if self.packed:
+                h.reset_packed(self._slice(obs, g), m, stream=s.cuda_stream, **kw)
+            elif m is None:
                 h.reset(self._slice(obs, g), stream=s.cuda_stream, **kw)
             else:
                 h.reset_dev(self._slice(obs, g), m, stream=s.cuda_stream, **kw)
         self.join()
 
     def step(self, actions, obs, reward, done, join: bool = False):
-        """Queue one env-step of every group (24 frames + reward + observation).  actions u8[E], obs u8[E, 23040], reward
+        """Queue one env-step of every group (24 frames + reward + observation).  actions u8[E], obs u8[E, 23040] (packed: u8[E, 2304]), reward
         f64[E], done u8[E], all on the device; group g uses rows [g * n, (g + 1) * n).  With join=False the call returns with
         the groups still running: call join() before the caller's stream reads the outputs."""
         self._fork()
         for g, (h, s) in enumerate(zip(self.handles, self.streams)):
-            h.step(self._slice(actions, g), self._slice(obs, g), self._slice(reward, g), self._slice(done, g), stream=s.cuda_stream)
+            a, o, r, d = (self._slice(t, g) for t in (actions, obs, reward, done))
+            if self.packed:
+                h.step_packed(a, None, o, r, d, stream=s.cuda_stream)
+            else:
+                h.step(a, o, r, d, stream=s.cuda_stream)
         if join:
             self.join()
 

@@ -3,7 +3,8 @@
 The reference is driven by a PufferLib fork (README.md:40, :116-118) that is neither in the reference tree nor installed
 here, so the contract is restated from PufferLib's published vector API (pufferlib.vector Serial / Multiprocessing, 1.0):
 
-  * observations are flat uint8 [N, 23040] (the emulation layer flattens the (72, 80, 4) Box);
+  * observations are flat uint8 [N, 23040] (the emulation layer flattens the (72, 80, 4) Box), or [N, 2304] over a
+    VecEnvironment with obs_format="packed" (the trainer decodes minibatches with VecEnvironment.unpack_obs);
   * `recv()` returns (obs, rewards, terminals, truncations, infos, env_ids, mask);
   * an env that reported `done` is reset on the NEXT `send`: that call's action for it is ignored, it is not stepped, and
     `recv` delivers its reset observation with reward 0 and terminal False (pufferlib.vector.Serial.send: `if env.done:
@@ -19,7 +20,6 @@ from __future__ import annotations
 
 import numpy as np
 
-from . import _capi
 from .info import info_row_to_dict
 from .vec_env import VecEnvironment
 
@@ -32,6 +32,7 @@ class PufferVecAdaptor:
         self.full_infos = bool(full_infos)
         self.num_envs = vec.num_envs
         self.env_ids = np.arange(self.num_envs)
+        self._row_bytes = int(np.prod(vec.observation_space.shape))
         t = vec.torch
         self._pending = t.zeros(self.num_envs, dtype=t.uint8, device=vec.device)  # envs whose episode ended on the last step
         self._any_pending = False
@@ -62,6 +63,6 @@ class PufferVecAdaptor:
 
     def recv(self):
         obs, rew, done, infos = self._last
-        flat = obs.reshape(self.num_envs, _capi.OBS_BYTES)
+        flat = obs.reshape(self.num_envs, self._row_bytes)
         mask = np.ones(self.num_envs, dtype=bool)
         return flat, rew, done, done, infos, self.env_ids, mask

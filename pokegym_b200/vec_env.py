@@ -50,6 +50,7 @@ except Exception:  # pragma: no cover - exercised implicitly
 
 
 OBS_SHAPE = (_capi.OBS_H, _capi.OBS_W, _capi.OBS_C)
+OBS_FORMATS = ("reference", "packed")
 _LIB = None
 
 
@@ -139,12 +140,19 @@ class VecEnvironment:
     obs      uint8 [N, 72, 80, 4]  (a view into `rollout[t]` when a rollout tensor is supplied)
     reward   float64 [N]           (the reference returns Python floats)
     done     bool [N]              (terminated == truncated in the reference)
+
+    obs_format="packed" stores each observation in 2,304 B instead of 23,040 (include/gbenv.h has the layout): reset() and
+    step() return uint8 [N, 2304], a rollout is [T, N, 2304], and unpack_obs() turns any set of those rows back into the
+    reference observations on the device, bit for bit.
     """
 
     def __init__(self, num_envs: int, rom_path, state_paths: Union[None, str, bytes, Sequence] = None, device="cuda:0", rollout=None,
                  auto_reset: bool = False, max_episode_steps: int = 20480, reward_scale: float = 4.0, boot_frames: int = 60,
-                 validate_actions: bool = False):
+                 validate_actions: bool = False, obs_format: str = "reference"):
         import torch
+
+        if obs_format not in OBS_FORMATS:
+            raise ValueError(f"obs_format must be one of {OBS_FORMATS}, not {obs_format!r}")
 
         self.torch = torch
         self.device = torch.device(device)
@@ -152,7 +160,9 @@ class VecEnvironment:
             raise _capi.GbEnvError("VecEnvironment runs on CUDA devices only (there is no CPU fallback)")
         self.num_envs = int(num_envs)
         self.handle = _capi.Handle(_lib(), self.num_envs, _read_rom(rom_path), device_id=self.device.index or 0)
-        self.observation_space = Box(low=0, high=255, shape=OBS_SHAPE, dtype=np.uint8)
+        self.packed = obs_format == "packed"
+        self._obs_shape = (_capi.OBS_PACKED_BYTES,) if self.packed else OBS_SHAPE  # one env's observation as step() returns it
+        self.observation_space = Box(low=0, high=255, shape=self._obs_shape, dtype=np.uint8)
         self.action_space = Discrete(_capi.NUM_ACTIONS)
         self.max_episode_steps, self.reward_scale, self.auto_reset = int(max_episode_steps), float(reward_scale), bool(auto_reset)
         self.rollout = rollout
@@ -160,7 +170,7 @@ class VecEnvironment:
         self._t = 0
         self._recorder = None
         with torch.cuda.device(self.device):
-            self._obs = torch.zeros((self.num_envs, *OBS_SHAPE), dtype=torch.uint8, device=self.device)
+            self._obs = torch.zeros((self.num_envs, *self._obs_shape), dtype=torch.uint8, device=self.device)
             self._reward = torch.zeros(self.num_envs, dtype=torch.float64, device=self.device)
             self._done = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
             self._done_prev = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
@@ -188,23 +198,34 @@ class VecEnvironment:
             return self._obs
         r = self.rollout
         ok = (self.torch.is_tensor(r) and r.dtype == self.torch.uint8 and r.device == self.device and r.is_contiguous() and r.dim() >= 3
-              and r.shape[1] == self.num_envs and r[0, 0].numel() == _capi.OBS_BYTES)
+              and r.shape[1] == self.num_envs)
+        if self.packed:
+            if not (ok and r.dim() == 3 and r.shape[2] == _capi.OBS_PACKED_BYTES):
+                raise ValueError(f"rollout must be a contiguous uint8 tensor [T, {self.num_envs}, {_capi.OBS_PACKED_BYTES}] on {self.device}")
+            return r[self._t % r.shape[0]]
+        ok = ok and r[0, 0].numel() == _capi.OBS_BYTES
         if not ok:  # raw pointers cross the C ABI: a wrong layout would be out-of-bounds device writes, not an exception
             raise ValueError(f"rollout must be a contiguous uint8 tensor [T, {self.num_envs}, 72, 80, 4] (or [T, N, 23040]) on {self.device}")
         return r[self._t % r.shape[0]]
 
+    def _reset_into(self, obs, mask):
+        if self.packed:
+            self.handle.reset_packed(obs, mask_dev=mask, max_episode_steps=self.max_episode_steps, reward_scale=self.reward_scale,
+                                     stream=self._stream())
+        else:
+            self.handle.reset_dev(obs, mask_dev=mask, max_episode_steps=self.max_episode_steps, reward_scale=self.reward_scale,
+                                  obs_stride=_capi.OBS_BYTES, stream=self._stream())
+
     # -- API -----------------------------------------------------------------
     def reset(self, mask=None, max_episode_steps: Optional[int] = None, reward_scale: Optional[float] = None):
-        """Environment.reset for every env (or those with mask[e] != 0).  Returns (obs, {})."""
+        """Environment.reset for every env (or those with mask[e] != 0).  Returns (obs, {}); obs is [N, 2304] when packed."""
         if max_episode_steps is not None:
             self.max_episode_steps = int(max_episode_steps)
         if reward_scale is not None:
             self.reward_scale = float(reward_scale)
         obs = self._obs_target()
-        mask = device_mask(mask, self.num_envs, self.device, "reset")
-        self.handle.reset_dev(obs, mask_dev=mask, max_episode_steps=self.max_episode_steps, reward_scale=self.reward_scale,
-                              obs_stride=_capi.OBS_BYTES, stream=self._stream())
-        return obs.view(self.num_envs, *OBS_SHAPE), {}
+        self._reset_into(obs, device_mask(mask, self.num_envs, self.device, "reset"))
+        return obs.view(self.num_envs, *self._obs_shape), {}
 
     def step(self, actions, skip=None):
         """Environment.step for every env.  `actions`: uint8/int tensor [N] on the device (or array-like).
@@ -221,14 +242,14 @@ class VecEnvironment:
             raise IndexError("action out of range 0..7")
         self._t += 1
         obs = self._obs_target()
-        if skip is None:
+        if self.packed:
+            if skip is not None:
+                self._check_skip(skip, obs)
+            self.handle.step_packed(actions, skip, obs, self._reward, self._done, stream=self._stream())
+        elif skip is None:
             self.handle.step(actions, obs, self._reward, self._done, obs_stride=_capi.OBS_BYTES, stream=self._stream())
         else:
-            if skip.dtype != torch.uint8 or skip.device != self.device or not skip.is_contiguous() or skip.numel() != self.num_envs:
-                raise ValueError(f"skip must be a contiguous uint8 tensor with {self.num_envs} entries on {self.device}")
-            if self.rollout is not None:  # a new rollout slot: the rows of the envs that sit out must carry over
-                prev = self.rollout[(self._t - 1) % self.rollout.shape[0]]
-                obs.view(self.num_envs, -1)[skip.bool()] = prev.view(self.num_envs, -1)[skip.bool()]
+            self._check_skip(skip, obs)
             self.handle.step_masked(actions, skip, obs, self._reward, self._done, obs_stride=_capi.OBS_BYTES, stream=self._stream())
         if self._recorder is not None:  # the frames this step ended on, before an auto-reset below
             self._recorder._capture(self._done, self._stream())
@@ -237,9 +258,29 @@ class VecEnvironment:
             # envs that just finished are reset on the device, masked by the done vector the step wrote: their row of `obs`
             # becomes the reset observation, as a vectoriser that resets after `done` would deliver it (no host round trip)
             self._done_prev.copy_(self._done)
-            self.handle.reset_dev(obs, mask_dev=self._done_prev, max_episode_steps=self.max_episode_steps, reward_scale=self.reward_scale,
-                                  obs_stride=_capi.OBS_BYTES, stream=self._stream())
-        return obs.view(self.num_envs, *OBS_SHAPE), self._reward, done, done, {}
+            self._reset_into(obs, self._done_prev)
+        return obs.view(self.num_envs, *self._obs_shape), self._reward, done, done, {}
+
+    def _check_skip(self, skip, obs):
+        if skip.dtype != self.torch.uint8 or skip.device != self.device or not skip.is_contiguous() or skip.numel() != self.num_envs:
+            raise ValueError(f"skip must be a contiguous uint8 tensor with {self.num_envs} entries on {self.device}")
+        if self.rollout is not None:  # a new rollout slot: the rows of the envs that sit out must carry over
+            prev = self.rollout[(self._t - 1) % self.rollout.shape[0]]
+            obs.view(self.num_envs, -1)[skip.bool()] = prev.view(self.num_envs, -1)[skip.bool()]
+
+    def unpack_obs(self, packed, out=None):
+        """uint8 [..., 2304] packed observations on the device (any leading dims: a step's rows, a rollout, a minibatch gathered
+        from it) -> uint8 [..., 72, 80, 4], the reference observations gbenv_step would have written, decoded on the device,
+        asynchronously.  compact_view applies to the result."""
+        torch = self.torch
+        if not (torch.is_tensor(packed) and packed.dtype == torch.uint8 and packed.device == self.device and packed.dim() >= 1
+                and packed.shape[-1] == _capi.OBS_PACKED_BYTES):
+            raise ValueError(f"packed must be a uint8 tensor [..., {_capi.OBS_PACKED_BYTES}] on {self.device}")
+        lead = tuple(packed.shape[:-1])
+        out = check_out(torch, out, (*lead, *OBS_SHAPE), torch.uint8, self.device)
+        if packed.numel():
+            self.handle.unpack_obs(packed.contiguous(), out, stream=self._stream())
+        return out
 
     def screens(self, env_ids=None, channels: int = 3, out=None):
         """uint8 [n, 144, 160, channels] device tensor: the current frame of the envs `env_ids` (None: all), grey
