@@ -168,15 +168,59 @@ struct CpuRegs {
 #define FAST_WR_BANK 0xFFFFFFFDu
 #define FAST_WR_P1 0xFFFFFFFCu  // the joypad select register: the stored byte is Interaction.pull of the written one
 __device__ __forceinline__ uint32_t mem_offset(uint32_t i) { return ((i >> 2) << 7) | (i & 3); }
-__device__ __forceinline__ uint32_t fast_store_target(uint32_t a) {  // single-lane build: first match wins
-    if (a - 0xC000u < 0x3E00u) return mem_offset(MEM_WRAM + (a & 0x1FFF));                               // WRAM and its echo
-    if (a - 0xFF80u < 0x7Fu || a - 0xFE00u < 0x100u) return mem_offset(MEM_HI + (a - 0xFE00));             // HRAM, OAM
-    if (a - 0x8000u < 0x2000u) return mem_offset(MEM_VRAM + (a - 0x8000));                                // VRAM
-    if (a - 0x2000u < 0x2000u) return FAST_WR_BANK;
-    if (a - 0xFF10u < 0x30u) return FAST_WR_DROP;
-    if (a == 0xFF00u) return FAST_WR_P1;
-    return FAST_WR_NONE;
+// Memory map of the single-lane fast body as one table lookup instead of a first-match compare chain: the compares ran on the
+// integer ALU pipe (half rate on sm_100), the lookup goes to the constant cache.  Key: the page (a >> 8) below 0xFF00, one
+// entry per byte from there on (IO registers and HRAM differ byte by byte): max(a >> 8, a - 0xFE01) as signed numbers, so key
+// 255 is 0xFF00 and 0xFF01..0xFFFF are 256..510.  ROM (a < 0x8000) is not looked up: its bank offset changes at run time.
+// Entry: GB_MAP_* flags; bits 14 and 18 (GB_MAP_BASE): B << 5, where byte index (a & 0x1FFF) + B of the env's plain-RAM
+// array holds address a (B = 0 for VRAM, 0x2000 for work RAM and its echo, 0x2200 for 0xFE00-0xFFFF); an entry that is
+// not plain RAM for stores carries the low nibble of its FAST_WR_* code.
+#define GB_MAP_RD 0x01000000u     // the fast body reads plain RAM here (VRAM, work RAM + echo, OAM page, P1 / SB / SC / 0xFF03, HRAM)
+#define GB_MAP_WR 0x02000000u     // the fast body stores to plain RAM here
+#define GB_MAP_DEFER MODE_DEFER   // VRAM / OAM page: stores go through the slow tick while the mode word has MODE_DEFER
+#define GB_MAP_BASE 0x00044000u
+__host__ __device__ constexpr uint32_t gb_map_entry(uint32_t k) {
+    return k >= 255 ? ((k - 255 >= 0x80u && k - 255 < 0xFFu) ? (GB_MAP_RD | GB_MAP_WR | 0x44000u)  // HRAM
+                       : k - 255 < 4u ? (GB_MAP_RD | 0x44000u | (k == 255 ? 0xCu : 0xFu))             // P1 (store: FAST_WR_P1), SB, SC, 0xFF03
+                       : k - 255 - 0x10u < 0x30u ? 0xEu                                               // sound: stores dropped
+                       : 0xFu)
+         : k - 0x80u < 0x20u ? (GB_MAP_RD | GB_MAP_WR | GB_MAP_DEFER)                                 // VRAM
+         : k - 0xC0u < 0x3Eu ? (GB_MAP_RD | GB_MAP_WR | 0x40000u)                                     // work RAM and its echo
+         : k == 0xFEu ? (GB_MAP_RD | GB_MAP_WR | GB_MAP_DEFER | 0x44000u)                            // OAM, 0xFEA0-0xFEFF
+         : k - 0x20u < 0x20u ? 0xDu                                                                   // MBC3 ROM bank select
+         : 0xFu;
 }
+#define GB_MAP_E2(k) gb_map_entry(k), gb_map_entry((k) + 1)
+#define GB_MAP_E8(k) GB_MAP_E2(k), GB_MAP_E2((k) + 2), GB_MAP_E2((k) + 4), GB_MAP_E2((k) + 6)
+#define GB_MAP_E32(k) GB_MAP_E8(k), GB_MAP_E8((k) + 8), GB_MAP_E8((k) + 16), GB_MAP_E8((k) + 24)
+#define GB_MAP_E128(k) GB_MAP_E32(k), GB_MAP_E32((k) + 32), GB_MAP_E32((k) + 64), GB_MAP_E32((k) + 96)
+__constant__ uint32_t c_mem_map[512] = {GB_MAP_E128(0u), GB_MAP_E128(128u), GB_MAP_E128(256u), GB_MAP_E128(384u)};
+__device__ __forceinline__ uint32_t gb_map_key(uint32_t a) {
+    const int k = (int)(a >> 8), kb = (int)a - 0xFE01;
+    return (uint32_t)(k > kb ? k : kb);
+}
+// byte offset of `a` inside the env's interleaved array, given its map entry (meaningful where the entry is plain RAM)
+__device__ __forceinline__ uint32_t gb_map_offset(uint32_t a, uint32_t e) {
+    return ((((a & 0x1FFCu) << 5) + (e & GB_MAP_BASE)) | (a & 3u));
+}
+// single-lane build: the store target (fast_store_target's codes) and the map entry
+__device__ __forceinline__ uint32_t fast_store_target_map(uint32_t a, uint32_t &e) {
+    e = c_mem_map[gb_map_key(a)];
+    return (e & GB_MAP_WR) ? gb_map_offset(a, e) : (e | 0xFFFFFFF0u);
+}
+// Z, N and H of INC / DEC from the result byte: entry [256 + b] for INC b, [b] for DEC b = res | flags << 8 without C
+__host__ __device__ constexpr uint32_t gb_incdec_entry(uint32_t k) {
+    return k < 256 ? (((k - 1) & 0xFFu) | ((((k - 1) & 0xFFu) == 0 ? 0x80u : 0u) | 0x40u | (((k - 1) & 0xFu) == 0xFu ? 0x20u : 0u)) << 8)
+                   : (((k + 1) & 0xFFu) | ((((k + 1) & 0xFFu) == 0 ? 0x80u : 0u) | (((k + 1) & 0xFu) == 0 ? 0x20u : 0u)) << 8);
+}
+#define GB_INCDEC_E2(k) gb_incdec_entry(k), gb_incdec_entry((k) + 1)
+#define GB_INCDEC_E8(k) GB_INCDEC_E2(k), GB_INCDEC_E2((k) + 2), GB_INCDEC_E2((k) + 4), GB_INCDEC_E2((k) + 6)
+#define GB_INCDEC_E32(k) GB_INCDEC_E8(k), GB_INCDEC_E8((k) + 8), GB_INCDEC_E8((k) + 16), GB_INCDEC_E8((k) + 24)
+#define GB_INCDEC_E128(k) GB_INCDEC_E32(k), GB_INCDEC_E32((k) + 32), GB_INCDEC_E32((k) + 64), GB_INCDEC_E32((k) + 96)
+__constant__ uint32_t c_incdec[512] = {GB_INCDEC_E128(0u), GB_INCDEC_E128(128u), GB_INCDEC_E128(256u), GB_INCDEC_E128(384u)};
+// ROM bank offset for a bank count that is not a power of two: an integer division, kept out of the hot bodies
+__device__ GB_NOINLINE uint32_t rom_off_mod(uint32_t bank, uint32_t banks) { return (bank % banks) * 0x4000u - 0x4000u; }
+
 // Plain RAM behind address `a`: work RAM and its echo, VRAM, OAM / 0xFEA0-0xFEFF, HRAM (0xFF80-0xFFFE).  Returns whether it
 // is, and the byte offset inside the env's interleaved array (meaningless otherwise).  Selects only.
 __device__ __forceinline__ bool fast_plain_offset(uint32_t a, uint32_t &off) {
@@ -214,11 +258,12 @@ __device__ __forceinline__ bool cpu_exec(Machine &m, const uint4 d, CpuRegs &r, 
         if (!SIMT) return false; \
         declined = true;       \
     } while (0)
-    auto rd8 = [&](uint32_t a) -> uint32_t {  // Motherboard.getitem; FAST: WRAM (+ echo), ROM and HRAM, else decline
+    auto rd8 = [&](uint32_t a) -> uint32_t {  // Motherboard.getitem; FAST: WRAM (+ echo), ROM, then what c_mem_map marks readable, else decline
         if (FAST) {
             if (a - 0xC000u < 0x3E00u) return memb[mem_offset(MEM_WRAM + (a & 0x1FFF))];
             if (a < 0x8000u) return __ldg(rom + (a + (a >> 14) * rom_off));
-            if (a - 0xFF80u < 0x7Fu || a - 0xFF00u < 4u) return memb[mem_offset(MEM_HI + (a - 0xFE00))];  // HRAM; P1, SB, SC
+            const uint32_t e = c_mem_map[gb_map_key(a)];
+            if (e & GB_MAP_RD) return memb[gb_map_offset(a, e)];
             declined = true;
             return 0;
         }
@@ -264,9 +309,10 @@ __device__ __forceinline__ bool cpu_exec(Machine &m, const uint4 d, CpuRegs &r, 
             }
         } else {  // single-lane build: branches are free (nothing diverges), the first matching region wins
             if (FAST && (wf & PDF_WR)) {
-                wt = fast_store_target(wa);
+                uint32_t e;
+                wt = fast_store_target_map(wa, e);
                 if (wt == FAST_WR_NONE) FAST_DECLINE();
-                if ((mode & MODE_DEFER) && (wa - 0x8000u < 0x2000u || wa - 0xFE00u < 0x100u)) FAST_DECLINE();  // render_flush first
+                if (mode & e & GB_MAP_DEFER) FAST_DECLINE();  // VRAM / OAM with the deferred PPU: render_flush first
             }
             if (wf & PDF_RD) {
                 v = rd8(wa);
@@ -293,6 +339,10 @@ __device__ __forceinline__ bool cpu_exec(Machine &m, const uint4 d, CpuRegs &r, 
         // rv = v
     } else if (!SIMT && (wf & PDF_JUMP)) {
         if (((f ^ ex) & op) == 0) { next_pc = imm16; cyc += ex & 0xF; }
+    } else if (FAST && !SIMT && (wf & PDF_INCDEC)) {  // op = +1 / -1 (mod 256): result, Z, N and H from c_incdec, C kept
+        // index: the operand byte, bytes 1..3 the sign of op (PRMT sign replication): b for INC, b - 256 for DEC
+        rv = c_incdec[256 + (int)gb_prmt(v, d.x, 0xDDD0u)] | ((hlaf >> 16) & (FLAG_C << 8));
+        wv = rv;
     } else if (!SIMT && (wf & PDF_INCDEC)) {  // op = +1 / -1 (mod 256), ex = 0 / N|H: DEC inverts the half carry like a subtraction
         const uint32_t b = v & 0xFF, sum = b + op, res = sum & 0xFF;
         const uint32_t nf = (f & FLAG_C) | ((((b ^ op ^ sum) & 0x10) << 1) ^ ex) | (res == 0 ? FLAG_Z : 0);
@@ -466,7 +516,8 @@ __device__ __forceinline__ bool cpu_exec(Machine &m, const uint4 d, CpuRegs &r, 
                 uint32_t bank = wv & 0x7F;
                 bank = bank ? bank : 1;
                 m.rombank = bank;
-                rom_off = (bank_mask ? (bank & bank_mask) : (bank % m.rom_banks)) * 0x4000u - 0x4000u;
+                if (SIMT) rom_off = (bank_mask ? (bank & bank_mask) : (bank % m.rom_banks)) * 0x4000u - 0x4000u;
+                else rom_off = bank_mask ? (bank & bank_mask) * 0x4000u - 0x4000u : rom_off_mod(bank, m.rom_banks);
                 m.rom_off = rom_off;
             }
         } else {
