@@ -32,9 +32,10 @@
 extern "C" {
 #endif
 
-#define GBENV_ABI_VERSION 7 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
+#define GBENV_ABI_VERSION 8 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
                                4: gbenv_counts_map_sum, gbenv_reduce_info_masked; 5: gbenv_capture_frames, gbenv_frames_to_rgb;
-                               6: gbenv_event_flags; 7: gbenv_step_packed, gbenv_reset_packed, gbenv_unpack_obs */
+                               6: gbenv_event_flags; 7: gbenv_step_packed, gbenv_reset_packed, gbenv_unpack_obs;
+                               8: gbenv_save_states */
 
 #define GBENV_STATE_BYTES 142610 /* PyBoy v9 save-state length (SURVEY.md 8c)              */
 #define GBENV_OBS_H 72           /* environment.py:154-166: (144//2, 160//2, 4) uint8       */
@@ -96,6 +97,16 @@ int gbenv_set_initial_template(gbenv_t *h, const int32_t *env_ids_host, int n, i
 int gbenv_power_on(gbenv_t *h, const int32_t *env_ids_host, int n);
 /* PyBoy.save_state: v9 blob of one env, synchronous. */
 int gbenv_save_state(gbenv_t *h, int env, uint8_t *blob_host /* GBENV_STATE_BYTES */);
+/* PyBoy.save_state for a list of envs: the v9 file of each listed env, GBENV_STATE_BYTES each, into
+ * blobs_dev uint8[n][GBENV_STATE_BYTES] (rows contiguous, so row i is a complete .state file that gbenv_add_state_template
+ * and PyBoy both load).  The contract is gbenv_capture_frames' / gbenv_event_flags': env_ids_dev is int32[n] on the device,
+ * any order, duplicates allowed; NULL means envs 0..n-1 (n <= n_envs).  A row whose id is outside [0, n_envs) is left
+ * untouched and nothing is read for it.  Asynchronous on `stream` and ordered after earlier calls on the handle.  For a
+ * valid id the row is bit-identical to what gbenv_save_state returns for that env at the same point in call order
+ * (gbenv_save_state is this call for one env followed by a copy to the host).  GBENV_E_ARG on a NULL handle, a NULL or
+ * non-16-byte-aligned blobs_dev with n > 0, n < 0, or NULL ids with n > n_envs; n == 0 is a successful no-op.
+ * The output is large (584 MB for 4,096 envs); pass ids to save fewer.                                                */
+int gbenv_save_states(gbenv_t *h, const int32_t *env_ids_dev, int n, uint8_t *blobs_dev, void *stream);
 
 /* ---- (1)+(2) emulator: tick loop + PPU ------------------------------------------------------
  * replaces pyboy_binding.run_action_on_emulator (:71-91): press, 24 x tick (release before tick 8,

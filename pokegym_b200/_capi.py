@@ -18,7 +18,7 @@ STATE_BYTES = 142_610
 OBS_H, OBS_W, OBS_C = 72, 80, 4
 OBS_BYTES = OBS_H * OBS_W * OBS_C
 INFO_SCALARS = 72
-ABI_VERSION = 7
+ABI_VERSION = 8
 COUNTS_H, COUNTS_W = 444, 436
 SCREEN_H, SCREEN_W = 144, 160
 FRAME_WORDS = 1440  # packed frame: 144 lines x 10 uint32 words of 16 2-bit shades (include/gbenv.h)
@@ -98,6 +98,7 @@ _SIGS = {
     "set_initial_template": ([C.c_void_p, C.c_void_p, C.c_int, C.c_int], C.c_int),
     "power_on": ([C.c_void_p, C.c_void_p, C.c_int], C.c_int),
     "save_state": ([C.c_void_p, C.c_int, C.c_void_p], C.c_int),
+    "save_states": ([C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p], C.c_int),
     "run_action": ([C.c_void_p, C.c_void_p, C.c_int, C.c_void_p], C.c_int),
     "tick": ([C.c_void_p, C.c_int, C.c_int, C.c_void_p], C.c_int),
     "send_input": ([C.c_void_p, C.c_int, C.c_int, C.c_void_p], C.c_int),
@@ -213,6 +214,13 @@ class Handle:
         out = np.empty(STATE_BYTES, dtype=np.uint8)
         self._check(self.lib.save_state(self._h, int(env), _ptr(out)), "save_state")
         return out.tobytes()
+
+    def save_states(self, out, env_ids=None, stream=None):
+        """The v9 .state file of the envs `env_ids` (int32, on the device for CUDA, host memory for the oracle; None: envs
+        0..len(out)-1) -> out uint8 [n, STATE_BYTES], each row what save_state() returns for its env.  Rows of ids outside
+        [0, n_envs) are left untouched."""
+        n = _byte_rows(out, STATE_BYTES, "out", None if env_ids is None else len(env_ids))
+        self._check(self.lib.save_states(self._h, _ptr(env_ids), int(n), _ptr(out), C.c_void_p(stream or 0)), "save_states")
 
     # -- emulator ------------------------------------------------------------
     def run_action(self, actions, frame_skip: int = ACT_FREQ, stream: int = 0):

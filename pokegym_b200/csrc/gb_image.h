@@ -1,4 +1,5 @@
-// gb_image.h -- PyBoy save-state blob <-> canonical per-env image (host code).
+// gb_image.h -- PyBoy save-state blob <-> canonical per-env image (host code), and the v9 section table the device
+// serialiser shares.
 //
 // The canonical image is the linear word layout of gb_layout.cuh (IMG_*): what state templates hold on the device and
 // what k_scatter_image / k_gather_image move in and out of the interleaved arrays.  Shared by libgbenv.so (gbenv.cu)
@@ -23,6 +24,121 @@ static inline uint8_t img_get_byte(const std::vector<uint32_t> &img, uint32_t ba
 }
 
 static const uint32_t SHADE_WORDS[4] = {0xFFFFFF01u, 0x99999900u, 0x55555500u, 0x00000000u};
+
+// ---- The PyBoy v9 file as a table of sections over the canonical image (SURVEY.md 8c).  This is the one definition of the
+// v9 layout on the C++ side: image_to_blob (host; also tests/hostsim) and k_save_states (gb_state.cu) both serialise from
+// it.  A section is a run of file bytes [off, off + len) with one source:
+//   SK_CONST  every byte is `src`
+//   SK_FIELD  one byte, (image word src >> shift) & mask  (the flag bits of R_INT, next_stat_mode)
+//   SK_BYTES  image bytes src .. src + len - 1, image byte i being byte i & 3 of image word i >> 2 (RAM, register bytes)
+//   SK_LP     144 scanline records of 5 bytes: the 4 bytes of IMG_LP word 2y, then bit 4 of word 2y + 1
+//   SK_FB     one PyBoy word per pixel, little-endian: SHADE_WORDS of the 2-bit shade, 16 pixels per IMG_FB word
+enum : uint8_t { SK_CONST, SK_FIELD, SK_BYTES, SK_LP, SK_FB };
+struct StateSection {
+    uint32_t off, len, src;
+    uint8_t kind, shift, mask;
+};
+#define STATE_SECTIONS 42
+struct StateLayout {
+    StateSection s[STATE_SECTIONS];
+};
+
+constexpr uint32_t state_reg_byte(uint32_t r, uint32_t byte) { return (IMG_REGS + r) * 4u + byte; }
+
+constexpr StateLayout make_state_layout() {
+    StateLayout t{};
+    uint32_t off = 0;
+    int i = 0;
+    struct Add {
+        StateLayout &t;
+        uint32_t &off;
+        int &i;
+        constexpr void operator()(uint8_t kind, uint32_t len, uint32_t src, uint8_t shift = 0, uint8_t mask = 0xFF) {
+            t.s[i].off = off; t.s[i].len = len; t.s[i].src = src; t.s[i].kind = kind; t.s[i].shift = shift; t.s[i].mask = mask;
+            off += len;
+            i++;
+        }
+    } add{t, off, i};
+    add(SK_CONST, 1, 9);                                  // version
+    add(SK_BYTES, 4, state_reg_byte(R_HDR, 0));           // bootrom_enabled, key1, double_speed, cgb
+    add(SK_BYTES, 2, state_reg_byte(R_HLAF, 2));          // A F
+    add(SK_BYTES, 1, state_reg_byte(R_BCDE, 1));          // B
+    add(SK_BYTES, 1, state_reg_byte(R_BCDE, 0));          // C
+    add(SK_BYTES, 1, state_reg_byte(R_BCDE, 3));          // D
+    add(SK_BYTES, 1, state_reg_byte(R_BCDE, 2));          // E
+    add(SK_BYTES, 2, state_reg_byte(R_HLAF, 0));          // HL
+    add(SK_BYTES, 4, state_reg_byte(R_SPPC, 0));          // SP PC
+    add(SK_FIELD, 1, IMG_REGS + R_INT, 0, 1);             // IME
+    add(SK_FIELD, 1, IMG_REGS + R_INT, 1, 1);             // halted
+    add(SK_FIELD, 1, IMG_REGS + R_INT, 2, 1);             // stopped
+    add(SK_BYTES, 1, state_reg_byte(R_INT, 1));           // IE
+    add(SK_FIELD, 1, IMG_REGS + R_INT, 3, 1);             // interrupt_queued
+    add(SK_BYTES, 1, state_reg_byte(R_INT, 2));           // IF
+    add(SK_BYTES, 0x2000, IMG_MEM * 4 + MEM_VRAM);        // VRAM
+    add(SK_BYTES, 0xA0, IMG_MEM * 4 + MEM_HI);            // OAM
+    add(SK_BYTES, 1, state_reg_byte(R_LCD0, 0));          // LCDC
+    add(SK_BYTES, 3, state_reg_byte(R_LCD2, 0));          // BGP OBP0 OBP1
+    add(SK_BYTES, 3, state_reg_byte(R_LCD0, 1));          // STAT LY LYC
+    add(SK_BYTES, 4, state_reg_byte(R_LCD1, 0));          // SCY SCX WY WX
+    add(SK_BYTES, 1, state_reg_byte(R_HDR, 3));           // cgb
+    add(SK_BYTES, 1, state_reg_byte(R_HDR, 2));           // double_speed
+    add(SK_BYTES, 4, state_reg_byte(R_CLOCK, 0));         // clock (u64; the emulator keeps 32 bits)
+    add(SK_CONST, 4, 0);
+    add(SK_BYTES, 4, state_reg_byte(R_TARGET, 0));        // clock_target (u64)
+    add(SK_CONST, 4, 0);
+    add(SK_FIELD, 1, IMG_REGS + R_LCD2, 26, 3);           // next_stat_mode
+    add(SK_LP, 144 * 5, IMG_LP);                          // scanline parameters
+    add(SK_FB, 144 * 160 * 4, IMG_FB);                    // screen
+    add(SK_BYTES, 0x2000, IMG_MEM * 4 + MEM_WRAM);        // WRAM
+    add(SK_BYTES, 96, IMG_MEM * 4 + MEM_HI + 0xA0);       // FEA0-FEFF
+    add(SK_BYTES, 76, IMG_MEM * 4 + MEM_HI + 0x100);      // IO FF00-FF4B
+    add(SK_BYTES, 127, IMG_MEM * 4 + MEM_HI + 0x180);     // HRAM
+    add(SK_BYTES, 52, IMG_MEM * 4 + MEM_HI + 0x14C);      // FF4C-FF7F
+    add(SK_BYTES, 2, state_reg_byte(R_TIMER, 0));         // DIV TIMA
+    add(SK_BYTES, 2, state_reg_byte(R_DIVC, 0));          // DIV_counter (u16)
+    add(SK_BYTES, 2, state_reg_byte(R_TIMAC, 0));         // TIMA_counter (u16)
+    add(SK_BYTES, 2, state_reg_byte(R_TIMER, 2));         // TMA TAC
+    add(SK_BYTES, 4, state_reg_byte(R_MBC, 0));           // rombank rambank ram_enabled memorymodel
+    add(SK_BYTES, CRAM_BYTES, IMG_CRAM * 4);              // cartridge RAM
+    add(SK_BYTES, 2, state_reg_byte(R_JOY, 0));           // joypad directional, standard
+    return t;
+}
+
+static constexpr StateLayout STATE_LAYOUT = make_state_layout();
+static_assert(STATE_LAYOUT.s[STATE_SECTIONS - 1].off + STATE_LAYOUT.s[STATE_SECTIONS - 1].len == GBENV_STATE_BYTES, "v9 file length");
+static_assert(STATE_LAYOUT.s[15].off == 23 && STATE_LAYOUT.s[30].off == 101285, "VRAM and WRAM offsets (SURVEY.md 8c)");
+
+// the PyBoy framebuffer word of shade s (SHADE_WORDS[s]): grey in bytes 1..3, the colour-0 flag byte set for white
+__host__ __device__ inline uint32_t state_shade_word(uint32_t s) { return ((0x005599FFu >> (8 * s)) & 0xFF) * 0x01010100u | (s == 0); }
+
+// the image word file byte o (inside section s, which is not SK_CONST) is taken from
+__host__ __device__ constexpr uint32_t state_word(const StateSection &s, uint32_t o) {
+    const uint32_t r = o - s.off;
+    return s.kind == SK_FIELD ? s.src
+         : s.kind == SK_BYTES ? (s.src + r) >> 2
+         : s.kind == SK_LP    ? IMG_LP + 2 * (r / 5) + (r % 5 == 4)
+                              : IMG_FB + (r >> 6);
+}
+// file byte o (inside section s) given w = image word state_word(s, o) (ignored for SK_CONST)
+__host__ __device__ inline uint8_t state_byte(const StateSection &s, uint32_t o, uint32_t w) {
+    const uint32_t r = o - s.off;
+    switch (s.kind) {
+    case SK_CONST: return (uint8_t)s.src;
+    case SK_FIELD: return (uint8_t)((w >> s.shift) & s.mask);
+    case SK_BYTES: return (uint8_t)(w >> (8 * ((s.src + r) & 3)));
+    case SK_LP: return (uint8_t)(r % 5 == 4 ? (w >> 4) & 1 : w >> (8 * (r % 5)));
+    default: return (uint8_t)(state_shade_word((w >> (2 * ((r >> 2) & 15))) & 3) >> (8 * (r & 3)));
+    }
+}
+// index of the section that holds file byte o
+__host__ __device__ constexpr int state_section_of(const StateLayout &t, uint32_t o) {
+    int lo = 0, hi = STATE_SECTIONS - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (t.s[mid].off <= o) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
 
 // PyBoy v9 / v7 blob -> canonical image (layout: SURVEY.md 8c).  Returns 0 or a negative error.
 static int blob_to_image(const uint8_t *b, size_t len, std::vector<uint32_t> &img, int *version_out, std::string &err) {
@@ -105,47 +221,9 @@ static int blob_to_image(const uint8_t *b, size_t len, std::vector<uint32_t> &im
     return GBENV_OK;
 }
 
-static void image_to_blob(const std::vector<uint32_t> &img, uint8_t *b) {
-    const uint32_t *regs = &img[IMG_REGS];
-    uint8_t *p = b;
-    uint32_t hdr = regs[R_HDR];
-    *p++ = 9; *p++ = hdr & 0xFF; *p++ = (hdr >> 8) & 0xFF; *p++ = (hdr >> 16) & 0xFF; *p++ = hdr >> 24;
-    uint32_t bcde = regs[R_BCDE], hlaf = regs[R_HLAF], sppc = regs[R_SPPC], in = regs[R_INT];
-    *p++ = (hlaf >> 16) & 0xFF; *p++ = hlaf >> 24; *p++ = (bcde >> 8) & 0xFF; *p++ = bcde & 0xFF; *p++ = bcde >> 24; *p++ = (bcde >> 16) & 0xFF;
-    *p++ = hlaf & 0xFF; *p++ = (hlaf >> 8) & 0xFF;
-    *p++ = sppc & 0xFF; *p++ = (sppc >> 8) & 0xFF; *p++ = (sppc >> 16) & 0xFF; *p++ = sppc >> 24;
-    *p++ = in & 1; *p++ = (in >> 1) & 1; *p++ = (in >> 2) & 1; *p++ = (in >> 8) & 0xFF; *p++ = (in >> 3) & 1; *p++ = (in >> 16) & 0xFF;
-    for (uint32_t i = 0; i < 0x2000; i++) *p++ = img_get_byte(img, IMG_MEM, MEM_VRAM + i);
-    for (uint32_t i = 0; i < 0xA0; i++) *p++ = img_get_byte(img, IMG_MEM, MEM_HI + i);
-    uint32_t l0 = regs[R_LCD0], l1 = regs[R_LCD1], l2 = regs[R_LCD2];
-    *p++ = l0 & 0xFF; *p++ = l2 & 0xFF; *p++ = (l2 >> 8) & 0xFF; *p++ = (l2 >> 16) & 0xFF; *p++ = (l0 >> 8) & 0xFF; *p++ = (l0 >> 16) & 0xFF; *p++ = l0 >> 24;
-    *p++ = l1 & 0xFF; *p++ = (l1 >> 8) & 0xFF; *p++ = (l1 >> 16) & 0xFF; *p++ = l1 >> 24;
-    *p++ = hdr >> 24; *p++ = (hdr >> 16) & 0xFF;
-    uint64_t clock = regs[R_CLOCK], target = regs[R_TARGET];
-    for (int i = 0; i < 8; i++) { *p++ = (uint8_t)clock; clock >>= 8; }
-    for (int i = 0; i < 8; i++) { *p++ = (uint8_t)target; target >>= 8; }
-    *p++ = (l2 >> 26) & 3;
-    for (uint32_t y = 0; y < 144; y++) {
-        uint32_t w0 = img[IMG_LP + 2 * y], w1 = img[IMG_LP + 2 * y + 1];
-        *p++ = w0 & 0xFF; *p++ = (w0 >> 8) & 0xFF; *p++ = (w0 >> 16) & 0xFF; *p++ = w0 >> 24; *p++ = (w1 >> 4) & 1;
-    }
-    for (uint32_t i = 0; i < 144 * 160; i++) {
-        uint32_t wv = SHADE_WORDS[(img[IMG_FB + (i >> 4)] >> (2 * (i & 15))) & 3];
-        *p++ = (uint8_t)wv; *p++ = (uint8_t)(wv >> 8); *p++ = (uint8_t)(wv >> 16); *p++ = (uint8_t)(wv >> 24);
-    }
-    for (uint32_t i = 0; i < 0x2000; i++) *p++ = img_get_byte(img, IMG_MEM, MEM_WRAM + i);
-    for (uint32_t i = 0; i < 96; i++) *p++ = img_get_byte(img, IMG_MEM, MEM_HI + 0xA0 + i);
-    for (uint32_t i = 0; i < 76; i++) *p++ = img_get_byte(img, IMG_MEM, MEM_HI + 0x100 + i);
-    for (uint32_t i = 0; i < 127; i++) *p++ = img_get_byte(img, IMG_MEM, MEM_HI + 0x180 + i);
-    for (uint32_t i = 0; i < 52; i++) *p++ = img_get_byte(img, IMG_MEM, MEM_HI + 0x14C + i);
-    uint32_t t = regs[R_TIMER];
-    *p++ = t & 0xFF; *p++ = (t >> 8) & 0xFF;
-    *p++ = regs[R_DIVC] & 0xFF; *p++ = (regs[R_DIVC] >> 8) & 0xFF; *p++ = regs[R_TIMAC] & 0xFF; *p++ = (regs[R_TIMAC] >> 8) & 0xFF;
-    *p++ = (t >> 16) & 0xFF; *p++ = t >> 24;
-    uint32_t mb = regs[R_MBC];
-    *p++ = mb & 0xFF; *p++ = (mb >> 8) & 0xFF; *p++ = (mb >> 16) & 0xFF; *p++ = mb >> 24;
-    for (uint32_t i = 0; i < 0x8000; i++) *p++ = img_get_byte(img, IMG_CRAM, i);
-    *p++ = regs[R_JOY] & 0xFF; *p++ = (regs[R_JOY] >> 8) & 0xFF;
+static inline void image_to_blob(const std::vector<uint32_t> &img, uint8_t *b) {
+    for (const StateSection &s : STATE_LAYOUT.s)
+        for (uint32_t o = s.off; o < s.off + s.len; o++) b[o] = state_byte(s, o, s.kind == SK_CONST ? 0u : img[state_word(s, o)]);
 }
 
 // fresh post-boot DMG machine (our convention; mirrors oracle gb_power_on)

@@ -169,17 +169,6 @@ __global__ void __launch_bounds__(32 * RENDER_LINES_PER_BLOCK) k_render_pending(
 #endif
 
 // ---------------------------------------------------------------------------------------------
-// Canonical per-env image <-> interleaved arrays.  image word j of env e lives at:
-//   IMG_MEM..: mem, IMG_CRAM..: cram, IMG_FB..: fb, IMG_LP..: lp (pair-interleaved), IMG_REGS..: regs
-__device__ __forceinline__ uint32_t *image_slot(const DevArrays &d, int env, uint32_t j) {
-    int tile = env >> 5, lane = env & 31;
-    if (j < IMG_CRAM) return d.mem + il_index(tile, MEM_WORDS, j - IMG_MEM, lane);
-    if (j < IMG_FB) return d.cram + il_index(tile, CRAM_WORDS, j - IMG_CRAM, lane);
-    if (j < IMG_LP) return d.fb + il_index(tile, FB_WORDS, j - IMG_FB, lane);
-    if (j < IMG_REGS) return d.lp + lp_index(tile, j - IMG_LP, lane);
-    return d.regs + il_index(tile, R_WORDS, j - IMG_REGS, lane);
-}
-
 // PyBoy load_state semantics that depend on the env's previous state (oracle GBQ_STAT_LOAD_KEEPS_MODE):
 // STAT bits 0-2 and STATRegister._mode survive a load; LCD-off states force mode 0 through set_lcdc.
 // For v7 blobs clock / clock_target / next_stat_mode / IF / interrupt_queued are not in the file.

@@ -98,3 +98,14 @@ __host__ __device__ inline size_t il_index(int tile, uint32_t words_per_env, uin
 __host__ __device__ inline size_t lp_index(int tile, uint32_t w, int lane) {
     return (size_t)tile * LP_WORDS * GB_TILE + ((size_t)(w >> 1) * GB_TILE + (size_t)lane) * 2 + (w & 1);
 }
+
+// Canonical per-env image <-> interleaved arrays.  image word j of env e lives at:
+//   IMG_MEM..: mem, IMG_CRAM..: cram, IMG_FB..: fb, IMG_LP..: lp (pair-interleaved), IMG_REGS..: regs
+__device__ __forceinline__ uint32_t *image_slot(const DevArrays &d, int env, uint32_t j) {
+    int tile = env >> 5, lane = env & 31;
+    if (j < IMG_CRAM) return d.mem + il_index(tile, MEM_WORDS, j - IMG_MEM, lane);
+    if (j < IMG_FB) return d.cram + il_index(tile, CRAM_WORDS, j - IMG_CRAM, lane);
+    if (j < IMG_LP) return d.fb + il_index(tile, FB_WORDS, j - IMG_FB, lane);
+    if (j < IMG_REGS) return d.lp + lp_index(tile, j - IMG_LP, lane);
+    return d.regs + il_index(tile, R_WORDS, j - IMG_REGS, lane);
+}

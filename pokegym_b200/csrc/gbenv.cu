@@ -15,6 +15,7 @@
 #include "gb_image.h"
 #include "gb_kernels.cuh"
 #include "gb_obs.cuh"
+#include "gb_state.cuh"
 #include "gb_wrap.cuh"
 
 struct StateTemplate {
@@ -36,6 +37,7 @@ struct gbenv {
     bool loads_pending = false;         // some env may still have its first reset (which loads its save-state) ahead
     unsigned long long *d_counters = nullptr;
     uint32_t *d_stage_image = nullptr;
+    uint8_t *d_stage_blob = nullptr;  // GBENV_STATE_BYTES, gbenv_save_state
     uint8_t *d_stage_buf = nullptr;  // 64 KiB scratch for bus access
     double *d_info_rows = nullptr;
     int32_t *d_env_ids = nullptr;
@@ -161,7 +163,7 @@ extern "C" int gbenv_destroy(gbenv *h) {
     cudaFree(h->w.ctl);
     if (h->pool_err_host) cudaFreeHost(h->pool_err_host);
     cudaFree(h->d_cm_dense);
-    cudaFree(h->d_counters); cudaFree(h->d_stage_image); cudaFree(h->d_stage_buf); cudaFree(h->d_info_rows);
+    cudaFree(h->d_counters); cudaFree(h->d_stage_image); cudaFree(h->d_stage_blob); cudaFree(h->d_stage_buf); cudaFree(h->d_info_rows);
     cudaFree(h->d_env_ids); cudaFree(h->d_mask); cudaFree(h->d_init_tmpl); cudaFree(h->d_tmpl_images); cudaFree(h->d_tmpl_versions);
     for (int k = 0; k < 2; k++) {
         cudaFree(h->d_actions[k]); cudaFree(h->d_obs[k]); cudaFree(h->d_done[k]); cudaFree(h->d_reward[k]);
@@ -283,6 +285,7 @@ static int create_impl(gbenv *&h, int n_envs, const uint8_t *rom_host, size_t ro
     }
     ALLOC(h->d_counters, 8 * sizeof(unsigned long long));
     ALLOC(h->d_stage_image, IMG_WORDS * sizeof(uint32_t));
+    ALLOC(h->d_stage_blob, GBENV_STATE_BYTES);
     ALLOC(h->d_stage_buf, 0x10000);
     ALLOC(h->d_info_rows, (size_t)n_envs * GBENV_INFO_SCALARS * sizeof(double));
     ALLOC(h->d_env_ids, (size_t)n_envs * sizeof(int32_t));
@@ -393,17 +396,24 @@ extern "C" int gbenv_power_on(gbenv *h, const int32_t *env_ids, int n) {
     return scatter(h, h->d_stage_image, 0 /* version 0 = raw, no merge */, env_ids, n, h->stream);
 }
 
+// gbenv_save_states for one env on the handle's stream, then to the host
 extern "C" int gbenv_save_state(gbenv *h, int env, uint8_t *blob) {
     if (!h || env < 0 || env >= h->n || !blob) return fail(h, GBENV_E_ARG, "gbenv_save_state: bad argument");
     CK(cudaSetDevice(h->device));
-    own(h);  // ordered after whatever was last queued on this handle, on any stream
-    k_gather_image<<<(IMG_WORDS + 255) / 256, 256, 0, h->stream>>>(h->d, h->d_stage_image, env);
+    CK(launch_save_states(h->d, nullptr, env, 1, h->d_stage_blob, own(h)));
     h->launches++;
-    CK(cudaGetLastError());
-    std::vector<uint32_t> img(IMG_WORDS);
-    CK(cudaMemcpyAsync(img.data(), h->d_stage_image, IMG_WORDS * 4, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaMemcpyAsync(blob, h->d_stage_blob, GBENV_STATE_BYTES, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    image_to_blob(img, blob);
+    return GBENV_OK;
+}
+
+extern "C" int gbenv_save_states(gbenv *h, const int32_t *env_ids_dev, int n, uint8_t *blobs_dev, void *stream) {
+    if (!h || n < 0 || (!env_ids_dev && n > h->n) || (n && !blobs_dev) || ((uintptr_t)blobs_dev & 15) || ((uintptr_t)env_ids_dev & 3))
+        return fail(h, GBENV_E_ARG, "gbenv_save_states: bad argument (NULL or misaligned buffer, n < 0, or NULL ids with n > n_envs)");
+    if (n == 0) return GBENV_OK;
+    CK(cudaSetDevice(h->device));
+    CK(launch_save_states(h->d, env_ids_dev, 0, n, blobs_dev, pick(h, stream)));
+    h->launches++;
     return GBENV_OK;
 }
 
