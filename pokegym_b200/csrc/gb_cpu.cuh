@@ -486,7 +486,7 @@ __device__ __forceinline__ bool cpu_exec(Machine &m, const uint4 d, CpuRegs &r, 
     }
     }
 #undef PAIR_OPERAND
-#if !defined(GB_HOSTSIM) && !defined(GB_OPT_NO_JOIN)
+#if !defined(GB_HOSTSIM)
     if (FAST && SIMT) {
         // Opaque join: the empty asm keeps nvcc from threading the handlers that cannot decline straight to the write-back,
         // past this test.  With every path through here, this point post-dominates the handler dispatch and gets a
@@ -550,110 +550,6 @@ __device__ __forceinline__ bool cpu_exec_by_class(Machine &m, const uint4 d, Cpu
 #undef GB_CLS_TEST
 }
 
-// The fast body of the lock-step build (k_run_frames, several envs per warp) as ONE straight line of code: no handler
-// dispatch at all.  Every lane computes the result of every kind of instruction the fast set knows -- the adder, the logic
-// unit, the rotator, BIT / RES / SET, CPL, the 16-bit increments and ADD HL, POP's mask, the branch condition -- from its own
-// control word, and selects pick what is written back; loads and stores are predicated.  A warp whose lanes are at
-// different instructions (the normal state of affairs: its envs are at different places of the game) therefore issues the
-// same instruction stream as a warp in lock-step; what it costs is the longest dependency chain (descriptor -> operand ->
-// ALU -> write-back), not the sum of the handlers its lanes happen to need.  Returns false, having changed nothing, for
-// whatever is outside the fast set (cpu_tick_slow redoes the tick).
-__device__ __forceinline__ bool cpu_exec_lockstep(Machine &m, const uint4 d, CpuRegs &r, uint32_t &rom_off, uint32_t mode, uint32_t &cyc, uint8_t *memb,
-                                                  const uint8_t *rom, uint32_t bank_mask, bool declined) {
-    const uint32_t bcde = r.bcde, hlaf = r.hlaf, sp = r.sp;
-    const uint32_t w = d.w, h = d.x & 0xFF, op = gb_prmt(d.x, 0, 0x4441), ex = gb_prmt(d.x, 0, 0x4442), imm16 = d.y & 0xFFFFu, fall = d.y >> 16;
-    const uint32_t f = hlaf >> 24, a8 = (hlaf >> 16) & 0xFF, hl = hlaf & 0xFFFF;
-    declined |= h >= H_RARE;
-    // ---- control: the branch condition (mask in op, expected flag value in ex; unconditional: mask 0)
-    const bool cond = ((f ^ ex) & op) == 0;
-    const bool is_call = h == H_CALL, is_ret = h == H_RET, is_push = h == H_PUSH, is_pop = h == H_POP;
-    const bool jumps = cond && ((w & PDF_JUMP) || is_call), returns = cond && is_ret, pushes = (cond && is_call) || is_push;
-    // ---- operand and address
-    uint32_t v = gb_prmt(bcde, hlaf, w);  // byte 0 = source register
-    v = (w & PDF_IMM) ? imm16 : v;
-    const uint32_t pair = gb_prmt(bcde, hlaf, w >> 16) & 0xFFFFu;
-    uint32_t wa = (w & PDF_AIMM) ? imm16 : pair;
-    wa = (w & PDF_ASP) ? sp : wa;
-    wa = pushes ? ((sp - 1) & 0xFFFF) : wa;
-    uint32_t off;
-    const bool plain = fast_plain_offset(wa, off);
-    const bool rd = (w & PDF_RD) != 0, rd16 = (w & PDF_RD16) != 0, wr = (w & PDF_WR) != 0;
-    // stores outside plain RAM: MBC3 bank select, sound registers (dropped), P1; anything else is not for the fast body
-    const bool wr_special = wr && !plain;
-    const uint32_t wt = (wa - 0x2000u < 0x2000u) ? FAST_WR_BANK : (wa - 0xFF10u < 0x30u) ? FAST_WR_DROP : wa == 0xFF00u ? FAST_WR_P1 : FAST_WR_NONE;
-    declined |= wr_special && wt == FAST_WR_NONE;
-    declined |= pushes && !fast_stack_push(sp);
-    declined |= wr && (mode & MODE_DEFER) && (wa - 0x8000u < 0x2000u || wa - 0xFE00u < 0x100u);  // deferred PPU: render_flush first
-    // loads: first byte from plain RAM, ROM or P1 / SB / SC; the second byte of POP / RET (always at SP + 1) from work RAM
-    const bool in_rom = wa < 0x8000u, rd_ok = plain || in_rom || (wa - 0xFF00u < 4u), rd16_ok = sp - 0xC000u < 0x3DFFu;
-    declined |= (rd && !rd_ok) || (rd16 && !rd16_ok);
-    v = fast_load_u8(in_rom ? rom : memb, in_rom ? wa + (wa >> 14) * rom_off : off, rd && rd_ok, v);
-    v |= fast_load_u8(memb, mem_offset(MEM_WRAM + ((sp + 1) & 0x1FFF)), rd16 && rd16_ok, 0) << 8;
-    const uint32_t b = v & 0xFF, b7 = b >> 7;
-    // ---- every unit computes
-    // adder.  INC / DEC: a = v, x = +1 / -1, C kept, ex = 0 / N|H;  ADD ADC SUB SBC CP: a = A, x = v or its complement (ex = 0 / 0xFF)
-    const bool inc = (w & PDF_INCDEC) != 0;
-    const uint32_t ad_a = inc ? b : a8, ad_x = inc ? op : (b ^ ex), ad_c = inc ? 0u : ((((f >> 4) & op) ^ ex) & 1);
-    const uint32_t sum = ad_a + ad_x + ad_c, ad_res = sum & 0xFF;
-    const uint32_t ad_f = ((((ad_a ^ ad_x ^ sum) & 0x10) << 1) ^ (ex & 0x60)) | (inc ? (f & FLAG_C) : (((sum >> 4) ^ ex) & 0x10)) | (ad_res == 0 ? FLAG_Z : 0);
-    // logic: AND a & v; XOR a ^ v; OR (a & v) | (a ^ v)
-    const uint32_t lg_res = ((a8 & b) & ex) | ((a8 ^ b) & op);
-    const uint32_t lg_f = (op ? 0 : FLAG_H) | (lg_res == 0 ? FLAG_Z : 0);
-    // rotates and shifts (pd_rot_ex)
-    const uint32_t right = ex & 1;
-    uint32_t rt_c = right ? (b & 1) : b7;
-    const uint32_t rt_in = (((ex >> 1) & rt_c) | ((ex >> 2) & (f >> 4)) | ((ex >> 3) & b7)) & 1;
-    uint32_t rt_res = right ? ((b >> 1) | (rt_in << 7)) : (((b << 1) | rt_in) & 0xFF);
-    rt_res = (ex & 0x10) ? (((b >> 4) | (b << 4)) & 0xFF) : rt_res;
-    rt_c = (ex & 0x10) ? 0u : rt_c;
-    const uint32_t rt_f = ((rt_res == 0 && !(op & 8)) ? FLAG_Z : 0) | (rt_c << 4);
-    // 16-bit: INC rr / DEC rr / HL+ / HL- and ADD HL,rr
-    const uint32_t hli = ((pair + gb_prmt(d.x, 0, 0x9991)) & 0xFFFFu) | (v << 16);
-    const uint32_t t16 = hl + pair;
-    const uint32_t addhl = (t16 & 0xFFFF) | (((f & FLAG_Z) | (((hl & 0xFFF) + (pair & 0xFFF)) > 0xFFF ? FLAG_H : 0) | (t16 > 0xFFFF ? FLAG_C : 0)) << 24);
-    // ---- select the result: 8-bit results travel as res | new F << 8 (the write-back selectors say what is kept)
-    uint32_t rv = v;
-    rv = (w & (PDF_INCDEC | PDF_ARITH)) ? (ad_res | (ad_f << 8)) : rv;
-    rv = h == H_LOGIC ? (lg_res | (lg_f << 8)) : rv;
-    rv = h == H_ROT ? (rt_res | (rt_f << 8)) : rv;
-    rv = h == H_BIT ? (((f & FLAG_C) | FLAG_H | ((b & imm16) ? 0 : FLAG_Z)) << 8) : rv;
-    rv = h == H_RESSET ? ((b & imm16) | (imm16 >> 8)) : rv;
-    rv = h == H_CPL ? ((~a8 & 0xFF) | ((f | FLAG_N | FLAG_H) << 8)) : rv;
-    rv = h == H_HLI ? hli : rv;
-    rv = h == H_ADD_HL ? addhl : rv;
-    rv = is_pop ? (v & (0xFF00u | op)) : rv;
-    // ---- next PC, stack pointer, cycles
-    uint32_t next_pc = jumps ? imm16 : fall;
-    next_pc = returns ? (v & 0xFFFF) : next_pc;
-    next_pc = h == H_JPHL ? hl : next_pc;
-    cyc = (d.x >> 24) + ((jumps || returns) ? (ex & 0xF) : 0u);
-    const uint32_t new_sp = (sp + ((is_pop || returns) ? 2u : 0u) - (pushes ? 2u : 0u)) & 0xFFFF;
-    // ---- what a store writes: the unit's 8-bit result (the register itself for LD (HL+-),A); a push the pair or the return
-    // address, high byte first
-    uint32_t wv = h == H_HLI ? v : rv;
-    wv = pushes ? gb_prmt(is_push ? pair : fall, 0, 0x4401) : wv;
-    if (declined) return false;  // nothing has been changed
-    r.bcde = gb_prmt(bcde, rv, d.z);
-    r.hlaf = gb_prmt(hlaf, rv, d.z >> 16);
-    r.sp = new_sp;
-    r.pc = next_pc;
-    if ((wr && plain) || pushes) memb[off] = (uint8_t)wv;
-    if (pushes) memb[mem_offset(MEM_WRAM + ((sp - 2) & 0x1FFF))] = (uint8_t)(wv >> 8);
-    if (wr_special) {
-        if (wt == FAST_WR_P1) {  // joypad matrix select (a game's input routine writes it several times a frame)
-            memb[mem_offset(MEM_HI + 0x100)] = (uint8_t)joypad_pull(m, wv & 0xFF);
-        } else if (wt == FAST_WR_BANK) {  // MBC3 ROM bank select (constant traffic in banked games)
-            uint32_t bank = wv & 0x7F;
-            bank = bank ? bank : 1;
-            m.rombank = bank;
-            rom_off = (bank_mask ? (bank & bank_mask) : (bank % m.rom_banks)) * 0x4000u - 0x4000u;
-            m.rom_off = rom_off;
-        }
-    }
-    if ((w & PDF_RETI) || h == H_IME) m.ime = h == H_IME ? op : 1u;
-    return true;
-}
-
 // One whole tick on the parked machine, for everything the fast loop declines: CPU.tick (interrupt check, HALT, one
 // instruction from anywhere, through the full bus) followed by Motherboard.tick's HALT fast-forward and Timer.tick's TIMA
 // half.  The caller has brought the clocks up to date; returns the T-cycles to advance them by.
@@ -715,11 +611,7 @@ __device__ __forceinline__ bool cpu_fast_loop(Machine &m, const RunCtx &cx, CpuR
             leave = true;
         }
         if (SIMT) {
-#if !defined(GB_OPT_LOCKSTEP)  // the fully predicated body lost on B200 (400 k vs 620 k env-steps/s at 32,768 envs): see cpu_exec_lockstep
             if (!cpu_exec<true, true>(m, d, r, rom_off, mode, cyc, memb, rom, cx.bank_mask, leave)) return false;
-#else
-            if (!cpu_exec_lockstep(m, d, r, rom_off, mode, cyc, memb, rom, cx.bank_mask, leave)) return false;
-#endif
         } else if (CLASSES) {
             if (!cpu_exec_by_class(m, d, r, rom_off, mode, cyc, memb, rom, cx.bank_mask)) return false;
         } else {

@@ -571,9 +571,6 @@ __device__ GB_NOINLINE int lcd_deadline(Machine &m) {
     const int t = (int)(m.target - m.clock);
     // t <= 0: an event is already due (only inconsistent loaded states get here): strict one event per tick
     if ((m.stat & 0x78) | (m.tmr & 0x04000000u) | (uint32_t)(t <= 0)) return t;
-#if defined(GB_NO_LAZY_LCD)
-    return t;
-#endif
     const uint32_t nm = m.next_mode, ly = m.ly;
     // no line of this frame needs the renderer at its HBlank: rendering is off, or the lines are only recorded (deferred PPU; the
     // first one of a frame is still a hard event: it arms defer_active, which sends VRAM / OAM writes through the slow tick)

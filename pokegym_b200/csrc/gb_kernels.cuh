@@ -6,12 +6,8 @@
 // 64-thread blocks, 12 of them per SM: an 80-register budget (at 64 registers the loop-entry paths spill the machine pointer and
 // the barrier state: 610 k vs 629 k env-steps/s at 32,768 envs) and 24 resident warps per SM -- the lanes policy (gbenv.cu) never
 // asks for more than 16 per SM below 113k envs.
-#ifndef STEP_THREADS
 #define STEP_THREADS 64
-#endif
-#ifndef STEP_MIN_BLOCKS
 #define STEP_MIN_BLOCKS 12
-#endif
 
 // pyboy_binding.ACTIONS (:40) Down Left Right Up A B Start Select -> joypad button ids
 // (Right Left Up Down A B Select Start, the bit order of PyBoy's Interaction nibbles)
@@ -110,9 +106,7 @@ __global__ void __launch_bounds__(STEP_THREADS, STEP_MIN_BLOCKS) k_run_frames(Ru
 // up to 32 blocks x 148 SMs = 4,736 envs in one wave).  With __launch_bounds__(1) ptxas knows that no branch can diverge and
 // emits none of the convergence-barrier scaffolding (BSSY / BSYNC / BREAK / BMOV: about one instruction in nine of the
 // multi-lane build's hot loop), keeps loop-invariant addresses in uniform registers and needs no spills.
-#ifndef STEP1_MIN_BLOCKS
 #define STEP1_MIN_BLOCKS 32
-#endif
 __global__ void __launch_bounds__(1, STEP1_MIN_BLOCKS) k_run_frames_1(RunParams p) {
     const int env = blockIdx.x;
     if (env >= p.d.n_envs || (p.skip && p.skip[env])) return;

@@ -440,7 +440,7 @@ static int launch_run(gbenv *h, const uint8_t *actions_dev, int n_frames, int re
     p.lanes = h->lanes;
     p.defer = h->defer && render_mode != 0;
     p.bank_mask = (h->d.rom_banks & (h->d.rom_banks - 1)) == 0 ? h->d.rom_banks - 1 : 0;
-    if (h->lanes == 1 && !getenv("GBENV_NO_SINGLE")) {  // one env per warp: the single-thread-block build of the same kernel
+    if (h->lanes == 1) {  // one env per warp: the single-thread-block build of the same kernel
         k_run_frames_1<<<h->n, 1, ENV_SMEM_BYTES(1), st>>>(p);
         h->launches++;
         CK(cudaGetLastError());
