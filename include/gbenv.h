@@ -32,10 +32,10 @@
 extern "C" {
 #endif
 
-#define GBENV_ABI_VERSION 8 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
+#define GBENV_ABI_VERSION 9 /* 2: info row widened from 64 to 72 doubles; 3: gbenv_reset_dev, gbenv_submit_host / gbenv_fetch_host, gbenv_check, gbenv_step_masked;
                                4: gbenv_counts_map_sum, gbenv_reduce_info_masked; 5: gbenv_capture_frames, gbenv_frames_to_rgb;
                                6: gbenv_event_flags; 7: gbenv_step_packed, gbenv_reset_packed, gbenv_unpack_obs;
-                               8: gbenv_save_states */
+                               8: gbenv_save_states; 9: gbenv_load_states */
 
 #define GBENV_STATE_BYTES 142610 /* PyBoy v9 save-state length (SURVEY.md 8c)              */
 #define GBENV_OBS_H 72           /* environment.py:154-166: (144//2, 160//2, 4) uint8       */
@@ -107,6 +107,27 @@ int gbenv_save_state(gbenv_t *h, int env, uint8_t *blob_host /* GBENV_STATE_BYTE
  * non-16-byte-aligned blobs_dev with n > 0, n < 0, or NULL ids with n > n_envs; n == 0 is a successful no-op.
  * The output is large (584 MB for 4,096 envs); pass ids to save fewer.                                                */
 int gbenv_save_states(gbenv_t *h, const int32_t *env_ids_dev, int n, uint8_t *blobs_dev, void *stream);
+/* PyBoy.load_state for a list of envs from device-resident v9 files: entry i loads env env_ids_dev[i] from row i of
+ * blobs_dev uint8[n][GBENV_STATE_BYTES] (rows contiguous, blobs_dev 16-byte aligned: the layout gbenv_save_states writes, so
+ * gbenv_load_states(ids, gbenv_save_states(ids)) works on one buffer).  env_ids_dev is int32[n] on the device; NULL means
+ * envs 0..n-1 (n <= n_envs).  For every env the result is bit-identical to gbenv_add_state_template + gbenv_load_template
+ * of the same bytes: the call equals loading the entries one at a time in list order, skipping the ones it rejects, except
+ * that of several accepted entries for one env only the last is loaded (an env never ends up with words of two rows).
+ *   - an entry whose id is outside [0, n_envs) is skipped and its row is not read;
+ *   - a row that is not a loadable v9 file is rejected and its env left untouched.  The rules are those of
+ *     gbenv_add_state_template for v9: byte 0 is 9, the cgb byte is 0, the high 32 bits of clock and clock_target are 0,
+ *     and every screen word is one of PyBoy's four DMG values.  A rejected entry does not block an earlier valid one for
+ *     the same env.
+ * status_dev int32[n] (NULL: not reported) gets per entry 0 when its row was loaded or lost to a later entry for the same
+ * env, GBENV_E_STATE when its row was rejected, GBENV_E_ARG when its id is out of range.
+ * Emulator state only, as gbenv_load_template: rewards, visited bitmaps, heat maps and info rows are unchanged, and so are
+ * the initial template and the reset count.  To start episodes from the loaded states call gbenv_reset_dev(mask) next; a
+ * reset after an env's first one reloads nothing (environment.py:1241-1242).  An env whose first reset is still ahead
+ * loads its initial template on that reset, replacing what this call loaded.
+ * Asynchronous on `stream` (no host synchronisation) and ordered after earlier calls on the handle.  GBENV_E_ARG on a NULL
+ * handle, a NULL or non-16-byte-aligned blobs_dev with n > 0, env_ids_dev or status_dev not 4-byte aligned, n < 0, or NULL
+ * ids with n > n_envs; n == 0 is a successful no-op.                                                                   */
+int gbenv_load_states(gbenv_t *h, const int32_t *env_ids_dev, int n, const uint8_t *blobs_dev, int32_t *status_dev, void *stream);
 
 /* ---- (1)+(2) emulator: tick loop + PPU ------------------------------------------------------
  * replaces pyboy_binding.run_action_on_emulator (:71-91): press, 24 x tick (release before tick 8,

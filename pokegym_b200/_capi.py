@@ -18,7 +18,7 @@ STATE_BYTES = 142_610
 OBS_H, OBS_W, OBS_C = 72, 80, 4
 OBS_BYTES = OBS_H * OBS_W * OBS_C
 INFO_SCALARS = 72
-ABI_VERSION = 8
+ABI_VERSION = 9
 COUNTS_H, COUNTS_W = 444, 436
 SCREEN_H, SCREEN_W = 144, 160
 FRAME_WORDS = 1440  # packed frame: 144 lines x 10 uint32 words of 16 2-bit shades (include/gbenv.h)
@@ -99,6 +99,7 @@ _SIGS = {
     "power_on": ([C.c_void_p, C.c_void_p, C.c_int], C.c_int),
     "save_state": ([C.c_void_p, C.c_int, C.c_void_p], C.c_int),
     "save_states": ([C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p], C.c_int),
+    "load_states": ([C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p], C.c_int),
     "run_action": ([C.c_void_p, C.c_void_p, C.c_int, C.c_void_p], C.c_int),
     "tick": ([C.c_void_p, C.c_int, C.c_int, C.c_void_p], C.c_int),
     "send_input": ([C.c_void_p, C.c_int, C.c_int, C.c_void_p], C.c_int),
@@ -221,6 +222,20 @@ class Handle:
         [0, n_envs) are left untouched."""
         n = _byte_rows(out, STATE_BYTES, "out", None if env_ids is None else len(env_ids))
         self._check(self.lib.save_states(self._h, _ptr(env_ids), int(n), _ptr(out), C.c_void_p(stream or 0)), "save_states")
+
+    def load_states(self, blobs, env_ids=None, status=None, stream=None):
+        """PyBoy.load_state of row i of blobs uint8 [n, STATE_BYTES] into env env_ids[i] (int32, on the device for CUDA, host
+        memory for the oracle; None: envs 0..n-1).  status (int32 [n], or None) gets 0 for a loaded row, GBENV_E_STATE (-2)
+        for a rejected one and GBENV_E_ARG (-1) for an id outside [0, n_envs), whose row is skipped."""
+        n = _byte_rows(blobs, STATE_BYTES, "blobs", None if env_ids is None else len(env_ids))
+        if status is not None:
+            if isinstance(status, np.ndarray):
+                ok = status.dtype == np.int32 and status.flags["C_CONTIGUOUS"]
+            else:
+                ok = str(status.dtype) == "torch.int32" and status.is_contiguous()
+            if not ok or _nbytes(status) != 4 * n:
+                raise ValueError(f"status must be a contiguous int32 buffer of {n} entries")
+        self._check(self.lib.load_states(self._h, _ptr(env_ids), int(n), _ptr(blobs), _ptr(status), C.c_void_p(stream or 0)), "load_states")
 
     # -- emulator ------------------------------------------------------------
     def run_action(self, actions, frame_skip: int = ACT_FREQ, stream: int = 0):

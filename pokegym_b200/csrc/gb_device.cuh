@@ -24,8 +24,6 @@
 #define IRQ_SERIAL 0x08u
 #define IRQ_JOYPAD 0x10u
 
-#define FRAME_CYCLES 70224u
-
 #define M_SCX(m) ((m).scroll & 0xFF)
 #define M_SCY(m) (((m).scroll >> 8) & 0xFF)
 #define M_WX(m) (((m).scroll >> 16) & 0xFF)

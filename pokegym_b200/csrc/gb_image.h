@@ -140,6 +140,108 @@ __host__ __device__ constexpr int state_section_of(const StateLayout &t, uint32_
     return lo;
 }
 
+// ---- The other direction, v9 file -> canonical image, from the same table: state_image_word is the inverse of state_word /
+// state_byte (k_load_states in gb_state.cu; tests/hostsim checks it against blob_to_image).
+
+// Image bits a v9 file does not carry, the one definition blob_to_image and state_image_word share: R_JOY's ly_window
+// (0xFF; a load keeps the env's own) and lp_dirty (144), R_MISC (0xFF: blank shade unknown, no lines pending), and R_LCD2's
+// stat_mode bits, STAT & 3 (a load keeps the env's own).  R_INT's fault bit is 0, like every other bit not listed here.
+__host__ __device__ constexpr uint32_t state_unfiled_bits(uint32_t j, uint32_t stat) {
+    return j == IMG_REGS + R_JOY ? (0xFFu << 16) | (144u << 24) : j == IMG_REGS + R_MISC ? 0xFFu : j == IMG_REGS + R_LCD2 ? (stat & 3) << 24 : 0u;
+}
+
+// the file byte that holds image byte b; where the file holds a byte twice (double_speed, cgb) the first copy, which is the
+// one blob_to_image reads
+constexpr uint32_t state_file_byte(const StateLayout &t, uint32_t b) {
+    for (int i = 0; i < STATE_SECTIONS; i++)
+        if (t.s[i].kind == SK_BYTES && b >= t.s[i].src && b < t.s[i].src + t.s[i].len) return t.s[i].off + (b - t.s[i].src);
+    return ~0u;
+}
+constexpr int state_section_of_kind(const StateLayout &t, uint8_t kind) {
+    for (int i = 0; i < STATE_SECTIONS; i++)
+        if (t.s[i].kind == kind) return i;
+    return -1;
+}
+static constexpr uint32_t STATE_OFF_LCDC = state_file_byte(STATE_LAYOUT, state_reg_byte(R_LCD0, 0));
+static constexpr uint32_t STATE_OFF_STAT = state_file_byte(STATE_LAYOUT, state_reg_byte(R_LCD0, 1));
+static constexpr uint32_t STATE_OFF_CGB = state_file_byte(STATE_LAYOUT, state_reg_byte(R_HDR, 3));
+static constexpr int STATE_FB_SECTION = state_section_of_kind(STATE_LAYOUT, SK_FB);
+static_assert(STATE_OFF_CGB == 4 && STATE_OFF_LCDC == 8375 && STATE_LAYOUT.s[STATE_FB_SECTION].off == 9125, "v9 offsets (SURVEY.md 8c)");
+
+__host__ __device__ inline int state_ctz64(uint64_t m) {
+#if defined(__CUDA_ARCH__)
+    return __ffsll((long long)m) - 1;
+#else
+    return __builtin_ctzll(m);
+#endif
+}
+
+// a screen word is one of PyBoy's four DMG values (SHADE_WORDS); the shade of one that is
+__host__ __device__ inline bool state_shade_ok(uint32_t v) {
+    return v == state_shade_word(0) || v == state_shade_word(1) || v == state_shade_word(2) || v == state_shade_word(3);
+}
+__host__ __device__ inline uint32_t state_shade_of(uint32_t v) {
+    return v == state_shade_word(1) ? 1u : v == state_shade_word(2) ? 2u : v == state_shade_word(3) ? 3u : 0u;
+}
+
+// Image word j of the canonical image of a v9 file.  `secs` has bit s set for the sections that may give word j bits (a
+// superset is fine: the others give none); rd(o) returns file bytes o .. o + 3 as a little-endian word, of which only the
+// bytes inside those sections are used.  Per section kind, the inverse of state_byte: SK_BYTES bytes go back into their
+// word, an SK_FIELD byte is masked and shifted into place, a scanline record is its 4 bytes plus 0x10 when byte 4 is
+// non-zero (blob_to_image's rule, not bit 0 shifted), and 16 screen words become 16 two-bit shades.  Where two sections
+// give the same bits (the second copies of double_speed and cgb) the first in file order wins; the bits no section gives
+// are state_unfiled_bits.  For a file state_row_valid accepts this is blob_to_image's word.
+template <class Rd>
+__host__ __device__ inline uint32_t state_image_word(const StateLayout &t, uint64_t secs, uint32_t j, const Rd &rd) {
+    uint32_t w = 0, have = 0;
+    for (; secs; secs &= secs - 1) {
+        const StateSection &s = t.s[state_ctz64(secs)];
+        uint32_t v = 0, m = ~0u;
+        if (s.kind == SK_BYTES) {
+            const uint32_t b0 = 4 * j > s.src ? 4 * j : s.src, b1 = 4 * j + 4 < s.src + s.len ? 4 * j + 4 : s.src + s.len;
+            if (b0 >= b1) continue;
+            m = (0xFFFFFFFFu >> (32 - 8 * (b1 - b0))) << (8 * (b0 & 3));
+            v = rd(s.off + (b0 - s.src)) << (8 * (b0 & 3));
+        } else if (s.kind == SK_FIELD) {
+            if (j != s.src) continue;
+            m = (uint32_t)s.mask << s.shift;
+            v = rd(s.off) << s.shift;
+        } else if (s.kind == SK_LP) {
+            const uint32_t r = j - IMG_LP;
+            if (r >= LP_WORDS) continue;
+            v = r & 1 ? (rd(s.off + 5 * (r >> 1) + 4) & 0xFF ? 0x10u : 0u) : rd(s.off + 5 * (r >> 1));
+        } else if (s.kind == SK_FB) {
+            const uint32_t q = j - IMG_FB;
+            if (q >= FB_WORDS) continue;
+            for (uint32_t p = 0; p < 16; p++) v |= state_shade_of(rd(s.off + 64 * q + 4 * p)) << (2 * p);
+        } else {
+            continue;
+        }
+        w |= v & m & ~have;
+        have |= m;
+    }
+    return w | state_unfiled_bits(j, j == IMG_REGS + R_LCD2 ? rd(STATE_OFF_STAT) : 0u);
+}
+
+// blob_to_image's acceptance rules for a v9 file (whose length is fixed): every SK_CONST section holds its constant (the
+// version byte is 9, the high halves of clock and clock_target are 0), the cgb byte is 0, and every screen word is one of
+// PyBoy's four DMG values.  state_head_ok is all but the screen; rd(o) as for state_image_word.
+template <class Rd>
+__host__ __device__ inline bool state_head_ok(const StateLayout &t, const Rd &rd) {
+    bool ok = (rd(STATE_OFF_CGB) & 0xFF) == 0;
+    for (int i = 0; i < STATE_SECTIONS; i++)
+        if (t.s[i].kind == SK_CONST)
+            for (uint32_t o = t.s[i].off; o < t.s[i].off + t.s[i].len; o++) ok &= (rd(o) & 0xFF) == t.s[i].src;
+    return ok;
+}
+template <class Rd>
+__host__ __device__ inline bool state_row_valid(const StateLayout &t, const Rd &rd) {
+    bool ok = state_head_ok(t, rd);
+    const StateSection &fb = t.s[STATE_FB_SECTION];
+    for (uint32_t o = fb.off; o < fb.off + fb.len; o += 4) ok &= state_shade_ok(rd(o));
+    return ok;
+}
+
 // PyBoy v9 / v7 blob -> canonical image (layout: SURVEY.md 8c).  Returns 0 or a negative error.
 static int blob_to_image(const uint8_t *b, size_t len, std::vector<uint32_t> &img, int *version_out, std::string &err) {
     if (len < 1) { err = "empty save-state"; return GBENV_E_STATE; }
@@ -183,7 +285,7 @@ static int blob_to_image(const uint8_t *b, size_t len, std::vector<uint32_t> &im
     }
     regs[R_LCD0] = LCDC | (STAT << 8) | (LY << 16) | (LYC << 24);
     regs[R_LCD1] = SCY | (SCX << 8) | (WY << 16) | (WX << 24);
-    regs[R_LCD2] = BGP | (OBP0 << 8) | (OBP1 << 16) | (((STAT & 3) | ((next_mode & 3) << 2)) << 24);
+    regs[R_LCD2] = BGP | (OBP0 << 8) | (OBP1 << 16) | ((next_mode & 3) << 26) | state_unfiled_bits(IMG_REGS + R_LCD2, STAT);
     regs[R_CLOCK] = (uint32_t)clock;
     regs[R_TARGET] = (uint32_t)target;
     for (uint32_t y = 0; y < 144; y++, p += 5) {
@@ -212,10 +314,10 @@ static int blob_to_image(const uint8_t *b, size_t len, std::vector<uint32_t> &im
     regs[R_MBC] = p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24);
     p += 4;
     for (uint32_t i = 0; i < 0x8000; i++) img_set_byte(img, IMG_CRAM, i, *p++);
-    regs[R_JOY] = p[0] | (p[1] << 8) | (0xFFu << 16) | (144u << 24);  // ly_window kept by the merge, lp_dirty = 144
+    regs[R_JOY] = p[0] | (p[1] << 8) | state_unfiled_bits(IMG_REGS + R_JOY, 0);  // ly_window kept by the merge, lp_dirty = 144
     p += 2;
     regs[R_HDR] = hdr;
-    regs[R_MISC] = 0xFF;
+    regs[R_MISC] = state_unfiled_bits(IMG_REGS + R_MISC, 0);
     if ((size_t)(p - b) != len) { err = "save-state length mismatch"; return GBENV_E_STATE; }
     *version_out = ver;
     return GBENV_OK;

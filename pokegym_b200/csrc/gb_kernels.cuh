@@ -163,33 +163,6 @@ __global__ void __launch_bounds__(32 * RENDER_LINES_PER_BLOCK) k_render_pending(
 #endif
 
 // ---------------------------------------------------------------------------------------------
-// PyBoy load_state semantics that depend on the env's previous state (oracle GBQ_STAT_LOAD_KEEPS_MODE):
-// STAT bits 0-2 and STATRegister._mode survive a load; LCD-off states force mode 0 through set_lcdc.
-// For v7 blobs clock / clock_target / next_stat_mode / IF / interrupt_queued are not in the file.
-__device__ __forceinline__ uint32_t merge_loaded_reg(uint32_t r, uint32_t old, uint32_t neu, int version, uint32_t new_lcdc) {
-    if (version == 0) return neu;  // raw image (power-on): no PyBoy load_state semantics
-    bool lcd_off = !(new_lcdc & 0x80);
-    if (r == R_LCD0) {
-        uint32_t old_stat = (old >> 8) & 0xFF;
-        if (lcd_off) old_stat &= 0xFC;  // set_lcdc -> STAT.set_mode(0)
-        uint32_t stat = (old_stat & 0x87) | ((neu >> 8) & 0x78);
-        return (neu & 0xFFFF00FFu) | (stat << 8);
-    }
-    if (r == R_LCD2) {
-        uint32_t oldf = old >> 24, mode = oldf & 3, next = (neu >> 26) & 3;
-        if (lcd_off) mode = 0;
-        if (version < 8) next = lcd_off ? 2 : ((oldf >> 2) & 3);
-        return (neu & 0x00FFFFFFu) | ((mode | (next << 2) | (oldf & 0x30)) << 24);
-    }
-    if (r == R_JOY) return (neu & 0xFF00FFFFu) | (old & 0x00FF0000u);  // Renderer.ly_window is not serialised
-    if (version < 8) {
-        if (r == R_CLOCK) return lcd_off ? 0 : old;
-        if (r == R_TARGET) return lcd_off ? FRAME_CYCLES : old;
-        if (r == R_INT) return (neu & 0x0000FF17u) | (old & 0x00FF0008u);  // keep IF and interrupt_queued
-    }
-    return neu;
-}
-
 // grid: (ceil(n / 32), ceil(IMG_WORDS / 8)); block (32, 8): x = env slot (coalesced), y = image word
 __global__ void k_scatter_image(DevArrays d, const uint32_t *image, const int32_t *env_ids, int n, int version) {
     int i = blockIdx.x * 32 + threadIdx.x;

@@ -1,4 +1,5 @@
-// gb_state.cu -- the PyBoy v9 file of a list of envs (gbenv_save_states), linked into libgbenv.so next to gbenv.cu.
+// gb_state.cu -- the PyBoy v9 file of a list of envs (gbenv_save_states) and back (gbenv_load_states), linked into
+// libgbenv.so next to gbenv.cu.
 //
 // The file layout is STATE_LAYOUT (gb_image.h), the same table image_to_blob serialises from.  Output row i is the file of
 // list entry i, rows back to back, so row i starts at byte i * GBENV_STATE_BYTES = 2i (mod 16) of the 16-byte aligned output,
@@ -176,5 +177,226 @@ __global__ void __launch_bounds__(GB_TILE * SAVE_WARPS) k_save_states(const DevA
 
 cudaError_t launch_save_states(const DevArrays &d, const int32_t *ids, int id0, int n, uint8_t *blobs, cudaStream_t st) {
     k_save_states<<<dim3((n + GB_TILE - 1) / GB_TILE, SAVE_CHUNKS), dim3(GB_TILE, SAVE_WARPS), 0, st>>>(d, ids, id0, n, blobs);
+    return cudaGetLastError();
+}
+
+// ---------------------------------------------------------------------------------------------------- gbenv_load_states
+// The reverse direction: rows (v9 files, laid out as k_save_states writes them) into the envs' state.  k_load_check decides
+// which entry each env takes, before anything is written; k_load_states then writes the image words of those entries.
+
+#define LOAD_CHUNK 1024  // file bytes of a bulk section per block (per list entry)
+#define LOAD_WARPS 8
+#define LOAD_CHECK_WARPS 8
+#define LOAD_MAX_CHUNKS 160
+#define LOAD_MAX_SEGS 160
+#define LOAD_MAX_WINS 160
+
+// Which image words a block writes and which file bytes it stages for them.  The bulk sections (RAM runs of at least
+// LOAD_CHUNK bytes, and the screen) are cut into LOAD_CHUNK-byte pieces, one chunk each: one window of file bytes, one
+// segment of whole image words.  The last chunk takes every other image word, in segments split at the image regions,
+// each with the sections that can feed it, and stages the file runs of all other sections.
+struct LoadPlan {
+    uint16_t seg0[LOAD_MAX_CHUNKS], nseg[LOAD_MAX_CHUNKS], win0[LOAD_MAX_CHUNKS], nwin[LOAD_MAX_CHUNKS];
+    uint32_t j0[LOAD_MAX_SEGS], j1[LOAD_MAX_SEGS];  // segment: image words j0 .. j1 - 1, fed by the sections in secs
+    uint64_t secs[LOAD_MAX_SEGS];
+    uint32_t lo[LOAD_MAX_WINS], hi[LOAD_MAX_WINS], base[LOAD_MAX_WINS];  // window: file bytes [lo, hi), staged at smem word base
+    uint32_t n_chunks, max_words;
+};
+
+constexpr bool load_bulk(const StateSection &s) {
+    return (s.kind == SK_BYTES && s.len >= LOAD_CHUNK) || s.kind == SK_FB;
+}
+// image words [w0, w1] a section gives bits to (w0 > w1: none)
+constexpr void load_image_range(const StateSection &s, uint32_t &w0, uint32_t &w1) {
+    w0 = 1;
+    w1 = 0;
+    if (s.kind == SK_BYTES) { w0 = s.src >> 2; w1 = (s.src + s.len - 1) >> 2; }
+    if (s.kind == SK_FIELD) { w0 = w1 = s.src; }
+    if (s.kind == SK_LP) { w0 = IMG_LP; w1 = IMG_LP + LP_WORDS - 1; }
+    if (s.kind == SK_FB) { w0 = IMG_FB; w1 = IMG_FB + FB_WORDS - 1; }
+}
+// staged words of a window: the aligned 16-byte units over [lo, hi + 3) at any row alignment
+constexpr uint32_t load_window_words(uint32_t lo, uint32_t hi) { return 4 * ((hi - lo + 3 + 15 + 15) / 16); }
+
+constexpr LoadPlan make_load_plan() {
+    LoadPlan p{};
+    uint32_t c = 0, sg = 0, wn = 0;
+    for (int i = 0; i < STATE_SECTIONS; i++) {
+        const StateSection &s = STATE_LAYOUT.s[i];
+        if (!load_bulk(s)) continue;
+        const uint32_t bytes_per_word = s.kind == SK_FB ? 64 : 4;
+        for (uint32_t o = 0; o < s.len; o += LOAD_CHUNK, c++, sg++, wn++) {
+            const uint32_t e = o + LOAD_CHUNK < s.len ? o + LOAD_CHUNK : s.len;
+            const uint32_t w0 = s.kind == SK_FB ? IMG_FB : s.src >> 2;
+            p.seg0[c] = (uint16_t)sg; p.nseg[c] = 1; p.win0[c] = (uint16_t)wn; p.nwin[c] = 1;
+            p.j0[sg] = w0 + o / bytes_per_word; p.j1[sg] = w0 + e / bytes_per_word; p.secs[sg] = 1ull << i;
+            p.lo[wn] = s.off + o; p.hi[wn] = s.off + e; p.base[wn] = 0;
+            if (load_window_words(s.off + o, s.off + e) > p.max_words) p.max_words = load_window_words(s.off + o, s.off + e);
+        }
+    }
+    // the last chunk: image words outside the bulk sections, in segments that do not cross a region boundary
+    uint32_t cut[32] = {0, IMG_CRAM, IMG_FB, IMG_LP, IMG_REGS, IMG_WORDS};
+    uint32_t ncut = 6;
+    for (int i = 0; i < STATE_SECTIONS; i++) {
+        uint32_t w0 = 0, w1 = 0;
+        load_image_range(STATE_LAYOUT.s[i], w0, w1);
+        if (load_bulk(STATE_LAYOUT.s[i])) { cut[ncut++] = w0; cut[ncut++] = w1 + 1; }
+    }
+    for (uint32_t a = 1; a < ncut; a++)  // sort
+        for (uint32_t b = a; b > 0 && cut[b - 1] > cut[b]; b--) { const uint32_t t = cut[b]; cut[b] = cut[b - 1]; cut[b - 1] = t; }
+    p.seg0[c] = (uint16_t)sg;
+    p.win0[c] = (uint16_t)wn;
+    for (uint32_t a = 0; a + 1 < ncut; a++) {
+        const uint32_t lo = cut[a], hi = cut[a + 1];
+        bool bulk = false;
+        uint64_t secs = 0;
+        for (int i = 0; i < STATE_SECTIONS; i++) {
+            uint32_t w0 = 0, w1 = 0;
+            load_image_range(STATE_LAYOUT.s[i], w0, w1);
+            if (w0 > w1 || w1 < lo || w0 >= hi) continue;
+            if (load_bulk(STATE_LAYOUT.s[i])) bulk = true;
+            else secs |= 1ull << i;
+        }
+        if (lo == hi || bulk) continue;
+        p.j0[sg] = lo; p.j1[sg] = hi; p.secs[sg] = secs;
+        sg++;
+    }
+    p.nseg[c] = (uint16_t)(sg - p.seg0[c]);
+    uint32_t words = 0;
+    for (int i = 0; i < STATE_SECTIONS; i++) {  // windows: the file runs of the other sections, adjacent ones merged
+        const StateSection &s = STATE_LAYOUT.s[i];
+        if (load_bulk(s)) continue;
+        if (wn > p.win0[c] && p.hi[wn - 1] == s.off) { p.hi[wn - 1] = s.off + s.len; continue; }
+        p.lo[wn] = s.off; p.hi[wn] = s.off + s.len;
+        wn++;
+    }
+    p.nwin[c] = (uint16_t)(wn - p.win0[c]);
+    for (uint32_t m = p.win0[c]; m < wn; m++) { p.base[m] = words; words += load_window_words(p.lo[m], p.hi[m]); }
+    if (words > p.max_words) p.max_words = words;
+    p.n_chunks = c + 1;
+    return p;
+}
+
+static constexpr LoadPlan LOAD_PLAN = make_load_plan();
+static_assert(LOAD_PLAN.n_chunks <= LOAD_MAX_CHUNKS && LOAD_PLAN.seg0[LOAD_PLAN.n_chunks - 1] + LOAD_PLAN.nseg[LOAD_PLAN.n_chunks - 1] <= LOAD_MAX_SEGS &&
+              LOAD_PLAN.win0[LOAD_PLAN.n_chunks - 1] + LOAD_PLAN.nwin[LOAD_PLAN.n_chunks - 1] <= LOAD_MAX_WINS, "raise the LOAD_MAX_* limits");
+// odd, so that the lanes of a warp, one entry each, read different banks; at least one word past the last window, which a
+// file word that starts on a word boundary reads (and ignores)
+#define LOAD_ROW ((LOAD_PLAN.max_words + 1) | 1)
+static_assert(GB_TILE * LOAD_ROW * 4 <= 48 * 1024, "staging fits the static shared-memory limit");
+
+static __constant__ LoadPlan c_lplan = LOAD_PLAN;
+
+__host__ __device__ constexpr unsigned long long load_key(uint32_t seq, int i) { return ((unsigned long long)seq << 32) | (uint32_t)i; }
+
+// grid ceil(n / LOAD_CHECK_WARPS), block (32, LOAD_CHECK_WARPS): warp y checks list entry blockIdx.x * LOAD_CHECK_WARPS + y.
+// The screen section is read as aligned 16-byte units; its words all start at the same byte of a 32-bit word (rows start at
+// 2i mod 16), so each is a funnel shift of two loaded words.  An accepted entry claims its env with atomicMax of its key:
+// of the accepted entries for one env, the last in the list holds the claim when the kernel ends.
+__global__ void __launch_bounds__(32 * LOAD_CHECK_WARPS) k_load_check(const int32_t *__restrict__ ids, int n, int n_envs, const uint8_t *__restrict__ blobs,
+                                                                      int32_t *__restrict__ status, unsigned long long *__restrict__ claim, uint32_t seq) {
+    const int i = blockIdx.x * LOAD_CHECK_WARPS + threadIdx.y, lane = threadIdx.x;
+    if (i >= n) return;
+    const int env = ids ? ids[i] : i;
+    if (env < 0 || env >= n_envs) {
+        if (status && lane == 0) status[i] = GBENV_E_ARG;
+        return;
+    }
+    const uint8_t *row = blobs + (size_t)i * GBENV_STATE_BYTES;
+    bool ok = true;
+    if (lane == 0) ok = state_head_ok(c_layout, [&](uint32_t o) { return (uint32_t)__ldg(row + o); });
+    const StateSection &fb = c_layout.s[STATE_FB_SECTION];
+    const size_t g0 = (size_t)i * GBENV_STATE_BYTES + fb.off, g1 = g0 + fb.len;  // screen bytes, from the aligned base
+    const uint32_t sh = 8 * (uint32_t)(g0 & 3);
+    const uint4 *units = reinterpret_cast<const uint4 *>(blobs);
+    const uint32_t *words = reinterpret_cast<const uint32_t *>(blobs);
+    for (size_t u = (g0 >> 4) + lane; u < (g1 + 15) >> 4; u += 32) {
+        const uint4 q = __ldg(units + u);
+        const uint32_t v[5] = {q.x, q.y, q.z, q.w, __ldg(words + 4 * u + 4)};  // the screen is followed by WRAM: still in the row
+#pragma unroll
+        for (int t = 0; t < 4; t++) {
+            const size_t a = 16 * u + 4 * t + (g0 & 3);  // the screen word that starts in word t of the unit
+            if (a >= g0 && a < g1) ok &= state_shade_ok(__funnelshift_r(v[t], v[t + 1], sh));
+        }
+    }
+    ok = __all_sync(0xFFFFFFFFu, ok);
+    if (lane == 0) {
+        if (status) status[i] = ok ? GBENV_OK : GBENV_E_STATE;
+        if (ok) atomicMax(claim + env, load_key(seq, i));
+    }
+}
+
+// grid (ceil(n / 32), LOAD_PLAN.n_chunks), block (32, LOAD_WARPS).
+// Staging: warp y takes entries y, y + 8, ..; its lanes read the chunk's windows of the entry's row as consecutive aligned
+// 16-byte units into shared memory, one row per entry.  Writing: lane x takes entry x and warp y every LOAD_WARPS-th image
+// word of the chunk, derived by state_image_word from the staged bytes (a file word is a funnel shift of two staged words)
+// and stored through image_slot, so when the entries are the 32 envs of a tile in order each warp store is one 128-byte
+// line.  Register words are merged with the env's old ones as a PyBoy v9 load does.  An entry whose env's claim is not its
+// own key (out-of-range id, rejected row, or a later entry for the same env) stages and writes nothing.
+__global__ void __launch_bounds__(GB_TILE * LOAD_WARPS) k_load_states(const DevArrays d, const int32_t *__restrict__ ids, int n, const uint8_t *__restrict__ blobs,
+                                                                     const unsigned long long *__restrict__ claim, uint32_t seq) {
+    __shared__ uint32_t s_img[GB_TILE * LOAD_ROW];
+    __shared__ int s_env[GB_TILE];
+    const int tx = threadIdx.x, ty = threadIdx.y, first = blockIdx.x * GB_TILE, c = blockIdx.y;
+    const uint32_t win0 = c_lplan.win0[c], nwin = c_lplan.nwin[c];
+    const size_t total = (size_t)n * GBENV_STATE_BYTES;
+    if (ty == 0) {
+        int env = -1;
+        if (first + tx < n) {
+            const int e = ids ? ids[first + tx] : first + tx;
+            if (e >= 0 && e < d.n_envs && claim[e] == load_key(seq, first + tx)) env = e;
+        }
+        s_env[tx] = env;
+    }
+    __syncthreads();
+    for (int k = ty; k < GB_TILE; k += LOAD_WARPS) {
+        if (s_env[k] < 0) continue;
+        const size_t row0 = (size_t)(first + k) * GBENV_STATE_BYTES;
+        uint32_t *srow = s_img + k * LOAD_ROW;
+        for (uint32_t m = 0; m < nwin; m++) {
+            const size_t u0 = (row0 + c_lplan.lo[win0 + m]) >> 4, end = row0 + c_lplan.hi[win0 + m] + 3;
+            const size_t u1 = ((end < total ? end : total) + 15) >> 4;
+            for (size_t u = u0 + tx; u < u1; u += 32) {
+                uint4 q;
+                if (16 * u + 16 <= total) {
+                    q = __ldg(reinterpret_cast<const uint4 *>(blobs) + u);
+                } else {  // the last unit of the buffer, which may end inside it
+                    uint32_t b[4] = {0, 0, 0, 0};
+                    for (size_t x = 16 * u; x < total; x++) b[(x >> 2) & 3] |= (uint32_t)blobs[x] << (8 * (x & 3));
+                    q = make_uint4(b[0], b[1], b[2], b[3]);
+                }
+                uint32_t *dst = srow + c_lplan.base[win0 + m] + 4 * (uint32_t)(u - u0);
+                dst[0] = q.x; dst[1] = q.y; dst[2] = q.z; dst[3] = q.w;
+            }
+        }
+    }
+    __syncthreads();
+    const int env = s_env[tx];
+    if (env < 0) return;
+    const size_t row0 = (size_t)(first + tx) * GBENV_STATE_BYTES;
+    const uint32_t *srow = s_img + tx * LOAD_ROW;
+    const auto rd = [&](uint32_t o) -> uint32_t {
+        uint32_t m = 0;
+        while (m + 1 < nwin && c_lplan.lo[win0 + m + 1] <= o) m++;
+        const size_t g = row0 + o;
+        const uint32_t w = c_lplan.base[win0 + m] + (uint32_t)((g >> 2) - (((row0 + c_lplan.lo[win0 + m]) >> 4) << 2));
+        return __funnelshift_r(srow[w], srow[w + 1], 8 * (uint32_t)(g & 3));
+    };
+    const uint32_t seg0 = c_lplan.seg0[c], nseg = c_lplan.nseg[c];
+    for (uint32_t sg = seg0; sg < seg0 + nseg; sg++) {
+        const uint64_t secs = c_lplan.secs[sg];
+        for (uint32_t j = c_lplan.j0[sg] + ty; j < c_lplan.j1[sg]; j += LOAD_WARPS) {
+            uint32_t v = state_image_word(c_layout, secs, j, rd);
+            uint32_t *slot = image_slot(d, env, j);
+            if (j >= IMG_REGS) v = merge_loaded_reg(j - IMG_REGS, *slot, v, 9, rd(STATE_OFF_LCDC) & 0xFF);
+            *slot = v;
+        }
+    }
+}
+
+cudaError_t launch_load_states(const DevArrays &d, const int32_t *ids, int n, const uint8_t *blobs, int32_t *status, unsigned long long *claim,
+                               uint32_t seq, cudaStream_t st) {
+    k_load_check<<<(n + LOAD_CHECK_WARPS - 1) / LOAD_CHECK_WARPS, dim3(32, LOAD_CHECK_WARPS), 0, st>>>(ids, n, d.n_envs, blobs, status, claim, seq);
+    k_load_states<<<dim3((n + GB_TILE - 1) / GB_TILE, LOAD_PLAN.n_chunks), dim3(GB_TILE, LOAD_WARPS), 0, st>>>(d, ids, n, blobs, claim, seq);
     return cudaGetLastError();
 }

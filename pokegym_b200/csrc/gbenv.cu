@@ -38,6 +38,8 @@ struct gbenv {
     unsigned long long *d_counters = nullptr;
     uint32_t *d_stage_image = nullptr;
     uint8_t *d_stage_blob = nullptr;  // GBENV_STATE_BYTES, gbenv_save_state
+    unsigned long long *d_load_claim = nullptr;  // [n] gbenv_load_states: (call << 32 | entry) of the entry an env takes
+    uint32_t load_calls = 0;                     // gbenv_load_states calls so far (the high half of the claim keys)
     uint8_t *d_stage_buf = nullptr;  // 64 KiB scratch for bus access
     double *d_info_rows = nullptr;
     int32_t *d_env_ids = nullptr;
@@ -163,7 +165,7 @@ extern "C" int gbenv_destroy(gbenv *h) {
     cudaFree(h->w.ctl);
     if (h->pool_err_host) cudaFreeHost(h->pool_err_host);
     cudaFree(h->d_cm_dense);
-    cudaFree(h->d_counters); cudaFree(h->d_stage_image); cudaFree(h->d_stage_blob); cudaFree(h->d_stage_buf); cudaFree(h->d_info_rows);
+    cudaFree(h->d_counters); cudaFree(h->d_stage_image); cudaFree(h->d_stage_blob); cudaFree(h->d_load_claim); cudaFree(h->d_stage_buf); cudaFree(h->d_info_rows);
     cudaFree(h->d_env_ids); cudaFree(h->d_mask); cudaFree(h->d_init_tmpl); cudaFree(h->d_tmpl_images); cudaFree(h->d_tmpl_versions);
     for (int k = 0; k < 2; k++) {
         cudaFree(h->d_actions[k]); cudaFree(h->d_obs[k]); cudaFree(h->d_done[k]); cudaFree(h->d_reward[k]);
@@ -286,6 +288,7 @@ static int create_impl(gbenv *&h, int n_envs, const uint8_t *rom_host, size_t ro
     ALLOC(h->d_counters, 8 * sizeof(unsigned long long));
     ALLOC(h->d_stage_image, IMG_WORDS * sizeof(uint32_t));
     ALLOC(h->d_stage_blob, GBENV_STATE_BYTES);
+    ALLOC(h->d_load_claim, (size_t)n_envs * sizeof(unsigned long long));
     ALLOC(h->d_stage_buf, 0x10000);
     ALLOC(h->d_info_rows, (size_t)n_envs * GBENV_INFO_SCALARS * sizeof(double));
     ALLOC(h->d_env_ids, (size_t)n_envs * sizeof(int32_t));
@@ -414,6 +417,22 @@ extern "C" int gbenv_save_states(gbenv *h, const int32_t *env_ids_dev, int n, ui
     CK(cudaSetDevice(h->device));
     CK(launch_save_states(h->d, env_ids_dev, 0, n, blobs_dev, pick(h, stream)));
     h->launches++;
+    return GBENV_OK;
+}
+
+extern "C" int gbenv_load_states(gbenv *h, const int32_t *env_ids_dev, int n, const uint8_t *blobs_dev, int32_t *status_dev, void *stream) {
+    if (!h || n < 0 || (!env_ids_dev && n > h->n) || (n && !blobs_dev) || ((uintptr_t)blobs_dev & 15) || ((uintptr_t)env_ids_dev & 3) ||
+        ((uintptr_t)status_dev & 3))
+        return fail(h, GBENV_E_ARG, "gbenv_load_states: bad argument (NULL or misaligned buffer, n < 0, or NULL ids with n > n_envs)");
+    if (n == 0) return GBENV_OK;
+    CK(cudaSetDevice(h->device));
+    cudaStream_t st = pick(h, stream);
+    if (++h->load_calls == 0) {  // the call counter wrapped: older keys would outrank the new ones
+        CK(cudaMemsetAsync(h->d_load_claim, 0, (size_t)h->n * sizeof(unsigned long long), st));
+        h->load_calls = 1;
+    }
+    CK(launch_load_states(h->d, env_ids_dev, n, blobs_dev, status_dev, h->d_load_claim, h->load_calls, st));
+    h->launches += 2;
     return GBENV_OK;
 }
 

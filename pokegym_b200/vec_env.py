@@ -419,6 +419,36 @@ class VecEnvironment:
         self.handle.save_states(out, ids, stream=self._stream())
         return out
 
+    def load_states(self, rows, env_ids=None):
+        """PyBoy.load_state of row i of `rows` (uint8 [n, 142610], the layout save_states returns) into env env_ids[i] (None:
+        envs 0..n-1), all in one launch on the device, asynchronously on the current stream.  Returns the int32 [n] status
+        tensor: 0 where the row was loaded, -2 (GBENV_E_STATE) where it is not a loadable v9 file and the env was left as it
+        was.  Of several rows for one env the last loadable one wins.  The ids are checked on the host; rows in host memory,
+        on another device, non-contiguous or not 16-byte aligned (a slice rows[k:] usually is not) are copied first.
+        This loads emulator state only: rewards, visited bitmaps and info rows stay as they are, and so does the state an
+        env's first reset loads.  To start episodes from the loaded states, reset those envs next (reset(mask)); an env whose
+        first reset is still ahead loads its initial state there instead.  One state into k envs:
+        load_states(row.expand(k, -1).contiguous(), ids)."""
+        torch = self.torch
+        if not torch.is_tensor(rows):
+            rows = torch.from_numpy(np.ascontiguousarray(rows))
+        if rows.dim() != 2 or rows.shape[1] != _capi.STATE_BYTES or rows.dtype != torch.uint8:
+            raise ValueError(f"rows must be a uint8 tensor or array [n, {_capi.STATE_BYTES}]")
+        n = rows.shape[0]
+        ids = None
+        if env_ids is not None:
+            a = host_env_ids(env_ids, self.num_envs)
+            if a.size != n:
+                raise ValueError(f"{a.size} env ids for {n} rows")
+            ids = torch.from_numpy(a).pin_memory().to(self.device, non_blocking=True)
+        elif n > self.num_envs:
+            raise ValueError(f"{n} rows for {self.num_envs} envs")
+        if rows.device != self.device or not rows.is_contiguous() or rows.data_ptr() % 16:
+            rows = torch.empty((n, _capi.STATE_BYTES), dtype=torch.uint8, device=self.device).copy_(rows, non_blocking=rows.device.type != "cpu")
+        status = torch.empty(n, dtype=torch.int32, device=self.device)
+        self.handle.load_states(rows, ids, status, stream=self._stream())
+        return status
+
     def load_state(self, blob: bytes, env_ids=None):
         """PyBoy.load_state for the listed envs (None: all): pyboy_binding.load_pyboy_state (:65-69)."""
         self.handle.load_template(self.handle.add_state_template(blob), env_ids)
